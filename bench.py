@@ -4,7 +4,14 @@
 One "step" = one matvec = set_weights(w) + evaluate(w, targets = sources) on a pre-built tree
 (exactly one solver matvec of the reference, ferreus_rbf/src/rbf.rs:1357-1364).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n POINTS]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n POINTS] [--dump-outputs DIR]
+
+* `--dump-outputs DIR`: after the timed steps, what each timed path returned in its last step goes to DIR/<name>.npy
+             (float64): `matvec` (the resident matvec of `value`; the oracle port's result with --impl reference),
+             `matvec_sqrt_exact` and `e2e` (the host-buffer result of the last e2e step), each shaped as its caller
+             receives it.  The workload is seeded, so two builds run with the same arguments can be compared output for
+             output.  The device sums are not bit-reproducible: compare with a tolerance (two runs of the default
+             workload on one B200 differ by 3e-16 in relative L2 norm, at most 2.2e-15 relative per row).
 
 * `value`  : whole-job Mpts/s with inputs resident in HBM (fb_tree_matvec_resident), device time from CUDA
              events on the library's launch stream, max over ranks.
@@ -47,6 +54,7 @@ except Exception:
     _TRAFFIC = {}
 NCU_DRAM_BYTES = {k: v["bytes"] for k, v in _TRAFFIC.items() if isinstance(v, dict)}
 NCU_CAPTURE = {k: v["capture"] for k, v in _TRAFFIC.items() if isinstance(v, dict)}
+DUMP_BYTES = 60 << 20  # --dump-outputs budget: the .npy files stay under 64 MB in all, headers included
 
 
 def make_workload(n, seed):
@@ -54,6 +62,19 @@ def make_workload(n, seed):
     pts = rng.random((n, 3))
     w = rng.random((n, 1))
     return pts, w
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy in float64.  Beyond DUMP_BYTES in all, each array keeps the same fixed,
+    seeded sample of its rows (in ascending order), so that two runs stay comparable row for row."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.shape[0] * DUMP_BYTES // total
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -159,30 +180,26 @@ def full_fit(n):
 def run_reference(args):
     """--impl reference: the reference's CPU algorithm (oracle port, all host threads) on the same workload.  Every
     step is one complete, fully timed 1M-point matvec (upward pass, M2L, P2L, L2L and the whole leaf pass; nothing is
-    extrapolated).  A step takes several seconds, so the number of steps actually run is bounded by a wall-clock
-    budget (REF_BUDGET_S) and reported in `steps`."""
+    extrapolated); --steps of them are timed."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    budget_s = float(os.environ.get("REF_BUDGET_S", "150"))
-    t_begin = time.perf_counter()
     pts, w = make_workload(args.n, 1000)
     ff, build_s, cores = cpu_baseline(pts, w, args.cpu_leaf_fraction)
     times = []
     warm = min(args.warmup, 1)
     for it in range(warm + args.steps):
         t0 = time.perf_counter()
-        ff.matvec(w)
+        out = ff.matvec(w)
         sec = time.perf_counter() - t0
         if it >= warm:
             times.append(sec)
-        if times and time.perf_counter() - t_begin + sec > budget_s:
-            break
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"matvec": out})
     ms = 1e3 * float(np.mean(times))
     val = args.n / (ms * 1e-3) / 1e6
-    sample = (f"{len(times)} complete 1M-point matvecs of the oracle port (oracle/fast.py + oracle/csrc/oracle_passes.c, "
-              f"OpenMP, {cores} threads), every stage timed in full; {args.steps} steps requested, bounded by a "
-              f"{budget_s:.0f} s budget")
+    sample = (f"{len(times)} complete {args.n}-point matvecs of the oracle port (oracle/fast.py + "
+              f"oracle/csrc/oracle_passes.c, OpenMP, {cores} threads), every stage timed in full")
     line = {"impl": "reference", "metric": "bbfmm_matvec_throughput", "value": val, "unit": "Mpts/s", "n_gpus": args.gpus,
             "steps": len(times), "warmup": warm, "ms_per_step": ms, "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -216,6 +233,8 @@ def main():
     ap.add_argument("--cpu-leaf-fraction", type=float, default=0.02)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-fit", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what each timed path computed in its last step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -310,6 +329,9 @@ def main():
     barrier()
     wall_s = time.perf_counter() - wall0
     total_ms = float(np.sum(dev_ms))
+    dumps = {}
+    if args.dump_outputs and rank == 0:  # read back before the e2e calls below reuse the tree's result buffer
+        dumps["matvec"] = np.array(tree.sharded_download() if world > 1 else tree.download_result())
 
     # ---- the same resident matvec with the third-order square root (tree rebuilt in that mode)
     exact = None
@@ -327,6 +349,8 @@ def main():
             torch.cuda.synchronize()
             tree_x.matvec_resident()
             xs.append(tree_x.last_matvec_ms())
+        if args.dump_outputs:
+            dumps["matvec_sqrt_exact"] = np.array(tree_x.download_result())
         exact = {"ms_per_step": float(np.mean(xs)), "value": n / (float(np.mean(xs)) * 1e-3) / 1e6, "unit": "Mpts/s",
                  "what": "fb_set_sqrt_mode(0): ~1 ulp square roots in the direct sums"}
         del tree_x
@@ -353,6 +377,9 @@ def main():
     barrier()
     e2e_s = time.perf_counter() - e0
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:
+        dumps["e2e"] = out
+        dump_outputs(args.dump_outputs, dumps)
 
     tms = torch.tensor([total_ms, e2e_s * 1e3], dtype=torch.float64, device="cuda")
     per_rank = None
