@@ -126,6 +126,8 @@ SIGNATURES = {
     "fb_tree_dump_list": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "fb_tree_m2l_rank": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "fb_tree_m2l_operator": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _dp, _dp]),
+    "fb_m2l_stream_warps": (C.c_int, [C.c_int, C.c_int]),
+    "fb_tree_m2l_stream_warps": (C.c_int, [C.c_void_p]),
     "fb_tree_leaf_work": (C.c_int, [C.c_void_p, _u64p, _dp]),
     "fb_tree_morton_order": (C.c_int, [C.c_void_p, _u64p]),
     "fb_tree_set_target_subset": (C.c_int, [C.c_void_p, _u64p, _sz]),

@@ -322,6 +322,10 @@ class FmmTree:
     def m2l_rank(self, level, ref):
         return self._lib.fb_tree_m2l_rank(self._h, level, ref)
 
+    def m2l_stream_warps(self):
+        """MMA warps of the streaming M2L kernel this tree runs (csrc/m2l.cu), 0 for the generic kernel"""
+        return self._lib.fb_tree_m2l_stream_warps(self._h)
+
     def m2l_operator(self, level, ref):
         r = self.m2l_rank(level, ref)
         P = self.info()["order"] ** self._dim

@@ -1620,6 +1620,10 @@ int fb_tree_m2l_rank(const fb_tree *t, int level, int ref) {
   return t->ops.m2l[level - 2][ref].rank;
 }
 
+int fb_m2l_stream_warps(int P, int compression) { return fb::m2l_stream_warps(P, compression); }
+
+int fb_tree_m2l_stream_warps(const fb_tree *t) { return t ? fb::m2l_stream_plan_warps(t->m2l_plan) : 0; }
+
 int fb_tree_m2l_operator(const fb_tree *t, int level, int ref, double *u_or_null, double *vt_or_null) {
   if (!t || level < 2 || level > t->ht.depth || ref < 0 || ref >= t->ops.n_ref) return FB_ERR_INVALID_ARGUMENT;
   const fb::M2LOperator &op = t->ops.m2l[level - 2][ref];

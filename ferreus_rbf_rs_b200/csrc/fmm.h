@@ -122,7 +122,9 @@ bool launch_l2p_fast(const TargetSet &ts, const int *leaf_cell, const double *lo
 // ---- M2L work lists, one group per (level, reference vector) -----------------------------------
 // m2l.cu: streaming M2L (TMA gathers / scatter-adds around register-resident operators); null plan = not applicable
 struct M2LStreamPlan;
-bool m2l_stream_supported(int P, int compression);
+int m2l_stream_warps(int P, int compression);  // MMA warps of the streaming kernel for P, 0 = generic kernel
+bool m2l_stream_supported(int P, int compression);  // the same, unless FB_M2L_STREAM=0 turns the stream off
+int m2l_stream_plan_warps(const M2LStreamPlan *plan);  // MMA warps the plan launches with, 0 for no plan
 M2LStreamPlan *m2l_stream_build(const HostTree &ht, const Operators &ops, int P, const int *d_inv_tab, cudaStream_t stream);
 struct M2LItemTable;  // work items restricted to the cells [level_lo, level_hi) of every level (a rank's share)
 M2LItemTable *m2l_stream_table_new(M2LStreamPlan *plan, int nrhs, const int *level_lo, const int *level_hi,

@@ -433,12 +433,19 @@ static int m2l_stream_warps(int P) {
   return 0;
 }
 
+// the dispatch rule alone (no environment override): uncompressed operators are never streamed
+int m2l_stream_warps(int P, int compression) {
+  if (compression == FB_COMPRESSION_NONE || P < 1) return 0;
+  return m2l_stream_warps(P);
+}
+
 bool m2l_stream_supported(int P, int compression) {
-  if (compression == FB_COMPRESSION_NONE) return false;
   if (const char *v = std::getenv("FB_M2L_STREAM"))
     if (v[0] == '0') return false;
-  return m2l_stream_warps(P) != 0;
+  return m2l_stream_warps(P, compression) != 0;
 }
+
+int m2l_stream_plan_warps(const M2LStreamPlan *p) { return p ? p->nw : 0; }
 
 void m2l_stream_free(M2LStreamPlan *p) { delete p; }
 

@@ -165,6 +165,13 @@ int fb_tree_dump_list(const fb_tree *t, int which, uint64_t *ptr, uint64_t *idx)
 int fb_tree_m2l_rank(const fb_tree *t, int level, int ref);
 /* dense copy of U (P x rank, column-major) / Vt (rank x P, column-major) */
 int fb_tree_m2l_operator(const fb_tree *t, int level, int ref, double *u_or_null, double *vt_or_null);
+/* which M2L kernel serves P = order^dim nodes per cell (host only): the number of MMA warps of the streaming kernel
+ * (csrc/m2l.cu), or 0 when the generic kernel does (uncompressed operators, or P outside the streaming windows).
+ * The environment variable FB_M2L_STREAM=0, read when a tree is built, is not consulted here.                    */
+int fb_m2l_stream_warps(int P, int compression_type);
+/* the same for a built tree: the MMA warps of the streaming plan it holds, 0 when it runs the generic kernel (its P
+ * is not served, FB_M2L_STREAM=0 at build time, depth < 2, or no V-list entries)                                  */
+int fb_tree_m2l_stream_warps(const fb_tree *t);
 
 
 /* ---- multi-GPU sharding by Morton-contiguous leaf ranges (SURVEY.md §8e) ---------------------------------
