@@ -418,7 +418,7 @@ int fb_tree_matvec_sharded(fb_tree *t) {
       sh.m2l_table = nullptr;
       sh.m2l_table = m2l_stream_table_new(t->m2l_plan, t->nrhs, sh.level_lo.data(), sh.level_hi.data(), s);
     }
-    t->downward(sh.ts.cell_flag, fuse ? &sh.ts : nullptr, true, false, sh.m2l_table);
+    t->downward(sh.ts.cell_flag, fuse ? &sh.ts : nullptr, true, sh.m2l_table);
     FB_CUDA(cudaEventRecord(sh.ev[2], s));
     FB_CUDA(cudaStreamWaitEvent(s, t->ev_join, 0));  // the near field joins in front of L2P (plain read-modify-write)
     if (t->timing) FB_CUDA(cudaEventRecord(t->ev[7], s));

@@ -226,8 +226,6 @@ void fb_tree::build(const double *points, size_t n_, int dim_, ptrdiff_t rs, ptr
     FB_CUDA(cudaStreamCreateWithPriority(&stream2, cudaStreamNonBlocking, prio_lo));
     FB_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
     FB_CUDA(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
-    const char *ov = std::getenv("FB_OVERLAP");
-    overlap_p2p = ov && ov[0] == '1';  // measured slower on B200 (15.1 vs 13.6 ms), kept as an opt-in experiment
   }
   for (auto &e : ev) FB_CUDA(cudaEventCreate(&e));
   for (auto &e : ev_mv) FB_CUDA(cudaEventCreate(&e));
@@ -558,10 +556,7 @@ void fb_tree::build(const double *points, size_t n_, int dim_, ptrdiff_t rs, ptr
     m2l_Pp = P4;
     while (m2l_Pp % 16 != 4 && m2l_Pp % 16 != 12) m2l_Pp += 4;  // bank-conflict-free B fragments
     m2l_nc = 0;
-    const char *nc_env = std::getenv("FB_M2L_NC");  // experiment knob: cap the column tile
-    const int nc_cap = nc_env ? std::atoi(nc_env) : 32;
-    for (int nc : {64, 32, 16, 8}) {  // columns per CTA: the largest tile that fits in shared memory
-      if (nc > nc_cap) continue;
+    for (int nc : {32, 16, 8}) {  // columns per CTA: the largest tile that fits in shared memory
       const size_t need = sizeof(double) * ((size_t)nc * m2l_Pp + (size_t)max_rp * (nc + 4));
       if (need <= 220 * 1024) {
         m2l_nc = nc;
@@ -655,8 +650,7 @@ void fb_tree::upward(const int *leaves, int n_leaves, const uint8_t *cell_flag) 
 }
 
 // -------------------------------------------------------------------------------------- downward
-void fb_tree::downward(const uint8_t *flags, const TargetSet *fuse_m2p, bool out_zeroed, bool m2l_one_cta_per_sm,
-                       const M2LItemTable *m2l_table) {
+void fb_tree::downward(const uint8_t *flags, const TargetSet *fuse_m2p, bool out_zeroed, const M2LItemTable *m2l_table) {
   const size_t nc = ht.ncells();
   const int p = order;
   d_loc.zero(nc * (size_t)nrhs * coef_stride(P), stream);
@@ -694,24 +688,19 @@ void fb_tree::downward(const uint8_t *flags, const TargetSet *fuse_m2p, bool out
       m2l_table_nrhs = nrhs;
     }
     const M2LGroupDev *tab = reinterpret_cast<const M2LGroupDev *>(d_m2l_table.p);
-    // sharing the SM with the concurrent P2P kernel: ask for more than half of the shared memory so that one CTA
-    // (half of the registers) is resident per SM and the P2P CTAs fit beside it
-    const size_t m2l_smem_launch = m2l_one_cta_per_sm ? std::max(m2l_smem, (size_t)116 * 1024) : m2l_smem;
 #define FB_M2L_LAUNCH(COMP, NCV)                                                                                   \
   do {                                                                                                             \
-    set_smem(k_m2l<COMP, NCV>, m2l_smem_launch);                                                                   \
-    FB_LAUNCH((k_m2l<COMP, NCV>), m2l_ctas, (NCV) == 64 ? 512 : 256, m2l_smem_launch, stream, tab, d_m2l_cta_group.p, d_m2l_tgt.p,   \
+    set_smem(k_m2l<COMP, NCV>, m2l_smem);                                                                          \
+    FB_LAUNCH((k_m2l<COMP, NCV>), m2l_ctas, 256, m2l_smem, stream, tab, d_m2l_cta_group.p, d_m2l_tgt.p,            \
               d_m2l_src.p, d_m2l_perm.p, d_oppool.p, d_perm_tab.p, d_inv_tab.p, P, m2l_P4, m2l_Pp, nrhs, flags,    \
               d_mult.p, d_loc.p);                                                                                  \
   } while (0)
     if (compressed) {
-      if (m2l_nc == 64) FB_M2L_LAUNCH(true, 64);
-      else if (m2l_nc == 32) FB_M2L_LAUNCH(true, 32);
+      if (m2l_nc == 32) FB_M2L_LAUNCH(true, 32);
       else if (m2l_nc == 16) FB_M2L_LAUNCH(true, 16);
       else FB_M2L_LAUNCH(true, 8);
     } else {
-      if (m2l_nc == 64) FB_M2L_LAUNCH(false, 64);
-      else if (m2l_nc == 32) FB_M2L_LAUNCH(false, 32);
+      if (m2l_nc == 32) FB_M2L_LAUNCH(false, 32);
       else if (m2l_nc == 16) FB_M2L_LAUNCH(false, 16);
       else FB_M2L_LAUNCH(false, 8);
     }
@@ -829,7 +818,6 @@ void fb_tree::leaf_pass(const TargetSet &ts, bool grads, bool m2p_done) {
   if (timing) FB_CUDA(cudaEventRecord(ev[8], stream));
   launch_p2p(ts, grads, m2p_done, stream, false);
   if (timing) FB_CUDA(cudaEventRecord(ev[9], stream));
-  last_overlapped = false;
 }
 
 // ----------------------------------------------------------------------------------- target sets
@@ -861,32 +849,8 @@ TargetSet fb_tree::source_target_set() {
 // targets = all sources: X is the transpose of W, so the P2L kernel applies the M2P half as well
 void fb_tree::evaluate_sources_fused(const TargetSet &ts) {
   const bool fuse = ht.adaptive && n_x_cells > 0 && ts.row_of_pos != nullptr;
-  if (!(fuse && overlap_p2p && !m2l_groups.empty())) {
-    downward(ts.cell_flag, fuse ? &ts : nullptr);
-    leaf_pass(ts, false, fuse);
-    return;
-  }
-  // Experiment (FB_OVERLAP=1): P2P needs only the sorted weights; M2L runs on the FP64 tensor pipe, P2P on the FP64
-  // FMA pipe, so the P2P kernel goes to a low-priority side stream and shares the SMs with M2L; its results and the
-  // fused M2P half are added with REDs, L2P joins last.  Result on B200: M2L at one CTA per SM (needed to leave
-  // registers for the P2P CTAs) slows from 2.9 to 4.8 ms and P2P then competes with the W/X pass for the FMA pipe:
-  // 15.1 ms against 13.6 ms for the serial order, so the serial order stays the default.
-  d_out.zero(ts.m * (size_t)nrhs, stream);
-  FB_CUDA(cudaEventRecord(ev_fork, stream));
-  FB_CUDA(cudaStreamWaitEvent(stream2, ev_fork, 0));
-  if (timing) FB_CUDA(cudaEventRecord(ev[10], stream2));
-  launch_p2p(ts, false, true, stream2, true);
-  if (timing) FB_CUDA(cudaEventRecord(ev[11], stream2));
-  FB_CUDA(cudaEventRecord(ev_join, stream2));
-  downward(ts.cell_flag, &ts, true, true);
-  FB_CUDA(cudaStreamWaitEvent(stream, ev_join, 0));
-  if (timing) FB_CUDA(cudaEventRecord(ev[7], stream));
-  launch_l2p(ts, false);
-  if (timing) {
-    FB_CUDA(cudaEventRecord(ev[8], stream));
-    FB_CUDA(cudaEventRecord(ev[9], stream));
-  }
-  last_overlapped = true;
+  downward(ts.cell_flag, fuse ? &ts : nullptr);
+  leaf_pass(ts, false, fuse);
 }
 
 // shared tail of bin_targets / subset_target_set: keys (leaf slot or sorted source position) -> TargetSet
@@ -1051,41 +1015,14 @@ TargetSet fb_tree::subset_target_set_dev(const unsigned long long *d_idx, size_t
 }
 
 // weights already in d_w_user: upward pass, downward pass restricted to the target set, leaf pass -> d_out.
-// The near-field pass (U lists) needs the sorted weights and nothing else: it is forked to the low-priority side stream
-// right away, so the upward pass — P2M plus one small, latency-bound M2M launch per level — runs beside it instead of in
-// front of it; the high-priority main stream's CTAs are placed ahead of the P2P kernel's pending ones.  Every writer of
-// the result rows adds with REDs until the two streams join in front of L2P.  On one GPU the whole matvec is bound by
-// the one FP64 pipe, so this only moves work around (measured 9.96 against 10.03 ms at the 1M-point headline) and it
-// blurs the per-stage times: opt-in with FB_NEAR_OVERLAP=1.  A rank's share of a partitioned tree (comm.cu), where the
-// upward pass is latency-bound and an all-reduce follows it, always runs this way.
+// On one GPU the stages run in order on one stream: the whole matvec is bound by the one FP64 pipe, so forking the
+// near field (P2P) to the side stream only moves work around (9.96 against 10.03 ms at the 1M-point headline on B200)
+// and blurs the per-stage times.  A rank's share of a partitioned tree (fb_tree_matvec_sharded), where the upward pass
+// is latency-bound and an all-reduce follows it, forks it.
 void fb_tree::matvec_dev(const TargetSet &ts) {
-  static const bool serial = [] {
-    const char *v = std::getenv("FB_NEAR_OVERLAP");
-    return !(v && v[0] == '1');
-  }();
   sort_weights();
-  if (serial) {
-    upward();
-    evaluate_sources_fused(ts);
-    return;
-  }
-  const bool fuse = ht.adaptive && n_x_cells > 0 && ts.row_of_pos != nullptr;
-  d_out.zero(ts.m * (size_t)nrhs, stream);  // in front of the fork: both streams add into it
-  FB_CUDA(cudaEventRecord(ev_fork, stream));
-  FB_CUDA(cudaStreamWaitEvent(stream2, ev_fork, 0));
-  if (timing) FB_CUDA(cudaEventRecord(ev[10], stream2));
-  launch_p2p(ts, false, true, stream2, true);  // U lists only
-  if (timing) FB_CUDA(cudaEventRecord(ev[11], stream2));
-  FB_CUDA(cudaEventRecord(ev_join, stream2));
   upward();
-  downward(ts.cell_flag, fuse ? &ts : nullptr, true);
-  FB_CUDA(cudaStreamWaitEvent(stream, ev_join, 0));
-  if (timing) FB_CUDA(cudaEventRecord(ev[7], stream));
-  launch_l2p(ts, false);
-  if (timing) FB_CUDA(cudaEventRecord(ev[8], stream));
-  if (!fuse && n_w_entries > 0) launch_p2p(ts, false, false, stream, false, true);  // W lists on their own
-  if (timing) FB_CUDA(cudaEventRecord(ev[9], stream));
-  last_overlapped = true;
+  evaluate_sources_fused(ts);
 }
 
 void fb_tree::fetch_output(size_t m, bool grads, double *out_vals, double *out_grads, ptrdiff_t o_rs,
@@ -1160,7 +1097,7 @@ static void collect_timing(fb_tree *t) {
   t->last_ms[3] = ms(4, 5);  // p2l
   t->last_ms[4] = ms(5, 6);  // l2l
   t->last_ms[5] = ms(7, 8);  // l2p
-  t->last_ms[6] = t->last_overlapped ? ms(10, 11) : ms(8, 9);  // p2p (+ m2p); overlapped: its own span on the side stream
+  t->last_ms[6] = ms(8, 9);  // p2p (+ m2p)
   t->last_ms[7] = ms(0, 9);  // total
 }
 

@@ -151,9 +151,10 @@ void fb_shard_free(fb_shard *s);
 struct fb_tree {
   int device = 0;
   cudaStream_t stream = nullptr;
-  cudaStream_t stream2 = nullptr;  // low-priority side stream: P2P (FP64 FMA pipe) under M2L (FP64 tensor pipe)
+  // low-priority side stream: the near field (P2P) of a rank's share of a partitioned tree, beside the upward pass,
+  // the multipole all-reduce and the downward pass on `stream` (fb_tree_matvec_sharded)
+  cudaStream_t stream2 = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  bool overlap_p2p = false;
   int dim = 3, order = 0, P = 0;
   size_t n = 0;
   int nrhs = 1;
@@ -188,7 +189,6 @@ struct fb_tree {
   std::vector<std::vector<int>> h_parents;    // per level: non-leaf cells
   fb::DBuf<int> d_parents;                    // concatenated, offsets in parents_off
   std::vector<int> parents_off;
-  fb::DBuf<int> d_level_cells;                // cells level-major == identity, kept for clarity
   // lists
   fb::DBuf<long long> d_u_ptr, d_w_ptr, d_x_ptr, d_w_ptr_none;
   fb::DBuf<int> d_u_begin, d_u_count, d_w_cell, d_x_begin, d_x_count, d_x_cells;
@@ -232,7 +232,6 @@ struct fb_tree {
   bool timing = false;
   double last_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   cudaEvent_t ev[12] = {};
-  bool last_overlapped = false;
   cudaEvent_t ev_mv[2] = {};
   double last_matvec_ms = 0;
 
@@ -248,7 +247,7 @@ struct fb_tree {
   // fuse_m2p: the P2L kernel also applies the M2P transpose for that target set (ts.row_of_pos != null) into d_out
   // (zeroed here); leaf_pass(ts, false, m2p_done = true) must follow
   void downward(const uint8_t *flags, const fb::TargetSet *fuse_m2p = nullptr, bool out_zeroed = false,
-                bool m2l_one_cta_per_sm = false, const fb::M2LItemTable *m2l_table = nullptr);
+                const fb::M2LItemTable *m2l_table = nullptr);
   void leaf_pass(const fb::TargetSet &ts, bool grads, bool m2p_done = false);
   void launch_l2p(const fb::TargetSet &ts, bool grads);
   // m2p_done: the W lists are (or will be) applied elsewhere; w_only: the U lists are

@@ -403,7 +403,7 @@ struct M2LGroupDev {  // one (level, reference vector) group of the fused M2L la
 };
 
 template <bool COMPRESSED, int NC>
-__global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(const M2LGroupDev *groups, const int *cta_group, const int *e_tgt_all,
+__global__ void __launch_bounds__(256, NC == 32 ? 2 : 1) k_m2l(const M2LGroupDev *groups, const int *cta_group, const int *e_tgt_all,
                                                 const int *e_src_all, const int *e_perm_all, const double *pool,
                                                 const int *perm_tab, const int *inv_tab, int P, int P4, int Pp, int nrhs,
                                                 const uint8_t *flag, const double *mult, double *loc) {
@@ -418,8 +418,7 @@ __global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const size_t ncols = n_entries * (size_t)nrhs;
   constexpr int kM2LCols = NC, kM2LColsPad = NC + 4;
-  constexpr int NW = NC == 64 ? 16 : 8;  // warps per CTA (NC = 64: one 512-thread CTA per SM, operator fragments re-read half as often)
-  constexpr int NH = (NC + 31) / 32;     // 32-column halves, each with its own run table
+  constexpr int NW = 8;              // warps per CTA
   constexpr int kNT = NC / 8;        // 8-column tiles
   const size_t col0 = (size_t)cta * kM2LCols;
   const int nc = (int)min((size_t)kM2LCols, ncols - col0);
@@ -427,7 +426,7 @@ __global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(
   double *Ys = Xs + (size_t)kM2LCols * Pp;                // [rank_pad][NC + 4]
   __shared__ int s_tgt[kM2LCols], s_rhs[kM2LCols], s_perm[kM2LCols], s_src[kM2LCols];
   __shared__ int s_list[kM2LCols], s_off[kM2LCols], s_len[kM2LCols];  // columns grouped by (target, rhs) run
-  __shared__ int s_runs[kM2LCols], s_nruns[NH];                      // first column of every run, per half
+  __shared__ int s_runs[kM2LCols], s_nruns;                          // first column of every run, number of runs
   __shared__ int s_any;
   if (tid == 0) s_any = 0;
   __syncthreads();
@@ -449,11 +448,10 @@ __global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(
   }
   __syncthreads();
   if (!s_any) return;
-  if (warp < NH) {
+  if (warp == 0) {
     // runs of columns that add into the same (target, rhs): s_list holds the columns run by run; the first column
-    // of a run carries the run's offset and length, every other column length 0.  One warp per 32-column half; a run
-    // that crosses the halves is flushed as two
-    const int hb = warp * 32, col = hb + lane;
+    // of a run carries the run's offset and length, every other column length 0
+    const int col = lane;
     const bool valid = col < kM2LCols && s_tgt[col] >= 0;
     const int key = valid ? s_tgt[col] * nrhs + s_rhs[col] : -(lane + 1);
     const unsigned same = __match_any_sync(0xffffffffu, key);
@@ -468,12 +466,12 @@ __global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(
     const bool is_first = valid && first == lane;
     const unsigned firsts = __ballot_sync(0xffffffffu, is_first);
     if (col < kM2LCols) {
-      if (valid) s_list[hb + before + rank_in_run] = col;
-      s_off[col] = hb + before;
+      if (valid) s_list[before + rank_in_run] = col;
+      s_off[col] = before;
       s_len[col] = is_first ? __popc(same) : 0;
-      if (is_first) s_runs[hb + __popc(firsts & ((1u << lane) - 1u))] = col;
+      if (is_first) s_runs[__popc(firsts & ((1u << lane) - 1u))] = col;
     }
-    if (lane == 0) s_nruns[warp] = __popc(firsts);
+    if (lane == 0) s_nruns = __popc(firsts);
   }
   // stage permuted multipoles (zero padding up to P4 and for idle columns); 4 gathers in flight per lane
   for (int c = warp; c < kM2LCols; c += NW) {
@@ -599,11 +597,10 @@ __global__ void __launch_bounds__(NC == 64 ? 512 : 256, NC == 32 ? 2 : 1) k_m2l(
   __syncthreads();
   // ---- flush: L_tgt[i] += sum_{c in run} Zs[c][inv_perm_c[i]]; four gathers in flight per lane
   const int nchunks = (P + 31) >> 5;
-  const int nruns0 = s_nruns[0], nruns = nruns0 + (NH > 1 ? s_nruns[NH - 1] : 0);
-  const int nitems = nruns * nchunks;  // (run, 32-node chunk) pairs, dealt round-robin to the warps
+  const int nitems = s_nruns * nchunks;  // (run, 32-node chunk) pairs, dealt round-robin to the warps
   for (int item = warp; item < nitems; item += NW) {
     const int run = item / nchunks, i = (item - run * nchunks) * 32 + lane;
-    const int c0 = run < nruns0 ? s_runs[run] : s_runs[32 + run - nruns0];
+    const int c0 = s_runs[run];
     const int len = s_len[c0];
     const int *lst = s_list + s_off[c0];
     if (i < P) {

@@ -355,172 +355,31 @@ __global__ void __launch_bounds__(256) k_chol_big_update(double *A, int n, int k
   chol_update_column(A, n, kb, bs, jb, Pj, Pi, ib, n);  // at most one i tile per warp
 }
 
-// Domain::solve (domain.rs:393-467) + scatter of schwarz.rs:94-155, one CTA of kSolveThreads threads per domain.
+// ---- Domain::solve (domain.rs:393-467) + scatter of schwarz.rs:94-155, one CTA of kSolveThreads threads per domain
 //   mode 0: fine level — write internal points only;  mode 1: coarse — write all points (+ polynomial tail)
-// The two substitutions are chains of 2 x mm / 32 dependent block steps; a step is a row-block x vector product (read
-// straight from HBM) and a 32 x 32 triangular solve.  With 8 warps a step took ~30 us (four rows per warp, one after the
-// other) and a 978-point domain 2 ms — 6.4 ms for the 2048-domain level against 1.2 ms of factor streaming; 32 warps
-// give every row of the block its own warp and four independent partial sums per lane.
-constexpr int kSolveThreads = 1024;
-constexpr int kSolveWarps = kSolveThreads / 32;
-__global__ void __launch_bounds__(kSolveThreads) k_dom_solve(DomainTable t, const double *qpool, const double *lpool,
-                                                             const double *res, double *out, int mode, int add_poly,
-                                                             const double *a_special, const double *sp_inv,
-                                                             size_t n_total, int basis) {
-  const int d = blockIdx.x;
-  const int rk = t.rank[d];
-  const long long p0 = t.pt_ptr[d];
-  const int n = (int)(t.pt_ptr[d + 1] - p0), mm = n - rk;
-  const int *idx = t.pt_idx + p0;
-  const uint8_t *mask = t.pt_mask + p0;
-  const double *Q = qpool + t.q_off[d];
-  const double *L = lpool + t.l_off[d];
-  extern __shared__ double sm[];
-  double *dv = sm;        // n gathered residuals
-  double *x = dv + n;     // mm rhs / solution
-  double *red = x + mm;   // kSolveWarps x 32 partial sums
-  double *top = red + kSolveWarps * 32;  // rk
-  __shared__ double Dg[32][33];          // the diagonal block of the current step (lower triangle)
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int i = tid; i < n; i += kSolveThreads) dv[i] = res[idx[i]];
-  __syncthreads();
-  for (int j = tid; j < mm; j += kSolveThreads) {  // rhs = Q^T d_special + d_rest
-    double v = dv[rk + j];
-    for (int a = 0; a < rk; ++a) v += Q[(size_t)a * mm + j] * dv[a];
-    x[j] = v;
-  }
-  __syncthreads();
-  const bool inverse = t.use_inverse != nullptr && t.use_inverse[d] != 0;
-  if (inverse) {
-    // Cholesky failed for this domain (Q^T A Q indefinite; domain.rs:63-68 falls back to a pivoted factorisation): the
-    // slot holds the explicit inverse, gamma = Inv rhs.  d_rest (dv[rk..n)) is dead once rhs is formed: it takes gamma
-    for (int r = warp; r < mm; r += kSolveWarps) {
-      const double *row = L + (size_t)r * mm;
-      double sacc = 0.0;
-      for (int c = lane; c < mm; c += 32) sacc += row[c] * x[c];
-      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-      if (lane == 0) dv[rk + r] = sacc;
-    }
-    __syncthreads();
-    for (int j = tid; j < mm; j += kSolveThreads) x[j] = dv[rk + j];
-    __syncthreads();
-  }
-  // forward substitution L y = rhs: row r of the block belongs to warp r
-  for (int kb = 0; !inverse && kb < mm; kb += 32) {
-    const int bs = min(32, mm - kb);
-    if (warp < bs) {
-      const double *row = L + (size_t)(kb + warp) * mm;
-      double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
-      int c = lane;
-      for (; c + 96 < kb; c += 128) {
-        s0 += row[c] * x[c];
-        s1 += row[c + 32] * x[c + 32];
-        s2 += row[c + 64] * x[c + 64];
-        s3 += row[c + 96] * x[c + 96];
-      }
-      for (; c < kb; c += 32) s0 += row[c] * x[c];
-      Dg[warp][lane] = lane <= warp ? row[kb + lane] : 0.0;  // the block's own triangle, staged for the serial part
-      double sacc = (s0 + s1) + (s2 + s3);
-      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-      if (lane == 0) red[warp] = sacc;
-    }
-    __syncthreads();
-    if (warp == 0) {
-      double v = lane < bs ? x[kb + lane] - red[lane] : 0.0;
-      for (int k = 0; k < bs; ++k) {
-        const double piv = __shfl_sync(0xffffffffu, v, k) / Dg[k][k];
-        if (lane == k) v = piv;
-        if (lane > k && lane < bs) v -= Dg[lane][k] * piv;
-      }
-      if (lane < bs) x[kb + lane] = v;
-    }
-    __syncthreads();
-  }
-  // backward substitution L^T gamma = y
-  for (int kb = ((mm - 1) / 32) * 32; !inverse && kb >= 0; kb -= 32) {
-    const int bs = min(32, mm - kb);
-    double sacc = 0.0;
-    if (lane < bs) {
-      double s0 = 0.0, s1 = 0.0;
-      int j = kb + bs + warp;
-      for (; j + kSolveWarps < mm; j += 2 * kSolveWarps) {
-        s0 += L[(size_t)j * mm + kb + lane] * x[j];
-        s1 += L[(size_t)(j + kSolveWarps) * mm + kb + lane] * x[j + kSolveWarps];
-      }
-      if (j < mm) s0 += L[(size_t)j * mm + kb + lane] * x[j];
-      sacc = s0 + s1;
-    }
-    red[warp * 32 + lane] = sacc;
-    if (warp < bs) Dg[warp][lane] = lane <= warp ? L[(size_t)(kb + warp) * mm + kb + lane] : 0.0;
-    __syncthreads();
-    if (warp == 0) {
-      double acc = 0.0;
-      for (int w = 0; w < kSolveWarps; ++w) acc += red[w * 32 + lane];
-      double v = lane < bs ? x[kb + lane] - acc : 0.0;
-      for (int k = bs - 1; k >= 0; --k) {
-        const double piv = __shfl_sync(0xffffffffu, v, k) / Dg[k][k];
-        if (lane == k) v = piv;
-        if (lane < k) v -= Dg[k][lane] * piv;
-      }
-      if (lane < bs) x[kb + lane] = v;
-    }
-    __syncthreads();
-  }
-  // lambda_top = Q gamma
-  for (int a = warp; a < rk; a += kSolveWarps) {
-    double sacc = 0.0;
-    for (int j = lane; j < mm; j += 32) sacc += Q[(size_t)a * mm + j] * x[j];
-    for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-    if (lane == 0) top[a] = sacc;
-  }
-  __syncthreads();
-  for (int i = tid; i < n; i += kSolveThreads) {
-    const double lam = i < rk ? top[i] : x[i - rk];
-    if (mode == 1 || mask[i]) out[idx[i]] = lam;
-  }
-  if (mode == 1 && add_poly && rk > 0 && a_special) {
-    // r = d_special - A_special lambda;  poly = sp_mono^-1 r  (domain.rs:446-463)
-    __syncthreads();
-    for (int a = warp; a < rk; a += kSolveWarps) {
-      const double *row = a_special + (size_t)a * n;
-      double sacc = 0.0;
-      for (int i = lane; i < n; i += 32) sacc += row[i] * (i < rk ? top[i] : x[i - rk]);
-      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-      if (lane == 0) red[a] = dv[a] - sacc;
-    }
-    __syncthreads();
-    if (tid < rk) {
-      double sacc = 0.0;
-      for (int b = 0; b < rk; ++b) sacc += sp_inv[tid * rk + b] * red[b];
-      out[n_total - rk + tid] = sacc;  // schwarz.rs:147-152: tail rows
-    }
-  }
-}
-
-// ---- Domain::solve, second form ------------------------------------------------------------------------------------
-// ncu on k_dom_solve at the 1M-point fit (2048 domains of ~980 points): 7.0 ms per launch for 15.7 GB of factor reads
-// (2.4 ms at the HBM peak).  The time went into what sits between the loads: per 32-row step a serial substitution with
-// 32 dependent divisions on one warp, and in the backward pass a column-block walk (256 B out of every 7.8 KB row).
-// This form removes both:
+// The two substitutions are chains of 2 x mm / 32 dependent block steps over the lower triangle of L, streamed from HBM
+// row block by row block.  What sits between the loads is kept off the critical path:
 //   * the 32 x 32 diagonal blocks of L are inverted in place once, at setup (k_inv_diag_inplace), so a block step is a
 //     32-lane dot product per row, all 32 warps at once, no division, no dependency chain;
+//   * the forward substitution is left-looking: every row of the block has its own warp and four independent partial
+//     sums per lane;
 //   * the backward substitution is right-looking: as soon as the 32 values of a block are known, every thread subtracts
-//     their contribution from ITS column of the right-hand side — 32 independent, row-contiguous loads per thread — so
-//     both passes stream the lower triangle of L row block by row block.
-__global__ void k_inv_diag_inplace(DomainTable t, double *lpool) {
-  const int d = blockIdx.x;
-  const int mm = (int)(t.pt_ptr[d + 1] - t.pt_ptr[d]) - t.rank[d];
-  const int kb = blockIdx.y * kNB;
-  if (kb >= mm) return;
-  const int bs = min(kNB, mm - kb), lane = threadIdx.x;
-  double *L = lpool + t.l_off[d];
+//     their contribution from ITS column of the right-hand side — 32 independent, row-contiguous loads per thread —
+//     instead of walking a column block (256 B out of every 7.8 KB row).
+constexpr int kSolveThreads = 1024;
+constexpr int kSolveWarps = kSolveThreads / 32;
+
+// A^-1 of the lower-triangular bs x bs block A (row stride ld, bs <= kNB) into the lower triangle of Ainv, which may be
+// A itself; one warp, lane c forms column c by forward substitution.  The strict upper triangle of Ainv is not written.
+__device__ __forceinline__ void tri_inv_block(const double *A, size_t ld, int bs, double *Ainv) {
+  const int lane = threadIdx.x;
   __shared__ double D[kNB][kNB + 1];
-  for (int r = 0; r < bs; ++r) D[r][lane] = (lane < bs && lane <= r) ? L[(size_t)(kb + r) * mm + kb + lane] : 0.0;
+  for (int r = 0; r < bs; ++r) D[r][lane] = (lane < bs && lane <= r) ? A[(size_t)r * ld + lane] : 0.0;
   __syncwarp();
   double x[kNB];
 #pragma unroll
   for (int r = 0; r < kNB; ++r) x[r] = 0.0;
-  if (lane < bs) {  // column `lane` of the inverse by forward substitution
+  if (lane < bs) {
 #pragma unroll
     for (int r = 0; r < kNB; ++r) {
       if (r < bs && r >= lane) {
@@ -532,17 +391,69 @@ __global__ void k_inv_diag_inplace(DomainTable t, double *lpool) {
       }
     }
   }
+  // a lane reads and writes only its own column; this fence keeps ptxas from scheduling the stores into the
+  // substitution, which takes the in-place kernel from 90 to 117 registers
   __syncwarp();
   if (lane < bs)
 #pragma unroll
     for (int r = 0; r < kNB; ++r)
-      if (r < bs && r >= lane) L[(size_t)(kb + r) * mm + kb + lane] = x[r];
+      if (r < bs && r >= lane) Ainv[(size_t)r * ld + lane] = x[r];
 }
 
-__global__ void __launch_bounds__(kSolveThreads) k_dom_solve_v2(DomainTable t, const double *qpool, const double *lpool,
-                                                                const double *res, double *out, int mode, int add_poly,
-                                                                const double *a_special, const double *sp_inv,
-                                                                size_t n_total) {
+__global__ void k_inv_diag_inplace(DomainTable t, double *lpool) {
+  const int d = blockIdx.x;
+  const int mm = (int)(t.pt_ptr[d + 1] - t.pt_ptr[d]) - t.rank[d];
+  const int kb = blockIdx.y * kNB;
+  if (kb >= mm) return;
+  double *blk = lpool + t.l_off[d] + (size_t)kb * mm + kb;
+  tri_inv_block(blk, mm, min(kNB, mm - kb), blk);
+}
+
+// The end of Domain::solve (domain.rs:434-463) and its scatter, for one domain on one CTA of kSolveThreads threads:
+// lambda = [Q gamma; gamma] goes to out[idx] (mode 1: every point; mode 0: the internal ones), and in mode 1 the
+// polynomial tail follows: r = d_special - A_special lambda, poly = sp_mono^-1 r.  Every dot product is one warp per
+// row, lane-strided, reduced with __shfl_down to lane 0.  d_special: the rk residuals at the special points; top and
+// red: shared scratch of rk doubles each (red may be d_special itself: an entry is read before it is overwritten).
+__device__ __forceinline__ void dom_solve_finish(const double *Q, const double *gamma, const double *d_special,
+                                                 const int *idx, const uint8_t *mask, int n, int rk, int mode,
+                                                 int add_poly, const double *a_special, const double *sp_inv,
+                                                 size_t n_total, double *top, double *red, double *out) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int mm = n - rk;
+  // lambda_top = Q gamma
+  for (int a = warp; a < rk; a += kSolveWarps) {
+    double sacc = 0.0;
+    for (int j = lane; j < mm; j += 32) sacc += Q[(size_t)a * mm + j] * gamma[j];
+    for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
+    if (lane == 0) top[a] = sacc;
+  }
+  __syncthreads();
+  for (int i = tid; i < n; i += kSolveThreads) {
+    const double lam = i < rk ? top[i] : gamma[i - rk];
+    if (mode == 1 || mask[i]) out[idx[i]] = lam;
+  }
+  if (mode == 1 && add_poly && rk > 0 && a_special) {
+    __syncthreads();
+    for (int a = warp; a < rk; a += kSolveWarps) {
+      const double *row = a_special + (size_t)a * n;
+      double sacc = 0.0;
+      for (int i = lane; i < n; i += 32) sacc += row[i] * (i < rk ? top[i] : gamma[i - rk]);
+      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
+      if (lane == 0) red[a] = d_special[a] - sacc;
+    }
+    __syncthreads();
+    if (tid < rk) {
+      double sacc = 0.0;
+      for (int b = 0; b < rk; ++b) sacc += sp_inv[tid * rk + b] * red[b];
+      out[n_total - rk + tid] = sacc;  // schwarz.rs:147-152: tail rows
+    }
+  }
+}
+
+__global__ void __launch_bounds__(kSolveThreads) k_dom_solve(DomainTable t, const double *qpool, const double *lpool,
+                                                             const double *res, double *out, int mode, int add_poly,
+                                                             const double *a_special, const double *sp_inv,
+                                                             size_t n_total) {
   const int d = blockIdx.x;
   const int rk = t.rank[d];
   const long long p0 = t.pt_ptr[d];
@@ -567,7 +478,9 @@ __global__ void __launch_bounds__(kSolveThreads) k_dom_solve_v2(DomainTable t, c
   }
   __syncthreads();
   const bool inverse = t.use_inverse != nullptr && t.use_inverse[d] != 0;
-  if (inverse) {  // indefinite fallback: the slot holds the explicit inverse (see k_dom_solve)
+  if (inverse) {
+    // Cholesky failed for this domain (Q^T A Q indefinite; domain.rs:63-68 falls back to a pivoted factorisation): the
+    // slot holds the explicit inverse, gamma = Inv rhs.  d_rest (dv[rk..n)) is dead once rhs is formed: it takes gamma
     for (int r = warp; r < mm; r += kSolveWarps) {
       const double *row = L + (size_t)r * mm;
       double sacc = 0.0;
@@ -633,65 +546,19 @@ __global__ void __launch_bounds__(kSolveThreads) k_dom_solve_v2(DomainTable t, c
     }
     __syncthreads();
   }
-  // lambda_top = Q gamma
-  for (int a = warp; a < rk; a += kSolveWarps) {
-    double sacc = 0.0;
-    for (int j = lane; j < mm; j += 32) sacc += Q[(size_t)a * mm + j] * x[j];
-    for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-    if (lane == 0) top[a] = sacc;
-  }
-  __syncthreads();
-  for (int i = tid; i < n; i += kSolveThreads) {
-    const double lam = i < rk ? top[i] : x[i - rk];
-    if (mode == 1 || mask[i]) out[idx[i]] = lam;
-  }
-  if (mode == 1 && add_poly && rk > 0 && a_special) {
-    // r = d_special - A_special lambda;  poly = sp_mono^-1 r  (domain.rs:446-463)
-    __syncthreads();
-    for (int a = warp; a < rk; a += kSolveWarps) {
-      const double *row = a_special + (size_t)a * n;
-      double sacc = 0.0;
-      for (int i = lane; i < n; i += 32) sacc += row[i] * (i < rk ? top[i] : x[i - rk]);
-      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-      if (lane == 0) red[a] = dv[a] - sacc;
-    }
-    __syncthreads();
-    if (tid < rk) {
-      double sacc = 0.0;
-      for (int b = 0; b < rk; ++b) sacc += sp_inv[tid * rk + b] * red[b];
-      out[n_total - rk + tid] = sacc;  // schwarz.rs:147-152: tail rows
-    }
-  }
+  dom_solve_finish(Q, x, dv, idx, mask, n, rk, mode, add_poly, a_special, sp_inv, n_total, top, red, out);
 }
 
 // ---- the single coarse domain (n ~ 2000) -----------------------------------------------------------------------------
-// k_dom_solve gives a domain one CTA: its two substitutions are chains of 2 x mm / 32 dependent steps, 3.5 ms for the
-// coarse domain of the 1M-point fit, three times per preconditioner cycle.  For a one-domain level the triangular factor
-// is inverted once at setup (X = L^-1, kept with its transpose), and Domain::solve becomes two triangular matrix-vector
-// products spread over the whole GPU:  gamma = X^T (X rhs)  — the same L^-T L^-1 rhs, a few rounding errors apart.
+// One CTA per domain leaves the two substitutions of the coarse domain as chains of 2 x mm / 32 dependent steps on one SM:
+// 3.5 ms for the coarse domain of the 1M-point fit with the first form of k_dom_solve (since removed), three times per
+// preconditioner cycle.  For a one-domain level the triangular factor is inverted once at setup (X = L^-1, kept with its
+// transpose), and Domain::solve becomes two triangular matrix-vector products spread over the whole GPU:
+// gamma = X^T (X rhs)  — the same L^-T L^-1 rhs, a few rounding errors apart.
 __global__ void k_tri_inv_diag(const double *L, int n, double *X) {  // X[kb.., kb..] = L[kb.., kb..]^-1, one warp per block
-  const int kb = blockIdx.x * kNB, bs = min(kNB, n - kb), lane = threadIdx.x;
-  __shared__ double D[kNB][kNB + 1];
-  for (int r = 0; r < bs; ++r) D[r][lane] = (lane < bs && lane <= r) ? L[(size_t)(kb + r) * n + kb + lane] : 0.0;
-  __syncwarp();
-  if (lane < bs) {  // column `lane` of the inverse by forward substitution
-    double x[kNB];
-#pragma unroll
-    for (int r = 0; r < kNB; ++r) x[r] = 0.0;
-#pragma unroll
-    for (int r = 0; r < kNB; ++r) {
-      if (r < bs && r >= lane) {
-        double v = r == lane ? 1.0 : 0.0;
-#pragma unroll
-        for (int k = 0; k < kNB; ++k)
-          if (k < r && k >= lane) v -= D[r][k] * x[k];
-        x[r] = v / D[r][r];
-      }
-    }
-#pragma unroll
-    for (int r = 0; r < kNB; ++r)
-      if (r < bs) X[(size_t)(kb + r) * n + kb + lane] = r >= lane ? x[r] : 0.0;
-  }
+  const int kb = blockIdx.x * kNB;
+  const size_t off = (size_t)kb * n + kb;
+  tri_inv_block(L + off, n, min(kNB, n - kb), X + off);  // the strict upper triangle of X is zeroed beforehand
 }
 
 // block column j of X = L^-1 below the diagonal, one CTA per block column:  X_ij = -X_ii sum_{k=j}^{i-1} L_ik X_kj
@@ -783,39 +650,18 @@ __global__ void __launch_bounds__(256) k_tri_gemv(const double *M, int n, const 
   if (lane == 0) y[r] = sacc;
 }
 
-// lambda_top = Q gamma, scatter, polynomial tail (the end of k_dom_solve for the coarse domain), one CTA
-__global__ void __launch_bounds__(1024) k_big_finish(DomainTable t, const double *qpool, const double *gamma,
-                                                     const double *res, double *out, int add_poly,
-                                                     const double *a_special, const double *sp_inv, size_t n_total) {
+// lambda_top = Q gamma, scatter, polynomial tail of the coarse domain, one CTA (the end of k_dom_solve)
+__global__ void __launch_bounds__(kSolveThreads) k_big_finish(DomainTable t, const double *qpool, const double *gamma,
+                                                              const double *res, double *out, int mode, int add_poly,
+                                                              const double *a_special, const double *sp_inv,
+                                                              size_t n_total) {
+  const long long p0 = t.pt_ptr[0];
   const int rk = t.rank[0];
-  const int n = (int)(t.pt_ptr[1] - t.pt_ptr[0]), mm = n - rk;
-  const int *idx = t.pt_idx + t.pt_ptr[0];
-  const double *Q = qpool + t.q_off[0];
+  const int *idx = t.pt_idx + p0;
   __shared__ double top[16], red[16];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int a = warp; a < rk; a += 32) {
-    double sacc = 0.0;
-    for (int j = lane; j < mm; j += 32) sacc += Q[(size_t)a * mm + j] * gamma[j];
-    for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-    if (lane == 0) top[a] = sacc;
-  }
-  __syncthreads();
-  for (int i = tid; i < n; i += 1024) out[idx[i]] = i < rk ? top[i] : gamma[i - rk];
-  if (add_poly && rk > 0 && a_special) {  // r = d_special - A_special lambda;  poly = sp_mono^-1 r  (domain.rs:446-463)
-    for (int a = warp; a < rk; a += 32) {
-      const double *row = a_special + (size_t)a * n;
-      double sacc = 0.0;
-      for (int i = lane; i < n; i += 32) sacc += row[i] * (i < rk ? top[i] : gamma[i - rk]);
-      for (int o = 16; o > 0; o >>= 1) sacc += __shfl_down_sync(0xffffffffu, sacc, o);
-      if (lane == 0) red[a] = res[idx[a]] - sacc;
-    }
-    __syncthreads();
-    if (tid < rk) {
-      double sacc = 0.0;
-      for (int b = 0; b < rk; ++b) sacc += sp_inv[tid * rk + b] * red[b];
-      out[n_total - rk + tid] = sacc;  // schwarz.rs:147-152: tail rows
-    }
-  }
+  if ((int)threadIdx.x < rk) red[threadIdx.x] = res[idx[threadIdx.x]];  // d_special
+  dom_solve_finish(qpool + t.q_off[0], gamma, red, idx, t.pt_mask + p0, (int)(t.pt_ptr[1] - p0), rk, mode, add_poly,
+                   a_special, sp_inv, n_total, top, red, out);
 }
 
 // A[special, :] rows of the coarse domain (domain.rs:366)
@@ -841,7 +687,6 @@ struct LevelDev {
   // one-domain level: X = L^-1 and its transpose (row-major mm x mm), vectors of the spread solve
   bool big_inverse = false;
   DBuf<double> linv, linv_t, big_v;
-  bool diag_inverted = false;  // the 32 x 32 diagonal blocks of every factor hold their inverses (k_dom_solve_v2)
   DBuf<uint8_t> fail;         // per domain: Cholesky met a non-positive pivot
   std::vector<int> h_mms;     // order of every domain's Q^T A Q (host copy, for the fallback)
   std::vector<long long> h_l_off;
@@ -1019,7 +864,6 @@ struct DeviceSolver {
       FB_LAUNCH(k_cholesky, (unsigned)nd, 256, smem, stream, lv.tab, lv.lpool.p, lv.fail.p);
       FB_LAUNCH(k_inv_diag_inplace, dim3((unsigned)nd, (unsigned)((lv.max_mm + kNB - 1) / kNB)), 32, 0, stream, lv.tab,
                 lv.lpool.p);
-      lv.diag_inverted = true;
     }
   }
 
@@ -1196,13 +1040,15 @@ struct DeviceSolver {
   }
 
   void solve_level(const LevelDev &lv, const double *res, double *out, int mode, int add_poly, cudaStream_t stream) {
-    if (lv.big_inverse && lv.n_fallback == 0 && mode == 1) {  // the coarse domain, spread over the GPU
+    // the coarse domain, spread over the GPU.  Fine levels come from bisection in pairs of domains, so a one-domain
+    // level is the coarse level or a naive / dense solve: always solved in mode 1
+    if (lv.big_inverse && lv.n_fallback == 0) {
       const int mm = (int)lv.max_mm;
       double *rhs = lv.big_v.p, *y = rhs + mm, *gamma = y + mm;
       FB_LAUNCH(k_big_rhs, nblk(mm, 256), 256, 0, stream, lv.tab, lv.qpool.p, res, rhs);
       FB_LAUNCH((k_tri_gemv<true>), (unsigned)((mm + 7) / 8), 256, 0, stream, lv.linv.p, mm, rhs, y);
       FB_LAUNCH((k_tri_gemv<false>), (unsigned)((mm + 7) / 8), 256, 0, stream, lv.linv_t.p, mm, y, gamma);
-      FB_LAUNCH(k_big_finish, 1, 1024, 0, stream, lv.tab, lv.qpool.p, gamma, res, out, add_poly,
+      FB_LAUNCH(k_big_finish, 1, kSolveThreads, 0, stream, lv.tab, lv.qpool.p, gamma, res, out, mode, add_poly,
                 lv.solve_for_poly ? lv.a_special.p : nullptr, lv.solve_for_poly ? lv.sp_inv.p : nullptr, nt);
       return;
     }
@@ -1213,18 +1059,9 @@ struct DeviceSolver {
                   "a subdomain of " + std::to_string(lv.max_n) + " points exceeds the shared-memory budget of the batched "
                   "subdomain solve (about 14300 points per domain): lower naive_solve_threshold / "
                   "DDMParams.coarse_threshold / DDMParams.leaf_threshold below that");
-    if (lv.diag_inverted) {
-      FB_CUDA(cudaFuncSetAttribute(k_dom_solve_v2, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                   (int)std::max<size_t>(smem, 1024)));
-      FB_LAUNCH(k_dom_solve_v2, (unsigned)lv.n_domains, kSolveThreads, smem, stream, lv.tab, lv.qpool.p, lv.lpool.p, res,
-                out, mode, add_poly, lv.solve_for_poly ? lv.a_special.p : nullptr,
-                lv.solve_for_poly ? lv.sp_inv.p : nullptr, nt);
-      return;
-    }
     FB_CUDA(cudaFuncSetAttribute(k_dom_solve, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<size_t>(smem, 1024)));
     FB_LAUNCH(k_dom_solve, (unsigned)lv.n_domains, kSolveThreads, smem, stream, lv.tab, lv.qpool.p, lv.lpool.p, res, out, mode,
-              add_poly, lv.solve_for_poly ? lv.a_special.p : nullptr, lv.solve_for_poly ? lv.sp_inv.p : nullptr, nt,
-              (int)m);
+              add_poly, lv.solve_for_poly ? lv.a_special.p : nullptr, lv.solve_for_poly ? lv.sp_inv.p : nullptr, nt);
   }
 
   // ---- vector helpers (device scalars are read back: Givens rotations stay on the host)
@@ -2076,9 +1913,10 @@ int fr_evaluate_targets(fr_model *m, const double *targets, size_t n_targets, pt
   });
 }
 
-// x = A^-1 b for a dense symmetric matrix through the subdomain machinery (k_cholesky / k_chol_big_* and k_dom_solve on a
-// one-domain level without special points; indefinite matrices take the fallback of factorise_pool): the entry point of
-// the reference's reproducible known-answer tests linalg.rs:638-764 (make_spd) against the device factorisation.
+// x = A^-1 b for a dense symmetric matrix through the subdomain machinery on a one-domain level without special points
+// (k_cholesky and k_dom_solve; from n = 512 on k_chol_big_* and the spread solve; indefinite matrices take the fallback
+// of factorise_pool and k_dom_solve): the entry point of the reference's reproducible known-answer tests
+// linalg.rs:638-764 (make_spd) against the device factorisation.
 int fr_dense_spd_solve(const double *a, int n, const double *b, int nrhs, double *x, int *used_fallback) {
   return fr_guarded([&] {
     FB_REQUIRE(a && b && x && n > 0 && nrhs > 0, "fr_dense_spd_solve: bad arguments");

@@ -1,7 +1,9 @@
 """The reference's reproducible known-answer tests (SURVEY.md section 8c), re-expressed against the library:
   * monomial bases, polynomials.rs:163-239 (9 exact cases incl. the column order)              CPU, host entry point
-  * RFP Cholesky solve on the closed-form SPD matrix make_spd, linalg.rs:638-764                GPU, k_cholesky + k_dom_solve
-  * the indefinite fallback of domain.rs:63-68 (linalg.rs:514-616)                              GPU
+  * RFP Cholesky solve on the closed-form SPD matrix make_spd, linalg.rs:638-764                GPU, see below
+  * the indefinite fallback of domain.rs:63-68 (linalg.rs:514-616)                              GPU, k_dom_solve
+The SPD cases run k_cholesky + k_dom_solve below n = 512 and k_chol_big_* + k_tri_gemv (one domain spread over the GPU)
+from there on.
 """
 import ctypes as C
 
@@ -105,9 +107,10 @@ def test_blocked_cholesky_sizes(n):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("n", [40, 300])
+@pytest.mark.parametrize("n", [40, 300, 700])
 def test_indefinite_matrix_takes_the_fallback(n):
-    """domain.rs:63-68: a subdomain matrix that is not positive definite is solved by the pivoted fallback"""
+    """domain.rs:63-68: a subdomain matrix that is not positive definite is solved by the pivoted fallback (n = 700: a
+    single domain above the 512 threshold of the whole-GPU factorisation, whose spread solve the fallback bypasses)"""
     a = make_spd(n, 1.0) - 1.5 * np.eye(n)      # eigenvalues on both sides of zero
     ev = np.linalg.eigvalsh(a)
     assert ev[0] < -0.1 and ev[-1] > 0.1

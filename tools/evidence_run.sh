@@ -11,7 +11,7 @@ ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/ev
 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file $O/ev_fit_launches.csv python tools/fit_bench.py 1000000 0 1 > $O/ev_fit_launches.log 2>&1
 ncu --set full --clock-control none --import-source on -k 'regex:k_p2l_grid|k_p2p_sym|k_m2l_stream|k_p2m_t|k_l2p_t' -s 10 -c 5 -f -o $O/ev_full \
     python bench.py --steps 1 --warmup 3 --no-fit --no-cpu-baseline > $O/ev_full.log 2>&1
-ncu --set full --clock-control none --import-source on -k 'regex:k_dom_solve_v2|k_cholesky|k_tri_gemv' -s 6 -c 8 -f -o $O/ev_solver \
+ncu --set full --clock-control none --import-source on -k 'regex:k_dom_solve|k_cholesky|k_tri_gemv' -s 6 -c 8 -f -o $O/ev_solver \
     python tools/fit_bench.py 1000000 0 1 > $O/ev_solver.log 2>&1
 timeout 900 compute-sanitizer --tool memcheck --error-exitcode 9 python tools/sanitize_smoke.py > $O/ev_memcheck.log 2>&1; echo "memcheck rc=$?" >> $O/ev_memcheck.log
 timeout 900 compute-sanitizer --tool racecheck --racecheck-report all --error-exitcode 9 python tools/sanitize_smoke.py > $O/ev_racecheck.log 2>&1; echo "racecheck rc=$?" >> $O/ev_racecheck.log
