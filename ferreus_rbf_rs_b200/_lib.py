@@ -108,6 +108,9 @@ SIGNATURES = {
     "fb_tree_set_local_coefficients": (C.c_int, [C.c_void_p, _dp, _sz, _sz, _pd, _pd]),
     "fb_tree_evaluate": (C.c_int, [C.c_void_p, _dp, _sz, _sz, _pd, _pd, _dp, _sz, _pd, _pd, _dp, _dp, _pd, _pd,
                                    _u64p]),
+    "fb_tree_set_weights_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _sz, _pd, _pd, C.c_void_p]),
+    "fb_tree_evaluate_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _sz, _pd, _pd, C.c_void_p, _sz, _pd, _pd,
+                                          C.c_void_p, C.c_void_p, _pd, _pd, C.c_void_p, _u64p]),
     "fb_tree_evaluate_leaves": (C.c_int, [C.c_void_p, _dp, _sz, _sz, _pd, _pd, _dp, _sz, _pd, _pd, _dp, _dp, _pd,
                                           _pd, _u64p]),
     "fb_tree_evaluate_at_sources": (C.c_int, [C.c_void_p, _dp, _sz, _sz, _pd, _pd, _u64p, _sz, _dp, _pd, _pd]),
@@ -178,6 +181,9 @@ SOLVER_SIGNATURES = {
     "fr_evaluate_at_source": (C.c_int, [C.c_void_p, C.c_int, _dp]),
     "fr_build_evaluator": (C.c_int, [C.c_void_p, _dp]),
     "fr_evaluate_targets": (C.c_int, [C.c_void_p, _dp, _sz, _pd, _pd, _dp, _dp]),
+    "fr_evaluate_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _pd, _pd, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_evaluate_targets_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _pd, _pd, C.c_void_p, C.c_void_p,
+                                             C.c_void_p]),
     "fr_dense_spd_solve": (C.c_int, [_dp, C.c_int, _dp, C.c_int, _dp, _i32p]),
     "fr_evaluate_monomials": (C.c_int, [_dp, _sz, C.c_int, C.c_int, _dp, _dp, _dp, _i32p]),
     "fr_ddm_level": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p, _u64p, _u64p, _u64p, _u8p]),
@@ -265,3 +271,20 @@ pinned = _PinnedPool()
 def strides_of(a):
     """element strides (row, col) of a 2-D float64 array"""
     return a.strides[0] // 8, a.strides[1] // 8
+
+
+def cuda_matrix(obj, what):
+    """A 1-D or 2-D float64 CUDA tensor as (data_ptr, rows, cols, row_stride, col_stride, device); 1-D is a column.
+    torch is imported here, not when the package is, so the numpy API works without it."""
+    import torch
+    if not isinstance(obj, torch.Tensor) or not obj.is_cuda or obj.dtype != torch.float64 or obj.dim() not in (1, 2):
+        raise TypeError(f"Expected a 1D/2D float64 CUDA tensor for {what}")
+    if obj.dim() == 1:
+        return obj.data_ptr(), obj.shape[0], 1, obj.stride(0), 1, obj.device
+    return obj.data_ptr(), obj.shape[0], obj.shape[1], obj.stride(0), obj.stride(1), obj.device
+
+
+def cuda_stream(device):
+    """handle of torch's current stream on `device` (0 for the legacy default stream)"""
+    import torch
+    return torch.cuda.current_stream(device).cuda_stream

@@ -201,6 +201,31 @@ class FmmTree:
         self._check(rc)
         return _to_numpy(out)
 
+    # -- torch CUDA tensors in and out (fb_tree_*_device): no host round trip, ordered on torch's current stream ----
+    def set_weights_cuda(self, weights):
+        """set_weights with a float64 CUDA tensor (n x nrhs, any strides)."""
+        p, rows, cols, rs, cs, dev = _lib.cuda_matrix(weights, "weights")
+        self._check(self._lib.fb_tree_set_weights_device(self._h, p, rows, cols, rs, cs, _lib.cuda_stream(dev)))
+        self._nrhs = cols
+
+    def evaluate_cuda(self, weights, targets, *, gradients=False):
+        """evaluate / evaluate_with_gradients with float64 CUDA tensors; results are new tensors on the targets'
+        device, shaped as the numpy methods return them."""
+        import torch
+        wp, wrows, wcols, wrs, wcs, _ = _lib.cuda_matrix(weights, "weights")
+        xp, m, xcols, xrs, xcs, dev = _lib.cuda_matrix(targets, "target_points")
+        if xcols != self._dim:
+            raise ValueError(f"target_points must have {self._dim} columns, got {xcols}")
+        out = torch.empty((m, self._nrhs), dtype=torch.float64, device=dev)
+        g = torch.empty((m, self._nrhs * self._dim), dtype=torch.float64, device=dev) if gradients else None
+        bad = C.c_uint64(0)
+        rc = self._lib.fb_tree_evaluate_device(self._h, wp, wrows, wcols, wrs, wcs, xp, m, xrs, xcs, out.data_ptr(),
+                                               g.data_ptr() if gradients else None, self._nrhs, 1,
+                                               _lib.cuda_stream(dev), C.byref(bad))
+        self._check(rc, bad)
+        vals = out[:, 0] if self._nrhs == 1 else out
+        return (vals, g[:, 0] if g.shape[1] == 1 else g) if gradients else vals
+
     def upload_weights(self, weights):
         w = _as_matrix(weights, "weights")
         rs, cs = _lib.strides_of(w)

@@ -150,20 +150,6 @@ struct fb_shard {
 
 void fb_shard_free(fb_shard *s) { delete s; }
 
-template <class F>
-static int guarded(F &&f) {
-  try {
-    f();
-    return FB_OK;
-  } catch (const fb::Error &e) {
-    set_last_error(e.what());
-    return e.code;
-  } catch (const std::exception &e) {
-    set_last_error(e.what());
-    return FB_ERR_CUDA;
-  }
-}
-
 extern "C" {
 
 int fb_partition_by_work(const double *work, size_t n_leaves, int parts, uint64_t *bounds_out) {

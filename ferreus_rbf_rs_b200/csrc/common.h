@@ -22,6 +22,22 @@ struct Error : std::runtime_error {
 void set_last_error(const std::string &msg);
 extern std::atomic<uint64_t> g_launches;
 
+// body of a C entry point: exceptions become error codes and the fb_last_error() message
+template <class F>
+int guarded(F &&f, uint64_t *bad = nullptr) {
+  try {
+    f();
+    return FB_OK;
+  } catch (const Error &e) {
+    set_last_error(e.what());
+    if (bad && e.code == FB_ERR_POINT_OUTSIDE_TREE) *bad = e.index;
+    return e.code;
+  } catch (const std::exception &e) {
+    set_last_error(e.what());
+    return FB_ERR_CUDA;
+  }
+}
+
 #define FB_CUDA(expr)                                                                              \
   do {                                                                                             \
     cudaError_t _e = (expr);                                                                       \

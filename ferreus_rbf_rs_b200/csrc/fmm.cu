@@ -910,7 +910,6 @@ static int bits_for(size_t v) {
 TargetSet fb_tree::bin_targets(const double *targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, uint64_t *bad) {
   FB_REQUIRE(targets != nullptr && m > 0, "target_points must be a non-empty m x dim matrix");
   FB_REQUIRE(m < (1ull << 31), "at most 2^31-1 targets per call");
-  const int nl = (int)ht.leaves.size();
   // targets bit-identical to the source points, in the same order (what ferreus_rbf's solver passes on every
   // matvec, rbf.rs:1357-1364): compared on the host, nothing is uploaded or binned
   if (m == n && cs == 1 && rs == (ptrdiff_t)dim && same_bytes(targets, host_points.data(), n * dim * sizeof(double)))
@@ -924,6 +923,11 @@ TargetSet fb_tree::bin_targets(const double *targets, size_t m, ptrdiff_t rs, pt
       for (int d = 0; d < dim; ++d) h_stage.p[i * dim + d] = targets[(ptrdiff_t)i * rs + (ptrdiff_t)d * cs];
     FB_CUDA(cudaMemcpyAsync(d_t_user.p, h_stage.p, m * dim * sizeof(double), cudaMemcpyHostToDevice, stream));
   }
+  return bin_user_targets(m, bad);
+}
+
+TargetSet fb_tree::bin_user_targets(size_t m, uint64_t *bad) {
+  const int nl = (int)ht.leaves.size();
   TargetBuffers &tb = tb_scratch;
   tb.key.reserve(m);
   tb.key2.reserve(m);
@@ -1069,21 +1073,6 @@ void fb_tree::fetch_output(size_t m, bool grads, double *out_vals, double *out_g
 }
 
 // ------------------------------------------------------------------------------------------ C ABI
-template <class F>
-static int guarded(F &&f, uint64_t *bad = nullptr) {
-  try {
-    f();
-    return FB_OK;
-  } catch (const fb::Error &e) {
-    set_last_error(e.what());
-    if (bad && e.code == FB_ERR_POINT_OUTSIDE_TREE) *bad = e.index;
-    return e.code;
-  } catch (const std::exception &e) {
-    set_last_error(e.what());
-    return FB_ERR_CUDA;
-  }
-}
-
 static void collect_timing(fb_tree *t) {
   if (!t->timing) return;
   auto ms = [&](int a, int b) {

@@ -119,6 +119,45 @@ bool launch_l2p_fast(const TargetSet &ts, const int *leaf_cell, const double *lo
                      const double *ccz, const double *chalf, const double *tnodes, int p, int dim, int nrhs,
                      double *out, cudaStream_t s);
 
+// ---- device_io.cu: inputs and outputs in caller-owned device memory (the *_device entry points) -------------------
+// FB_ERR_INVALID_ARGUMENT naming `what` unless the first and the last element of the rows x cols matrix at p (element
+// strides rs, cs) lie in device memory of `device`
+void require_device_matrix(const void *p, size_t rows, size_t cols, ptrdiff_t rs, ptrdiff_t cs, int device,
+                           const char *what);
+// Orders `own` (a handle's non-blocking stream) after the work queued so far on `caller`, and, in join() or when the
+// object goes out of scope (a call that fails half way), `caller` after everything queued on `own` meanwhile.
+struct StreamJoin {
+  cudaStream_t caller, own;
+  bool joined = false;
+  StreamJoin(cudaStream_t caller_, cudaStream_t own_);
+  void join();
+  ~StreamJoin();
+};
+struct AffineMap {  // x' = [x 1] * a, a (dim+1) x (dim+1) row-major; on = 0: identity
+  int on = 0;
+  double a[16] = {0};
+};
+// rows x cols strided copy between device matrices, each row optionally mapped through `aff` (cols = dim)
+void launch_copy_rows(const double *src, ptrdiff_t s_rs, ptrdiff_t s_cs, size_t rows, int cols, double *dst,
+                      ptrdiff_t d_rs, ptrdiff_t d_cs, const AffineMap &aff, cudaStream_t s);
+// [mins..., maxs...] over the rows of a strided m x dim device matrix; scratch is device memory for the partial
+// results.  Blocks until the 2*dim values are on the host.
+void device_extents(const double *x, size_t m, int dim, ptrdiff_t rs, ptrdiff_t cs, DBuf<double> &scratch,
+                    cudaStream_t s, double *ext);
+// finish of the interpolant (fr_model::eval_tree) on the device: one thread per (target, value column)
+struct RbfFinish {
+  size_t m = 0;
+  int dim = 0, n_cols = 0, basis = 0, degree = 0;
+  const double *targets = nullptr;  // original coordinates
+  ptrdiff_t t_rs = 0, t_cs = 0;
+  const double *vals = nullptr, *grads = nullptr;  // leaf pass results [m][n_cols], [m][n_cols * dim] (null: none)
+  const double *poly = nullptr;                    // basis x n_cols row-major
+  double translation[3] = {0, 0, 0}, scale[3] = {1, 1, 1};
+  AffineMap trend;                                 // gradients are mapped back through its linear part when on
+  double *out = nullptr, *out_grads = nullptr;     // row-major, as fr_evaluate
+};
+void launch_rbf_finish(const RbfFinish &f, cudaStream_t s);
+
 // ---- M2L work lists, one group per (level, reference vector) -----------------------------------
 // m2l.cu: streaming M2L (TMA gathers / scatter-adds around register-resident operators); null plan = not applicable
 struct M2LStreamPlan;
@@ -256,6 +295,15 @@ struct fb_tree {
   void evaluate_sources_fused(const fb::TargetSet &ts);  // downward + leaf pass for targets that are source points
   fb::TargetSet source_target_set();
   fb::TargetSet bin_targets(const double *targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, uint64_t *bad);
+  // device_io.cu: targets in caller-owned device memory, mapped through the affine matrix `aff` ((dim+1) x (dim+1),
+  // row-major, applied to homogeneous row vectors) when it is non-null
+  fb::TargetSet bin_targets_dev(const double *d_targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, const double *aff,
+                                uint64_t *bad);
+  // shared tail of bin_targets / bin_targets_dev: the m targets are in d_t_user (row-major); blocks the host until they
+  // are binned (the outside-the-tree check reads d_err)
+  fb::TargetSet bin_user_targets(size_t m, uint64_t *bad);
+  // device_io.cu: weights in caller-owned device memory -> d_w_user, d_w (no upward pass)
+  void upload_weights_dev(const double *d_w, size_t n_rows, size_t nrhs_, ptrdiff_t rs, ptrdiff_t cs);
   fb::TargetSet subset_target_set(const uint64_t *idx, size_t n_idx);
   // subset of the sources as targets, index list already on the device; storage owned by `tb`
   fb::TargetSet subset_target_set_dev(const unsigned long long *d_idx, size_t n_idx, fb::TargetBuffers &tb);

@@ -734,6 +734,11 @@ struct fr_model {
   fb_tree *make_tree(bool sparse, const double *extents);
   void eval_tree(fb_tree *t, const double *targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, bool leaves, bool add_nugget,
                  double *out_vals, double *out_grads);
+  // eval_tree for targets and outputs in device memory (fr_evaluate_device, fr_evaluate_targets_device), on t->stream
+  void eval_tree_dev(fb_tree *t, const double *d_targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
+                     double *d_out, double *d_grads);
+  DBuf<double> d_poly;  // poly_coeff on the device (the device path), uploaded on first use
+  DBuf<double> d_ext;   // partial results of the device extents reduction (fr_evaluate_device)
   void emit(int kind, uint64_t iter, double residual, double progress, const char *msg) {
     if (!cb) return;
     fr_event ev{kind, iter, residual, progress, msg};
@@ -1626,6 +1631,44 @@ void fr_model::eval_tree(fb_tree *t, const double *targets, size_t mt, ptrdiff_t
   }
 }
 
+void fr_model::eval_tree_dev(fb_tree *t, const double *d_targets, size_t mt, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
+                             double *d_out, double *d_grads) {
+  const int m = st.basis_size;
+  if (m > 0 && d_poly.cap < (size_t)m * n_cols) {  // once per model: the coefficients never change after the fit
+    d_poly.reserve((size_t)m * n_cols);
+    FB_CUDA(cudaMemcpy(d_poly.p, poly_coeff.data(), (size_t)m * n_cols * sizeof(double), cudaMemcpyHostToDevice));
+  }
+  uint64_t bad = 0;
+  TargetSet ts = t->bin_targets_dev(d_targets, mt, rs, cs, has_trend ? aff : nullptr, &bad);
+  if (!t->have_weights || t->nrhs != (int)n_cols)  // as eval_tree
+    t->upload_weights(point_coeff.data(), n, n_cols, (ptrdiff_t)n_cols, 1);
+  if (!leaves) t->downward(ts.cell_flag);
+  t->leaf_pass(ts, d_grads != nullptr);
+  RbfFinish f;
+  f.m = mt;
+  f.dim = dim;
+  f.n_cols = (int)n_cols;
+  f.basis = m;
+  f.degree = st.polynomial_degree;
+  f.targets = d_targets;
+  f.t_rs = rs;
+  f.t_cs = cs;
+  f.vals = t->d_out.p;
+  f.grads = d_grads ? t->d_gout.p : nullptr;
+  f.poly = m > 0 ? d_poly.p : nullptr;
+  for (int d = 0; d < dim && m > 0; ++d) {
+    f.translation[d] = translation[d];
+    f.scale[d] = scale[d];
+  }
+  if (has_trend) {
+    f.trend.on = 1;
+    std::copy(aff, aff + 16, f.trend.a);
+  }
+  f.out = d_out;
+  f.out_grads = d_grads;
+  launch_rbf_finish(f, t->stream);
+}
+
 // ------------------------------------------------------------------------------------------ C ABI
 template <class F>
 static int fr_guarded(F &&f) {
@@ -1910,6 +1953,61 @@ int fr_evaluate_targets(fr_model *m, const double *targets, size_t n_targets, pt
     FB_REQUIRE(m && targets && out_vals && n_targets > 0, "model, targets and output are required");
     FB_REQUIRE(m->evaluator != nullptr, "build_evaluator must be called before evaluate_targets");
     m->eval_tree(m->evaluator.get(), targets, n_targets, t_rs, t_cs, true, false, out_vals, out_grads_or_null);
+  });
+}
+
+// the arguments of fr_evaluate_device / fr_evaluate_targets_device (pointer checks on `device`)
+static void require_device_eval_args(const fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs,
+                                     ptrdiff_t t_cs, double *d_out, double *d_grads, int device) {
+  require_device_matrix(d_targets, n_targets, m->dim, t_rs, t_cs, device, "target_points");
+  require_device_matrix(d_out, n_targets, m->n_cols, (ptrdiff_t)m->n_cols, 1, device, "output");
+  if (d_grads)
+    require_device_matrix(d_grads, n_targets, m->n_cols * m->dim, (ptrdiff_t)(m->n_cols * m->dim), 1, device,
+                          "gradient output");
+}
+
+int fr_evaluate_device(fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
+                       double *d_out, double *d_grads_or_null, void *stream) {
+  return fr_guarded([&] {
+    FB_REQUIRE(m && d_targets && d_out && n_targets > 0, "model, targets and output are required");
+    int device = 0;
+    FB_CUDA(cudaGetDevice(&device));
+    require_device_eval_args(m, d_targets, n_targets, t_rs, t_cs, d_out, d_grads_or_null, device);
+    // union of source and target extents (rbf.rs:640-668), as fr_evaluate; the target part is reduced on the device
+    const int dim = m->dim;
+    double ext[6];
+    device_extents(d_targets, n_targets, dim, t_rs, t_cs, m->d_ext, (cudaStream_t)stream, ext);
+    for (int d = 0; d < dim; ++d) {
+      double lo = m->points[d], hi = lo;
+      for (size_t i = 0; i < m->n; ++i) {
+        lo = std::min(lo, m->points[i * dim + d]);
+        hi = std::max(hi, m->points[i * dim + d]);
+      }
+      ext[d] = std::min(lo, ext[d]);
+      ext[dim + d] = std::max(hi, ext[dim + d]);
+    }
+    m->transform_extents(ext);
+    std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(m->make_tree(false, ext), fb_tree_free);
+    tree->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
+    tree->upward();
+    StreamJoin sj((cudaStream_t)stream, tree->stream);
+    m->eval_tree_dev(tree.get(), d_targets, n_targets, t_rs, t_cs, false, d_out, d_grads_or_null);
+    sj.join();
+    FB_CUDA(cudaStreamSynchronize(tree->stream));  // the tree is freed on return
+  });
+}
+
+int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
+                               double *d_out, double *d_grads_or_null, void *stream) {
+  return fr_guarded([&] {
+    FB_REQUIRE(m && d_targets && d_out && n_targets > 0, "model, targets and output are required");
+    FB_REQUIRE(m->evaluator != nullptr, "build_evaluator must be called before evaluate_targets");
+    fb_tree *t = m->evaluator.get();
+    FB_CUDA(cudaSetDevice(t->device));
+    require_device_eval_args(m, d_targets, n_targets, t_rs, t_cs, d_out, d_grads_or_null, t->device);
+    StreamJoin sj((cudaStream_t)stream, t->stream);
+    m->eval_tree_dev(t, d_targets, n_targets, t_rs, t_cs, true, d_out, d_grads_or_null);
+    sj.join();
   });
 }
 

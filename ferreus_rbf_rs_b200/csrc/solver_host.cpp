@@ -10,6 +10,8 @@
 #include <numeric>
 #include <string>
 
+#include "monomials.h"
+
 namespace fb {
 
 bool resolve_settings(const fr_settings &in, int dim, Settings &out, std::string &err) {
@@ -83,15 +85,7 @@ void evaluate_monomials(const double *pts, const int64_t *idx, size_t n, int dim
     const double *p = pts + (size_t)(idx ? idx[i] : (int64_t)i) * dim;
     double s[3] = {0, 0, 0};
     for (int d = 0; d < dim; ++d) s[d] = (p[d] - translation[d]) / scale[d];
-    double *o = out + i * basis;
-    o[0] = 1.0;
-    if (degree >= 1)
-      for (int d = 0; d < dim; ++d) o[1 + d] = s[d];
-    if (degree == 2) {
-      int k = 1 + dim;
-      for (int a = 0; a < dim; ++a)
-        for (int b = a; b < dim; ++b) o[k++] = s[a] * s[b];
-    }
+    monomial_row(s, dim, degree, out + i * basis);
   }
 }
 

@@ -328,6 +328,29 @@ class RBFInterpolator:
         # python_bindings.rs:818-826 routes this to the one-shot evaluate_with_gradients (SURVEY.md quirk viii)
         return self._eval(self._L.fr_evaluate, target_points, True)
 
+    # ---- torch CUDA tensors in and out (fr_evaluate*_device): no host round trip, ordered on torch's current stream --
+    def _eval_cuda(self, fn, targets, gradients):
+        import torch
+        p, m, cols, rs, cs, dev = _lib.cuda_matrix(targets, "target_points")
+        if cols != self._dim:
+            raise ValueError(f"target_points must have {self._dim} columns, got {cols}")
+        out = torch.empty((m, self._cols), dtype=torch.float64, device=dev)
+        g = torch.empty((m, self._cols * self._dim), dtype=torch.float64, device=dev) if gradients else None
+        self._check(fn(self._h, p, m, rs, cs, out.data_ptr(), g.data_ptr() if gradients else None,
+                       _lib.cuda_stream(dev)))
+        vals = out[:, 0] if self._cols == 1 else out
+        return (vals, g) if gradients else vals
+
+    def evaluate_cuda(self, targets, *, gradients=False):
+        """evaluate / evaluate_with_gradients with a float64 CUDA tensor of targets (m x dim, any strides); returns
+        tensors on its device.  Blocks until the results are complete (the one-shot tree is freed on return)."""
+        return self._eval_cuda(self._L.fr_evaluate_device, targets, gradients)
+
+    def evaluate_targets_cuda(self, targets, *, gradients=False):
+        """evaluate_targets through the tree of build_evaluator, with a float64 CUDA tensor of targets; gradients come
+        from that tree too.  Returns once the targets are binned; the results are ordered on torch's current stream."""
+        return self._eval_cuda(self._L.fr_evaluate_targets_device, targets, gradients)
+
     # ---- introspection -----------------------------------------------------------------------
     def ddm_level(self, level):
         nd, npts = C.c_uint64(), C.c_uint64()

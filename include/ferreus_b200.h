@@ -7,7 +7,8 @@
  * `ferreus_rbf::RBFInterpolator` (ferreus_rbf/src/rbf.rs:304-924).  Plain pointers and sizes
  * only; matrices are passed with element strides so faer column-major (`row_stride = 1,
  * col_stride = nrows`) and numpy row-major (`row_stride = ncols, col_stride = 1`) both pass
- * zero-copy.  All host pointers; the library owns all device memory.
+ * zero-copy.  Host pointers, and the library owns all device memory, except in the *_device entry points, whose
+ * matrices are caller-owned device memory (see fb_tree_evaluate_device).
  *
  * A handle is NOT thread-safe (same contract as `&mut self` in the reference); distinct
  * handles may be used concurrently.  No function aborts the process: errors are returned as
@@ -111,6 +112,32 @@ int fb_tree_set_local_coefficients(fb_tree *t, const double *w, size_t n_rows, s
 int fb_tree_evaluate(fb_tree *t, const double *w, size_t n_rows, size_t nrhs, ptrdiff_t w_rs, ptrdiff_t w_cs,
                      const double *targets, size_t m, ptrdiff_t t_rs, ptrdiff_t t_cs, double *out_vals,
                      double *out_grads_or_null, ptrdiff_t o_rs, ptrdiff_t o_cs, uint64_t *bad_index);
+/* ---- device-memory variants (not in the reference API) ---------------------------------------------------------
+ * fb_tree_set_weights_device and fb_tree_evaluate_device have the semantics of fb_tree_set_weights and fb_tree_evaluate
+ * (the w given to evaluate feeds the near field; the multipoles come from the last set-weights call), but every matrix
+ * argument is device memory and the work is ordered on the caller's CUDA stream `stream` (a cudaStream_t; NULL is the
+ * legacy default stream).  Layouts are those of the host functions; gradients are row-major m x (nrhs*dim) when
+ * o_cs == 1, column-major otherwise, as fb_tree_evaluate writes them.
+ *  - Pointers: each matrix must be device memory of the handle's device (cudaPointerGetAttributes, checked at its
+ *    first and last element before any kernel reads it); anything else, a NULL handle or pointer, m == 0 or a wrong
+ *    column count returns FB_ERR_INVALID_ARGUMENT with a message naming the argument.
+ *  - Stream order: the handle's (non-blocking) stream waits for an event recorded on `stream` at entry; `stream`
+ *    waits for an event recorded on the handle's stream after the last piece of work.  Nothing else orders the library
+ *    against the caller.
+ *  - Host blocking: fb_tree_evaluate_device blocks until the targets are binned (the outside-the-tree check reads one
+ *    flag back), hence until the work queued on `stream` before the call has finished; it returns before the results
+ *    are complete.  fb_tree_set_weights_device does not block.
+ *  - Input lifetime: every input has been read before the completion event; the caller may reuse the memory for work
+ *    queued on `stream` after the call.
+ *  - Errors: FB_ERR_POINT_OUTSIDE_TREE with *bad_index and the message of fb_tree_evaluate.  The handle stays usable
+ *    after any error.  A host upload that follows a device one is always sent (the repeat-upload test of
+ *    fb_tree_set_weights only compares host bytes).                                                                */
+int fb_tree_set_weights_device(fb_tree *t, const double *d_w, size_t n_rows, size_t nrhs, ptrdiff_t row_stride,
+                               ptrdiff_t col_stride, void *stream);
+int fb_tree_evaluate_device(fb_tree *t, const double *d_w, size_t n_rows, size_t nrhs, ptrdiff_t w_rs, ptrdiff_t w_cs,
+                            const double *d_targets, size_t m, ptrdiff_t t_rs, ptrdiff_t t_cs, double *d_out,
+                            double *d_grads_or_null, ptrdiff_t o_rs, ptrdiff_t o_cs, void *stream,
+                            uint64_t *bad_index);
 /* FmmTree::evaluate_leaves / evaluate_leaves_with_gradients (bbfmm.rs:537-616): leaf pass only. */
 int fb_tree_evaluate_leaves(fb_tree *t, const double *w, size_t n_rows, size_t nrhs, ptrdiff_t w_rs,
                             ptrdiff_t w_cs, const double *targets, size_t m, ptrdiff_t t_rs, ptrdiff_t t_cs,

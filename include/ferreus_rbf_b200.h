@@ -135,6 +135,21 @@ int fr_build_evaluator(fr_model *m, const double *extents_or_null);
 int fr_evaluate_targets(fr_model *m, const double *targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
                         double *out_vals, double *out_grads_or_null);
 
+/* ---- device-memory variants (not in the reference API): targets (n_targets x dim, element strides) and outputs
+ * (row-major, the layouts of fr_evaluate) are device memory of the current CUDA device; `stream` is the caller's
+ * cudaStream_t.  Pointer checks, stream order, input lifetime and errors as fb_tree_evaluate_device
+ * (ferreus_b200.h); the handle stays usable after any error.
+ *  - fr_evaluate_device: fr_evaluate, the one-shot tree over the union of source and target extents.  The extents
+ *    are reduced on `stream` and read back (2 * dim doubles), and the temporary tree is freed at the end, so this call
+ *    blocks until its results are complete.
+ *  - fr_evaluate_targets_device: fr_evaluate_targets, through the tree of fr_build_evaluator.  Blocks until the
+ *    targets are binned, not until the results are complete.  With d_grads it returns the evaluator's gradients
+ *    (unlike the reference's evaluate_targets_with_gradients, which takes the one-shot path).                    */
+int fr_evaluate_device(fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
+                       double *d_out, double *d_grads_or_null, void *stream);
+int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
+                               double *d_out, double *d_grads_or_null, void *stream);
+
 /* ---- introspection for the parity gates ------------------------------------------------------------- */
 /* DDM hierarchy: level l (0 = finest ... levels-1 = coarse): number of domains, and per domain the point
  * indices (CSR) with the internal mask.  Any pointer may be NULL (call once for sizes, once for data).     */
