@@ -1,7 +1,10 @@
 """Importable stand-in for the reference's PyO3 module ``ferreus_rbf`` (py_ferreus_rbf/src/lib.rs:15-87): the same
 top-level classes and the ``config`` / ``interpolant_config`` / ``progress`` submodules registered in ``sys.modules``
-exactly as the Rust module init does, all re-exported from the B200 mirror (``ferreus_rbf_rs_b200``).  Isosurfacing
-(``ferreus_rbf.isosurfacing``, ``Mesh``, ``BoundaryClosure``) is out of scope (SURVEY.md section 8f) and is absent."""
+exactly as the Rust module init does, all re-exported from the B200 mirror (``ferreus_rbf_rs_b200``).  The reference's
+isosurfacing (``ferreus_rbf.isosurfacing``, ``build_isosurface(s)``, ``Mesh``, ``BoundaryClosure``: the regularised
+surface following of ``ferreus_rmt``) is absent, and no function takes those names.  Isosurfaces of 3-D models come
+from ``RBFInterpolator.extract_isosurfaces`` / ``extract_isosurfaces_cuda`` instead: lattice marching tetrahedra with the
+vertices refined onto the interpolant, which gives different meshes."""
 import sys
 
 import numpy as np

@@ -184,6 +184,14 @@ SOLVER_SIGNATURES = {
     "fr_evaluate_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _pd, _pd, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fr_evaluate_targets_device": (C.c_int, [C.c_void_p, C.c_void_p, _sz, _pd, _pd, C.c_void_p, C.c_void_p,
                                              C.c_void_p]),
+    "fr_isosurface_extract": (C.c_int, [C.c_void_p, _dp, _u64p, _dp, C.c_int, C.c_int, C.c_int,
+                                        C.POINTER(C.c_void_p)]),
+    "fr_lattice_isosurface": (C.c_int, [C.c_void_p, _u64p, _dp, C.c_double, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "fr_isosurface_counts": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
+    "fr_isosurface_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_isosurface_timing": (C.c_int, [C.c_void_p, _dp]),
+    "fr_isosurface_refine_stats": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
+    "fr_isosurface_free": (None, [C.c_void_p]),
     "fr_dense_spd_solve": (C.c_int, [_dp, C.c_int, _dp, C.c_int, _dp, _i32p]),
     "fr_evaluate_monomials": (C.c_int, [_dp, _sz, C.c_int, C.c_int, _dp, _dp, _dp, _i32p]),
     "fr_ddm_level": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p, _u64p, _u64p, _u64p, _u8p]),

@@ -351,6 +351,36 @@ class RBFInterpolator:
         from that tree too.  Returns once the targets are binned; the results are ordered on torch's current stream."""
         return self._eval_cuda(self._L.fr_evaluate_targets_device, targets, gradients)
 
+    # ---- isosurfaces (fr_isosurface_extract): one lattice evaluation and one transient tree for all isovalues ------
+    def _isosurfaces(self, isovalues, extents, resolution, column, refine, device):
+        """(meshes, {"ms": stage times, "refine": [(evaluations, iterations)] per isovalue})"""
+        from .isosurface import Handle, lattice_args
+        ext, res = lattice_args(extents, resolution)
+        iso = np.ascontiguousarray(np.atleast_1d(np.asarray(isovalues, dtype=np.float64)).ravel())
+        with Handle() as h:
+            self._check(self._L.fr_isosurface_extract(self._h, _lib.dptr(ext), res.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                      _lib.dptr(iso), iso.size, int(column), int(bool(refine)),
+                                                      C.byref(h.h)))
+            meshes = [h.mesh(i, True, device) for i in range(iso.size)]
+            stats = {"ms": h.timing(), "refine": [h.refine_stats(i) for i in range(iso.size)]}
+        return meshes, stats
+
+    def extract_isosurfaces(self, isovalues, extents, resolution, *, column=0, refine=True):
+        """Meshes of the level sets of value column `column` of a 3-D model: one (vertices (V, 3) float64, faces (F, 3)
+        int64, normals (V, 3) float64) per isovalue.  The interpolant is evaluated on the lattice of `extents`
+        [x0, y0, z0, x1, y1, z1] and `resolution` (an int or (nx, ny, nz)); every lattice cube is split into six
+        tetrahedra, giving one vertex per crossing lattice edge.  With `refine` the vertices are moved along their edges
+        onto the interpolant.  Faces are oriented, and normals point, along increasing value.  Every mesh edge is shared
+        by two faces except on the lattice's boundary faces."""
+        return self._isosurfaces(isovalues, extents, resolution, column, refine, None)[0]
+
+    def extract_isosurfaces_cuda(self, isovalues, extents, resolution, *, column=0, refine=True):
+        """extract_isosurfaces with the meshes as torch CUDA tensors on the current CUDA device.  Blocks until they
+        are complete, like evaluate_cuda."""
+        import torch
+        dev = torch.device("cuda", torch.cuda.current_device())
+        return self._isosurfaces(isovalues, extents, resolution, column, refine, dev)[0]
+
     # ---- introspection -----------------------------------------------------------------------
     def ddm_level(self, level):
         nd, npts = C.c_uint64(), C.c_uint64()

@@ -150,6 +150,40 @@ int fr_evaluate_device(fr_model *m, const double *d_targets, size_t n_targets, p
 int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
                                double *d_out, double *d_grads_or_null, void *stream);
 
+/* ---- isosurfaces of 3-D interpolants (not in the reference API) ------------------------------------------------
+ * Lattice: extents = {x0, y0, z0, x1, y1, z1} with lo < hi, resolution = {nx, ny, nz} >= 2, at most 2^28 nodes; node
+ * idx on an axis is idx * step + lo, step = (hi - lo) / (n - 1), the last node exactly hi (np.linspace); node
+ * p = i + nx * (j + ny * k).  A node is below when its value is < iso.  Every cube is split into the 6 Kuhn
+ * tetrahedra, so the mesh has no cracks: one vertex per crossing lattice edge (numbered by edge id), triangles ordered
+ * by (cube, tetrahedron, triangle) and oriented so that (B-A) x (C-A) points along increasing value.  Every mesh edge
+ * is used by two triangles in opposite directions except on the lattice's boundary faces.  DESIGN.md has the full
+ * specification.
+ *  - fr_isosurface_extract: one transient tree over the union of the lattice and the source points (the rule of
+ *    fr_evaluate_device; fr_build_evaluator's tree is not touched) evaluates column `column` on the lattice; one
+ *    surface per isovalue.  refine != 0 moves every vertex along its edge onto the interpolant (Illinois regula falsi
+ *    from the lattice bracket: stops at a bracket of 2^-40 of the edge, f == iso, or 60 evaluations); normals are the
+ *    normalised interpolant gradient at the final vertices.  Blocks until complete.
+ *  - fr_lattice_isosurface: the mesh of caller-owned lattice values (device memory, nz x ny x nx contiguous) on the
+ *    caller's cudaStream_t; vertices stay on the lattice edges' linear interpolation and there are no normals.
+ *    Blocks until complete.
+ *  - results stay in the handle's device memory: fr_isosurface_counts, then fr_isosurface_copy to host or device
+ *    memory (vertices V x 3, faces F x 3 of int64 vertex indices, normals V x 3 or NULL; `which` = isovalue index).
+ *  - fr_isosurface_timing: milliseconds of {lattice evaluation with the tree, extraction, refinement, normals}.
+ *  - fr_isosurface_refine_stats: trial points evaluated by the refinement and its iteration count (the slowest
+ *    vertex's evaluations).
+ * Invalid arguments (a model that is not 3-D, a bad lattice, n_iso < 1, a non-finite isovalue or lattice value, a
+ * column out of range) return FB_ERR_INVALID_ARGUMENT and leave the model usable.                                 */
+typedef struct fr_isosurface fr_isosurface;
+int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *resolution, const double *isovalues,
+                          int n_iso, int column, int refine, fr_isosurface **out);
+int fr_lattice_isosurface(const double *d_values, const uint64_t *resolution, const double *extents, double isovalue,
+                          void *stream, fr_isosurface **out);
+int fr_isosurface_counts(const fr_isosurface *s, int which, uint64_t *n_vertices, uint64_t *n_faces);
+int fr_isosurface_copy(const fr_isosurface *s, int which, double *vertices, int64_t *faces, double *normals_or_null);
+int fr_isosurface_timing(const fr_isosurface *s, double *ms_out4);
+int fr_isosurface_refine_stats(const fr_isosurface *s, int which, uint64_t *evaluations, uint64_t *iterations);
+void fr_isosurface_free(fr_isosurface *s);
+
 /* ---- introspection for the parity gates ------------------------------------------------------------- */
 /* DDM hierarchy: level l (0 = finest ... levels-1 = coarse): number of domains, and per domain the point
  * indices (CSR) with the internal mask.  Any pointer may be NULL (call once for sizes, once for data).     */
