@@ -1,6 +1,6 @@
 // Evaluation with inputs and outputs in caller-owned device memory: the *_device entry points of
-// include/ferreus_b200.h (FmmTree) and the kernels behind them and behind fr_evaluate_device /
-// fr_evaluate_targets_device (solver.cu).  Targets and weights are gathered from the caller's strides on the device,
+// include/ferreus_b200.h (FmmTree) and the kernels behind them and behind every interpolant evaluation
+// (fr_model::eval_tree, solver.cu).  Targets and weights are gathered from the caller's strides on the device,
 // then the host path takes over unchanged from the binning (fb_tree::bin_user_targets) or the weight sort on; results
 // go back to the caller's memory with one more kernel or a device-to-device copy.  Nothing crosses the PCIe bus but the
 // outside-the-tree flag (and, for the one-shot interpolant, the 2 * dim extents).
@@ -61,8 +61,10 @@ StreamJoin::~StreamJoin() {
 
 // ------------------------------------------------------------------------------------------ kernels
 // Row i of src (strides s_rs, s_cs) -> row i of dst (d_rs, d_cs); with aff.on the row is the homogeneous vector
-// [x 1] times aff.a, in the order of fr_model::apply_affine (solver.cu) with every product and sum rounded on its own,
-// as the host compiles it (-ffp-contract=off).
+// [x 1] times aff.a, bit for bit as fr_model::apply_affine (solver.cu) computes it on the host (same order, every
+// product and sum rounded on its own; the host compiles with -ffp-contract=off).  With a global trend,
+// evaluate_at_source relies on it: the mapped source points must equal the tree's kernel-space points for
+// bin_user_targets to recognise them.
 __global__ void k_copy_rows(const double *__restrict__ src, ptrdiff_t s_rs, ptrdiff_t s_cs, size_t rows, int cols,
                             double *__restrict__ dst, ptrdiff_t d_rs, ptrdiff_t d_cs, AffineMap aff) {
   const size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
@@ -127,12 +129,14 @@ __global__ void k_extents_final(const double *part, int n_parts, int dim, double
   ext[j] = v;
 }
 
-// The per-target finish of fr_model::eval_tree (solver.cu), one thread per (target, value column), in the host loops'
-// order and association with every product and sum rounded on its own (the host compiles with -ffp-contract=off):
+// The per-target finish of fr_model::eval_tree (solver.cu), one thread per (target, value column), every product and
+// sum rounded on its own:
 //   1. kernel gradient mapped back through the trend, g <- g B^T;
-//   2. + sum_k mono_k(x) poly[k][c] on the original coordinates (monomial_row, monomials.h);
-//   3. + the drift gradient (degree 1 and 2, evaluate_monomial_gradients);
-//   4. stored row-major.
+//   2. + nugget * w[i][c] when w is given (evaluate_at_source(add_nugget)), before the drift;
+//   3. + sum_k mono_k(x) poly[k][c] on the original coordinates (monomial_row, monomials.h);
+//   4. + the drift gradient (degree 1 and 2, evaluate_monomial_gradients);
+//   5. stored row-major.
+// Each thread reads and writes only its own (target, column) elements, so out may be vals and out_grads grads.
 __global__ void k_rbf_finish(RbfFinish f) {
   const size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
   if (t >= f.m * (size_t)f.n_cols) return;
@@ -153,6 +157,7 @@ __global__ void k_rbf_finish(RbfFinish f) {
       }
     }
   }
+  if (f.w) val = __dadd_rn(val, __dmul_rn(f.nugget, f.w[t]));
   if (f.basis > 0) {
     double sp[3] = {0, 0, 0};
     for (int d = 0; d < dim; ++d)

@@ -144,13 +144,16 @@ void launch_copy_rows(const double *src, ptrdiff_t s_rs, ptrdiff_t s_cs, size_t 
 // results.  Blocks until the 2*dim values are on the host.
 void device_extents(const double *x, size_t m, int dim, ptrdiff_t rs, ptrdiff_t cs, DBuf<double> &scratch,
                     cudaStream_t s, double *ext);
-// finish of the interpolant (fr_model::eval_tree) on the device: one thread per (target, value column)
+// finish of the interpolant (fr_model::eval_tree): one thread per (target, value column).  out / out_grads may be
+// vals / grads (no pointer here is __restrict__)
 struct RbfFinish {
   size_t m = 0;
   int dim = 0, n_cols = 0, basis = 0, degree = 0;
   const double *targets = nullptr;  // original coordinates
   ptrdiff_t t_rs = 0, t_cs = 0;
   const double *vals = nullptr, *grads = nullptr;  // leaf pass results [m][n_cols], [m][n_cols * dim] (null: none)
+  const double *w = nullptr;                       // point coefficients [m][n_cols] when the nugget is added, else null
+  double nugget = 0;
   const double *poly = nullptr;                    // basis x n_cols row-major
   double translation[3] = {0, 0, 0}, scale[3] = {1, 1, 1};
   AffineMap trend;                                 // gradients are mapped back through its linear part when on

@@ -733,13 +733,20 @@ struct fr_model {
 
   void fit();
   fb_tree *make_tree(bool sparse, const double *extents);
-  void eval_tree(fb_tree *t, const double *targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, bool leaves, bool add_nugget,
-                 double *out_vals, double *out_grads);
-  // eval_tree for targets and outputs in device memory (fr_evaluate_device, fr_evaluate_targets_device), on t->stream
-  void eval_tree_dev(fb_tree *t, const double *d_targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
-                     double *d_out, double *d_grads);
-  DBuf<double> d_poly;  // poly_coeff on the device (the device path), uploaded on first use
-  DBuf<double> d_ext;   // partial results of the device extents reduction (fr_evaluate_device)
+  // make_tree with the point coefficients uploaded and their multipoles computed
+  std::unique_ptr<fb_tree, void (*)(fb_tree *)> transient_tree(bool sparse, const double *extents);
+  // [mins..., maxs...] of the source points and target_ext together, mapped to kernel space (ext may be target_ext)
+  void evaluation_extents(const double *target_ext, double *ext) const;
+  // the interpolant at targets in device memory, on t->stream; every evaluation entry point ends here
+  void eval_tree(fb_tree *t, const double *d_targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, bool leaves, bool add_nugget,
+                 double *d_out, double *d_grads);
+  // host targets for eval_staged: their rows, row-major, in d_targets, queued on s
+  void stage_targets(const double *targets, size_t m, ptrdiff_t rs, ptrdiff_t cs, cudaStream_t s);
+  // eval_tree of the staged targets into the tree's output buffers, then downloaded to row-major host arrays
+  void eval_staged(fb_tree *t, size_t m, bool leaves, bool add_nugget, double *out_vals, double *out_grads);
+  DBuf<double> d_poly;     // poly_coeff on the device, uploaded on first use
+  DBuf<double> d_ext;      // partial results of the device extents reduction (fr_evaluate, fr_evaluate_device)
+  DBuf<double> d_targets;  // host targets staged by stage_targets
   void emit(int kind, uint64_t iter, double residual, double progress, const char *msg) {
     if (!cb) return;
     fr_event ev{kind, iter, residual, progress, msg};
@@ -1208,6 +1215,13 @@ fb_tree *fr_model::make_tree(bool sparse, const double *extents) {
   return t;
 }
 
+std::unique_ptr<fb_tree, void (*)(fb_tree *)> fr_model::transient_tree(bool sparse, const double *extents) {
+  std::unique_ptr<fb_tree, void (*)(fb_tree *)> t(make_tree(sparse, extents), fb_tree_free);
+  t->upload_weights(point_coeff.data(), n, n_cols, (ptrdiff_t)n_cols, 1);
+  t->upward();
+  return t;
+}
+
 void fr_model::fit() {
   using clk = std::chrono::steady_clock;
   const auto t_start = clk::now();
@@ -1558,82 +1572,27 @@ void fr_model::transform_extents(double *ext) const {  // rbf.rs:603-615 (boundi
   }
 }
 
-// evaluate the interpolant through a tree whose multipoles hold the point coefficients (rbf.rs:1180-1270)
-void fr_model::eval_tree(fb_tree *t, const double *targets, size_t mt, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
-                         bool add_nugget, double *out_vals, double *out_grads) {
-  uint64_t bad = 0;
-  std::vector<double> ttg;
-  if (has_trend) {  // the kernel part is evaluated in the transformed space (rbf.rs:1181-1185)
-    ttg.resize(mt * dim);
-    apply_affine(aff, targets, mt, rs, cs, ttg.data());
-  }
-  TargetSet ts = has_trend ? t->bin_targets(ttg.data(), mt, dim, 1, &bad) : t->bin_targets(targets, mt, rs, cs, &bad);
-  // every caller has just uploaded the point coefficients into this tree (set_weights semantics, rbf.rs:684, 836):
-  // they stay resident, so repeated small-batch evaluate_targets calls move only the targets and the results
-  if (!t->have_weights || t->nrhs != (int)n_cols)
-    t->upload_weights(point_coeff.data(), n, n_cols, (ptrdiff_t)n_cols, 1);
-  if (!leaves) t->downward(ts.cell_flag);
-  t->leaf_pass(ts, out_grads != nullptr);
-  t->fetch_output(mt, out_grads != nullptr, out_vals, out_grads, (ptrdiff_t)n_cols, 1);
-  if (has_trend && out_grads) {  // grad_x f = grad_x' f * B^T, B = linear part of the transform (rbf.rs:1272-1298)
-    const int h = dim + 1;
-    for (size_t i = 0; i < mt; ++i)
-      for (size_t c = 0; c < n_cols; ++c) {
-        double *g = out_grads + i * (n_cols * dim) + c * dim;
-        double tmp[3] = {0, 0, 0};
-        for (int d = 0; d < dim; ++d) tmp[d] = g[d];
-        for (int k = 0; k < dim; ++k) {
-          double acc = 0.0;
-          for (int j = 0; j < dim; ++j) acc += tmp[j] * aff[k * h + j];  // B^T[j][k] = B[k][j]
-          g[k] = acc;
-        }
-      }
-  }
-  if (add_nugget)
-    for (size_t i = 0; i < mt && i < n; ++i)
-      for (size_t c = 0; c < n_cols; ++c) out_vals[i * n_cols + c] += point_coeff[i * n_cols + c] * st.nugget;
-  const int m = st.basis_size;
-  if (m == 0) return;
-  std::vector<double> tp(mt * dim), mono(mt * (size_t)m);
-  for (size_t i = 0; i < mt; ++i)
-    for (int d = 0; d < dim; ++d) tp[i * dim + d] = targets[(ptrdiff_t)i * rs + (ptrdiff_t)d * cs];
-  evaluate_monomials(tp.data(), nullptr, mt, dim, st.polynomial_degree, m, translation.data(), scale.data(),
-                     mono.data());
-  for (size_t i = 0; i < mt; ++i)
-    for (size_t c = 0; c < n_cols; ++c) {
-      double v = 0;
-      for (int k = 0; k < m; ++k) v += mono[i * m + k] * poly_coeff[(size_t)k * n_cols + c];
-      out_vals[i * n_cols + c] += v;
+// union of source and target extents (rbf.rs:640-668)
+void fr_model::evaluation_extents(const double *target_ext, double *ext) const {
+  for (int d = 0; d < dim; ++d) {
+    double lo = points[d], hi = lo;
+    for (size_t i = 0; i < n; ++i) {
+      lo = std::min(lo, points[i * dim + d]);
+      hi = std::max(hi, points[i * dim + d]);
     }
-  if (out_grads && st.polynomial_degree >= 1) {  // evaluate_monomial_gradients, polynomials.rs:64-116
-    const int deg = st.polynomial_degree;
-    for (size_t i = 0; i < mt; ++i) {
-      double sp[3] = {0, 0, 0};
-      for (int d = 0; d < dim; ++d) sp[d] = (tp[i * dim + d] - translation[d]) / scale[d];
-      for (size_t c = 0; c < n_cols; ++c) {
-        double *g = out_grads + i * (n_cols * dim) + c * dim;
-        for (int d = 0; d < dim; ++d) g[d] += poly_coeff[(size_t)(1 + d) * n_cols + c] / scale[d];
-        if (deg == 2) {
-          int k = 1 + dim;
-          for (int a = 0; a < dim; ++a)
-            for (int b = a; b < dim; ++b) {
-              const double cf = poly_coeff[(size_t)k * n_cols + c];
-              if (a == b) {
-                g[a] += cf * (2.0 * sp[a] / scale[a]);
-              } else {
-                g[a] += cf * (sp[b] / scale[a]);
-                g[b] += cf * (sp[a] / scale[b]);
-              }
-              ++k;
-            }
-        }
-      }
-    }
+    ext[d] = std::min(lo, target_ext[d]);
+    ext[dim + d] = std::max(hi, target_ext[dim + d]);
   }
+  transform_extents(ext);
 }
 
-void fr_model::eval_tree_dev(fb_tree *t, const double *d_targets, size_t mt, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
-                             double *d_out, double *d_grads) {
+// evaluate the interpolant through a tree whose multipoles hold the point coefficients (rbf.rs:1180-1270): the targets
+// are mapped through the trend and binned (bin_targets_dev), the leaf pass (after the downward pass unless `leaves`)
+// leaves the kernel part in t->d_out / t->d_gout, and k_rbf_finish adds the rest into d_out / d_grads.  These may be
+// t->d_out / t->d_gout themselves: the finish reads and writes only its own elements.  add_nugget: the targets are the
+// source points, in their order.
+void fr_model::eval_tree(fb_tree *t, const double *d_targets, size_t mt, ptrdiff_t rs, ptrdiff_t cs, bool leaves,
+                         bool add_nugget, double *d_out, double *d_grads) {
   const int m = st.basis_size;
   if (m > 0 && d_poly.cap < (size_t)m * n_cols) {  // once per model: the coefficients never change after the fit
     d_poly.reserve((size_t)m * n_cols);
@@ -1641,7 +1600,9 @@ void fr_model::eval_tree_dev(fb_tree *t, const double *d_targets, size_t mt, ptr
   }
   uint64_t bad = 0;
   TargetSet ts = t->bin_targets_dev(d_targets, mt, rs, cs, has_trend ? aff : nullptr, &bad);
-  if (!t->have_weights || t->nrhs != (int)n_cols)  // as eval_tree
+  // every caller has just uploaded the point coefficients into this tree (set_weights semantics, rbf.rs:684, 836):
+  // they stay resident, so repeated small-batch evaluate_targets calls move only the targets and the results
+  if (!t->have_weights || t->nrhs != (int)n_cols)
     t->upload_weights(point_coeff.data(), n, n_cols, (ptrdiff_t)n_cols, 1);
   if (!leaves) t->downward(ts.cell_flag);
   t->leaf_pass(ts, d_grads != nullptr);
@@ -1656,6 +1617,10 @@ void fr_model::eval_tree_dev(fb_tree *t, const double *d_targets, size_t mt, ptr
   f.t_cs = cs;
   f.vals = t->d_out.p;
   f.grads = d_grads ? t->d_gout.p : nullptr;
+  if (add_nugget) {
+    f.w = t->d_w_user.p;  // the point coefficients as uploaded, in input order
+    f.nugget = st.nugget;
+  }
   f.poly = m > 0 ? d_poly.p : nullptr;
   for (int d = 0; d < dim && m > 0; ++d) {
     f.translation[d] = translation[d];
@@ -1668,6 +1633,28 @@ void fr_model::eval_tree_dev(fb_tree *t, const double *d_targets, size_t mt, ptr
   f.out = d_out;
   f.out_grads = d_grads;
   launch_rbf_finish(f, t->stream);
+}
+
+void fr_model::stage_targets(const double *targets, size_t mt, ptrdiff_t rs, ptrdiff_t cs, cudaStream_t s) {
+  const size_t cnt = mt * dim;
+  std::vector<double> rows;
+  if (cs != 1 || rs != (ptrdiff_t)dim) {
+    rows.resize(cnt);
+    for (size_t i = 0; i < mt; ++i)
+      for (int d = 0; d < dim; ++d) rows[i * dim + d] = targets[(ptrdiff_t)i * rs + (ptrdiff_t)d * cs];
+    targets = rows.data();
+  }
+  d_targets.reserve(cnt);
+  // from pageable memory: returns once the source has been read, so `rows` may go
+  FB_CUDA(cudaMemcpyAsync(d_targets.p, targets, cnt * sizeof(double), cudaMemcpyHostToDevice, s));
+}
+
+void fr_model::eval_staged(fb_tree *t, size_t mt, bool leaves, bool add_nugget, double *out_vals, double *out_grads) {
+  // the leaf pass zeroes these in place: reserved here, their addresses hold from now on
+  t->d_out.reserve(mt * n_cols);
+  if (out_grads) t->d_gout.reserve(mt * n_cols * dim);
+  eval_tree(t, d_targets.p, mt, dim, 1, leaves, add_nugget, t->d_out.p, out_grads ? t->d_gout.p : nullptr);
+  t->fetch_output(mt, out_grads != nullptr, out_vals, out_grads, (ptrdiff_t)n_cols, 1);
 }
 
 // ------------------------------------------------------------------------------------------ C ABI
@@ -1896,38 +1883,22 @@ int fr_evaluate(fr_model *m, const double *targets, size_t n_targets, ptrdiff_t 
                 double *out_grads_or_null) {
   return fr_guarded([&] {
     FB_REQUIRE(m && targets && out_vals && n_targets > 0, "model, targets and output are required");
-    // union of source and target extents (rbf.rs:640-668), non-sparse adaptive tree (rbf.rs:677-681)
-    const int dim = m->dim;
+    // as fr_evaluate_device, on the legacy default stream (device_extents waits for it)
+    m->stage_targets(targets, n_targets, t_rs, t_cs, nullptr);
     double ext[6];
-    for (int d = 0; d < dim; ++d) {
-      double lo = m->points[d], hi = lo;
-      for (size_t i = 0; i < m->n; ++i) {
-        lo = std::min(lo, m->points[i * dim + d]);
-        hi = std::max(hi, m->points[i * dim + d]);
-      }
-      for (size_t i = 0; i < n_targets; ++i) {
-        const double v = targets[(ptrdiff_t)i * t_rs + (ptrdiff_t)d * t_cs];
-        lo = std::min(lo, v);
-        hi = std::max(hi, v);
-      }
-      ext[d] = lo;
-      ext[dim + d] = hi;
-    }
-    m->transform_extents(ext);
-    std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(m->make_tree(false, ext), fb_tree_free);
-    tree->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
-    tree->upward();
-    m->eval_tree(tree.get(), targets, n_targets, t_rs, t_cs, false, false, out_vals, out_grads_or_null);
+    device_extents(m->d_targets.p, n_targets, m->dim, m->dim, 1, m->d_ext, nullptr, ext);
+    m->evaluation_extents(ext, ext);
+    auto tree = m->transient_tree(false, ext);  // non-sparse adaptive tree (rbf.rs:677-681)
+    m->eval_staged(tree.get(), n_targets, false, false, out_vals, out_grads_or_null);
   });
 }
 
 int fr_evaluate_at_source(fr_model *m, int add_nugget, double *out_vals) {
   return fr_guarded([&] {
     FB_REQUIRE(m && out_vals, "model and output are required");
-    std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(m->make_tree(true, nullptr), fb_tree_free);  // rbf.rs:777-781
-    tree->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
-    tree->upward();
-    m->eval_tree(tree.get(), m->points.data(), m->n, m->dim, 1, false, add_nugget != 0, out_vals, nullptr);
+    auto tree = m->transient_tree(true, nullptr);  // rbf.rs:777-781
+    m->stage_targets(m->points.data(), m->n, m->dim, 1, tree->stream);
+    m->eval_staged(tree.get(), m->n, false, add_nugget != 0, out_vals, nullptr);
   });
 }
 
@@ -1939,10 +1910,8 @@ int fr_build_evaluator(fr_model *m, const double *extents_or_null) {
       std::copy(extents_or_null, extents_or_null + 2 * m->dim, ext);
       m->transform_extents(ext);
     }
-    m->evaluator.reset(m->make_tree(false, extents_or_null ? ext : nullptr));  // rbf.rs:830-838
+    m->evaluator = m->transient_tree(false, extents_or_null ? ext : nullptr);  // rbf.rs:830-838
     fb_tree *t = m->evaluator.get();
-    t->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
-    t->upward();
     t->downward(t->d_flag_all.p);
     FB_CUDA(cudaStreamSynchronize(t->stream));
   });
@@ -1953,7 +1922,9 @@ int fr_evaluate_targets(fr_model *m, const double *targets, size_t n_targets, pt
   return fr_guarded([&] {
     FB_REQUIRE(m && targets && out_vals && n_targets > 0, "model, targets and output are required");
     FB_REQUIRE(m->evaluator != nullptr, "build_evaluator must be called before evaluate_targets");
-    m->eval_tree(m->evaluator.get(), targets, n_targets, t_rs, t_cs, true, false, out_vals, out_grads_or_null);
+    fb_tree *t = m->evaluator.get();
+    m->stage_targets(targets, n_targets, t_rs, t_cs, t->stream);
+    m->eval_staged(t, n_targets, true, false, out_vals, out_grads_or_null);
   });
 }
 
@@ -1974,25 +1945,13 @@ int fr_evaluate_device(fr_model *m, const double *d_targets, size_t n_targets, p
     int device = 0;
     FB_CUDA(cudaGetDevice(&device));
     require_device_eval_args(m, d_targets, n_targets, t_rs, t_cs, d_out, d_grads_or_null, device);
-    // union of source and target extents (rbf.rs:640-668), as fr_evaluate; the target part is reduced on the device
-    const int dim = m->dim;
+    // the target part of the tree extents is reduced on the device
     double ext[6];
-    device_extents(d_targets, n_targets, dim, t_rs, t_cs, m->d_ext, (cudaStream_t)stream, ext);
-    for (int d = 0; d < dim; ++d) {
-      double lo = m->points[d], hi = lo;
-      for (size_t i = 0; i < m->n; ++i) {
-        lo = std::min(lo, m->points[i * dim + d]);
-        hi = std::max(hi, m->points[i * dim + d]);
-      }
-      ext[d] = std::min(lo, ext[d]);
-      ext[dim + d] = std::max(hi, ext[dim + d]);
-    }
-    m->transform_extents(ext);
-    std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(m->make_tree(false, ext), fb_tree_free);
-    tree->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
-    tree->upward();
+    device_extents(d_targets, n_targets, m->dim, t_rs, t_cs, m->d_ext, (cudaStream_t)stream, ext);
+    m->evaluation_extents(ext, ext);
+    auto tree = m->transient_tree(false, ext);
     StreamJoin sj((cudaStream_t)stream, tree->stream);
-    m->eval_tree_dev(tree.get(), d_targets, n_targets, t_rs, t_cs, false, d_out, d_grads_or_null);
+    m->eval_tree(tree.get(), d_targets, n_targets, t_rs, t_cs, false, false, d_out, d_grads_or_null);
     sj.join();
     FB_CUDA(cudaStreamSynchronize(tree->stream));  // the tree is freed on return
   });
@@ -2007,7 +1966,7 @@ int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_ta
     FB_CUDA(cudaSetDevice(t->device));
     require_device_eval_args(m, d_targets, n_targets, t_rs, t_cs, d_out, d_grads_or_null, t->device);
     StreamJoin sj((cudaStream_t)stream, t->stream);
-    m->eval_tree_dev(t, d_targets, n_targets, t_rs, t_cs, true, d_out, d_grads_or_null);
+    m->eval_tree(t, d_targets, n_targets, t_rs, t_cs, true, false, d_out, d_grads_or_null);
     sj.join();
   });
 }
@@ -2030,21 +1989,10 @@ int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *re
     const auto t0 = clk::now();
     // one transient tree over the union of the lattice and the source points, as fr_evaluate_device; the lattice, every
     // refinement batch and the normals are served from its leaf pass
-    double ext[6];
-    for (int d = 0; d < 3; ++d) {
-      double lo = L.lo[d], hi = L.hi[d];
-      for (size_t i = 0; i < m->n; ++i) {
-        lo = std::min(lo, m->points[i * 3 + d]);
-        hi = std::max(hi, m->points[i * 3 + d]);
-      }
-      ext[d] = lo;
-      ext[3 + d] = hi;
-    }
-    m->transform_extents(ext);
-    std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(m->make_tree(false, ext), fb_tree_free);
+    double ext[6] = {L.lo[0], L.lo[1], L.lo[2], L.hi[0], L.hi[1], L.hi[2]};
+    m->evaluation_extents(ext, ext);
+    auto tree = m->transient_tree(false, ext);
     fb_tree *t = tree.get();
-    t->upload_weights(m->point_coeff.data(), m->n, m->n_cols, (ptrdiff_t)m->n_cols, 1);
-    t->upward();
     t->downward(t->d_flag_all.p);
     const cudaStream_t s = t->stream;
     const uint64_t nodes = L.nodes();
@@ -2053,7 +2001,7 @@ int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *re
     xyz.reserve(3 * nodes);
     vals.reserve(nodes * nc);
     iso_lattice_points(L, xyz.p, s);
-    m->eval_tree_dev(t, xyz.p, nodes, 3, 1, true, vals.p, nullptr);
+    m->eval_tree(t, xyz.p, nodes, 3, 1, true, false, vals.p, nullptr);
     IsoScratch w;
     const double *v = vals.p + column;  // column `column` of the lattice values, stride n_cols
     const uint64_t bad = iso_first_nonfinite(v, nc, nodes, w, s);
@@ -2070,7 +2018,7 @@ int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *re
     const auto t2 = clk::now();
     if (refine) {
       const IsoEval eval = [&](const double *pts, size_t cnt, double *out_vals) {
-        m->eval_tree_dev(t, pts, cnt, 3, 1, true, out_vals, nullptr);
+        m->eval_tree(t, pts, cnt, 3, 1, true, false, out_vals, nullptr);
       };
       for (auto &f : h->surf) iso_refine(v, nc, L, (int)nc, column, eval, w, *f, s);
     }
@@ -2081,7 +2029,7 @@ int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *re
       if (f->nv) {
         gv.reserve(f->nv * nc);
         gg.reserve(f->nv * nc * 3);
-        m->eval_tree_dev(t, f->verts.p, f->nv, 3, 1, true, gv.p, gg.p);
+        m->eval_tree(t, f->verts.p, f->nv, 3, 1, true, false, gv.p, gg.p);
       }
       iso_normals(gg.p, (int)nc, column, *f, s);
     }

@@ -124,7 +124,10 @@ int fr_model_restore(const double *points, size_t n, int dim, const double *valu
                      const double *point_coefficients, const double *poly_coefficients_or_null,
                      const fr_model_state *state, fr_progress_cb cb_or_null, void *user, fr_model **out);
 
-/* evaluate / evaluate_with_gradients (rbf.rs:676-752): one-shot non-sparse adaptive tree on the union extents.
+/* Host-array evaluation: fr_evaluate, fr_evaluate_at_source and fr_evaluate_targets run the device path of
+ * fr_evaluate_device / fr_evaluate_targets_device below, behind one host-to-device copy of the targets and one
+ * device-to-host copy of the results.
+ * evaluate / evaluate_with_gradients (rbf.rs:676-752): one-shot non-sparse adaptive tree on the union extents.
  * out_vals m x n_cols row-major; out_grads (or NULL) m x (n_cols*dim).                                  */
 int fr_evaluate(fr_model *m, const double *targets, size_t n_targets, ptrdiff_t t_rs, ptrdiff_t t_cs,
                 double *out_vals, double *out_grads_or_null);

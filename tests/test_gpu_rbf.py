@@ -351,3 +351,40 @@ def test_indefinite_subdomain_falls_back_like_the_reference():
     assert ev[0] < -1e-3 and ev[-1] > 1e-3             # indefinite: the Cholesky path cannot have been taken
     lam = np.linalg.solve(k, vals)
     assert H.rel_l2(model.coefficients.point_coefficients, lam) <= 1e-8
+
+
+def test_strided_host_targets_match_a_contiguous_copy():
+    """The host-array evaluators gather the caller's rows at any strides: a Fortran-order array and a row-sliced view give
+    the results of a contiguous copy (the persistent evaluator bit for bit; the one-shot calls build a tree each, and
+    its M2L reductions reorder round-off, which reaches the gradients as up to ~2e-14, see test_gpu_device_eval)."""
+    import ferreus_rbf_rs_b200 as fb
+    pts = H.make_points(2000, 3, "uniform", seed=161)
+    vals = np.stack([_values(pts), np.cos(2 * pts[:, 0])], axis=1)
+    gt = fb.GlobalTrend.three(25.0, 70.0, 15.0, 3.0, 2.0, 1.0)
+    model = fb.RBFInterpolator(pts, vals, _settings(2, tol=1e-8), params=_params(2), global_trend=gt)
+    model.build_evaluator()
+    wide = np.random.default_rng(162).random((800, 3)) * 0.98 + 0.01
+    for x in (np.asfortranarray(wide), wide[::2]):
+        c = np.ascontiguousarray(x)
+        assert np.array_equal(model.evaluate_targets(x), model.evaluate_targets(c))
+        assert H.rel_l2(model.evaluate(x), model.evaluate(c)) <= 1e-14
+        v, g = model.evaluate_with_gradients(x)
+        vc, gc = model.evaluate_with_gradients(c)
+        assert H.rel_l2(v, vc) <= 1e-14 and H.rel_l2(g, gc) <= 1e-13
+
+
+@pytest.mark.parametrize("n,naive", [(600, 4096), (2400, 100)])
+def test_evaluate_at_source_adds_the_nugget(n, naive):
+    """evaluate_at_source(add_nugget=True) (rbf.rs:777-828) adds nugget * lambda to the interpolant at the source points,
+    which then reproduces the data: (K + nugget I) lambda + P c = f.  One dense domain, then the DDM solve."""
+    import ferreus_rbf_rs_b200 as fb
+    nugget, tol = 0.05, 1e-8
+    pts = H.make_points(n, 3, "uniform", seed=171)
+    vals = np.stack([_values(pts), np.cos(2 * pts[:, 0])], axis=1)
+    st = _settings(0, tol=tol, nugget=nugget, drift=fb.interpolant_config.Drift.Linear)
+    model = fb.RBFInterpolator(pts, vals, st, params=_params(0, naive=naive))
+    lam = model.coefficients.point_coefficients
+    plain = model.evaluate_at_source()
+    with_nugget = model.evaluate_at_source(add_nugget=True)
+    assert H.rel_l2(with_nugget - plain, nugget * lam) <= 1e-12
+    assert H.rel_l2(with_nugget, vals) <= 1e-6
