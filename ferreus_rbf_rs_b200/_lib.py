@@ -131,6 +131,7 @@ SIGNATURES = {
     "fb_tree_m2l_operator": (C.c_int, [C.c_void_p, C.c_int, C.c_int, _dp, _dp]),
     "fb_m2l_stream_warps": (C.c_int, [C.c_int, C.c_int]),
     "fb_tree_m2l_stream_warps": (C.c_int, [C.c_void_p]),
+    "fb_p2p_blocked_launch_count": (C.c_uint64, []),
     "fb_tree_leaf_work": (C.c_int, [C.c_void_p, _u64p, _dp]),
     "fb_tree_morton_order": (C.c_int, [C.c_void_p, _u64p]),
     "fb_tree_set_target_subset": (C.c_int, [C.c_void_p, _u64p, _sz]),

@@ -419,6 +419,27 @@ void fb_tree::build(const double *points, size_t n_, int dim_, ptrdiff_t rs, ptr
     d_w_ptr.upload(w_ptr, stream);
     d_w_ptr_none.upload(std::vector<long long>(nl + 1, 0), stream);
     d_w_cell.upload(w_c, stream);
+    // symmetric P2P of the all-sources set: a tile's pairs are its targets x (the sources of its U ranges behind it +
+    // half its own block).  The tiles go heaviest first, so that the big leaves of an adaptive tree (about 15x the
+    // pairs of a small one in a uniform cloud) start at the head of the grid instead of forming its tail.
+    {
+      std::vector<std::pair<long long, int>> work;
+      work.reserve(src_tiles);
+      for (int l = 0; l < nl; ++l)
+        for (int o = 0; o < tl_e[l] - tl_b[l]; o += kTile) {
+          const int cnt = std::min(kTile, tl_e[l] - tl_b[l] - o), te = tl_b[l] + o + cnt;
+          long long behind = 0;
+          for (long long e = u_ptr[l]; e < u_ptr[l + 1]; ++e)
+            behind += std::max(0, u_b[e] + u_c[e] - std::max(u_b[e], te));
+          work.emplace_back((long long)cnt * (behind + cnt / 2), (int)work.size());
+        }
+      std::stable_sort(work.begin(), work.end(), [](const std::pair<long long, int> &x, const std::pair<long long, int> &y) {
+        return x.first > y.first;
+      });
+      std::vector<int> order(work.size());
+      for (size_t i = 0; i < work.size(); ++i) order[i] = work[i].second;
+      d_src_tile_order.upload(order, stream);
+    }
     n_w_entries = (long long)w_c.size();
     // one CTA per X cell (p2l.cu), dispatched in blockIdx order: the cells are listed by descending source count so that
     // the long lists start first and the short ones fill the tail of the grid (a rank's share of a partitioned tree is
@@ -843,6 +864,7 @@ TargetSet fb_tree::source_target_set() {
   ts.own_lo = 0;
   ts.own_hi = (int)n;
   ts.row_of_pos = d_src_out_row.p;
+  ts.sym_tile_order = d_src_tile_order.p;
   return ts;
 }
 

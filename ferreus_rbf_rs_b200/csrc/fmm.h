@@ -34,6 +34,8 @@ struct TargetSet {
   const uint32_t *row_of_pos = nullptr;  // per sorted source position: output row, 0xFFFFFFFF when not a target
   const uint32_t *tgt_prefix = nullptr;  // n + 1 exclusive counts of targets over the sorted positions; null = all
   const uint8_t *cell_flag = nullptr;                      // per cell: subtree contains targets
+  // symmetric P2P (p2p_sym.cu): the tiles in the order the kernel takes them, heaviest first; null = tile order
+  const int *sym_tile_order = nullptr;
 };
 
 // device storage behind a TargetSet that is not the tree's own source set
@@ -239,6 +241,7 @@ struct fb_tree {
   int n_src_leaves = 0;
   // all-sources target set
   fb::DBuf<int> d_src_tl_begin, d_src_tl_end, d_src_tile_leaf, d_src_tile_off, d_src_ntiles;
+  fb::DBuf<int> d_src_tile_order;  // the tiles by descending symmetric-P2P work (TargetSet::sym_tile_order)
   fb::DBuf<uint32_t> d_src_out_row;
   int src_tiles = 0;
   // general target set scratch

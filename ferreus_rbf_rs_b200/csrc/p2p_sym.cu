@@ -6,9 +6,10 @@
 // here each unordered pair is evaluated ONCE and serves both rows:
 //     out[t] += k(t, s) w[s]      and      out[s] += k(t, s) w[t]        (all registry kernels are symmetric).
 // U is a symmetric relation (adjacent leaves at any level + the leaf itself, linear_tree.rs:177-395 / :397-485), and the
-// sources are stored in Morton order, so "each unordered pair once" = a warp owning the 32 consecutive sorted positions
+// sources are stored in Morton order, so "each unordered pair once" = a warp owning the consecutive sorted positions
 // [tb, tb + cnt) of a leaf takes the part of the leaf's merged U ranges that lies AFTER its own chunk (symmetric
-// tiles), plus its own cnt x cnt diagonal block evaluated in full.
+// tiles), plus its own cnt x cnt diagonal block.  One right-hand side runs k_p2p_sym_blocked (a warp per 128-target
+// tile, below); 2 - 4 right-hand sides, and one when FB_GENERIC_P2P=1, run k_p2p_sym (a warp per 64 targets).
 //
 // Cost model (tools/fp64_ubench.cu, tools/dmma_bench.cu): the FP64 pipe is the only resource (DMMA shares it, MUFU.RSQ64H
 // serialises with it), 10 DFMA + 1 MUFU per evaluation = 7.2 clk per warp step on an SM.  The symmetric step adds one
@@ -20,6 +21,7 @@
 #include "fmm.h"
 
 #include <algorithm>
+#include <atomic>
 #include <cstdlib>
 
 namespace fb {
@@ -233,9 +235,256 @@ __global__ void __launch_bounds__(kSymWPC * 32, NR == 1 ? 5 : (NR == 2 ? 4 : 3))
   else p2p_sym_body<FAM, FAST, false, NR>(a, sm, li, tb, cnt, lane, split, part);
 }
 
+// ---- one right-hand side: a warp per kTile = 128-target tile, NT = 1, 2 or 4 targets per lane -------------------------
+// Lane l owns the targets 32 u + l (u < NT) of the tile, NT picked from the tile's count so that a short leaf does not
+// run the four-target body on empty slots.  Per staged source: one broadcast of {x, y}, {z, w}, NT evaluations, the NT
+// source-side terms combined in registers (one DMUL + NT - 1 DFMA) and ONE store to part[j][l]: with NT = 4 that is a
+// quarter of the shared-memory stores, half the source broadcasts and a quarter of the flush per pair of the two-target
+// body above.  Flush: lane j sums row j in a fixed order (LDS.128, rows 34 doubles apart: 8 lanes of a quarter-warp
+// hit 8 distinct 16-byte bank groups) and issues one RED; no per-source loop, so no divergent collective.
+// Source tiles are gathered across the merged U ranges (a tile ends only where the sources behind the tile end), so
+// the inner loop runs 32 trips everywhere but in the last tile.
+// split: as in k_p2p_sym, `split` warps share a tile and take every split-th source tile (part 0 also the diagonal).
+// Order: with a warp per tile, a big leaf's tile (a depth-4 leaf of about 240 points in a 1M-point uniform cloud) holds
+// about 15x the pairs of a small leaf's, so in tile order the pass ends in a tail of them (2.51-2.56 ms against 2.40 for
+// k_p2p_sym on a B200).  The all-sources set lists its tiles by descending (targets x sources behind them), and the
+// warps take them in that order (TargetSet::sym_tile_order): 1.89 ms (profiles/r5_p2p_order.json).  Giving the big
+// tiles two warps instead reached 2.21 ms in tile order and 2.01 ms heaviest first.
+// Diagonal: the tile's own block, sub-block pairs (u < g) of 32 x 32 once each (source block g is the targets 32 g + j,
+// its source-side sums land in the owning lane's accumulator); only the 32 x 32 self-blocks run in full, self term
+// included as the reference does.
+constexpr int kBlkWPC = 4;       // warps per CTA
+constexpr int kBlkStride = 34;   // row stride of the partial-sum matrix (doubles): even, for the LDS.128 row reads
+
+struct BlkWarpSmem {
+  double2 st[2][2][32];           // double-buffered source tile: {x, y}, {z, w}
+  double part[32 * kBlkStride];   // part[j][l] = sum over lane l's targets of k(t, s_j) w[t]
+};
+
+// row j of the partial sums, fixed order
+__device__ __forceinline__ double blk_row_sum(const BlkWarpSmem &sm, int j) {
+  const double2 *pr = reinterpret_cast<const double2 *>(sm.part + j * kBlkStride);
+  double2 q[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) q[k] = pr[k];
+#pragma unroll
+  for (int l = 4; l < 16; l += 4)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const double2 v = pr[l + k];
+      q[k].x += v.x;
+      q[k].y += v.y;
+    }
+  return ((q[0].x + q[0].y) + (q[1].x + q[1].y)) + ((q[2].x + q[2].y) + (q[3].x + q[3].y));
+}
+
+template <int FAM, bool FAST, int NT>
+__device__ __forceinline__ void p2p_blk_body(const DirectArgs &a, BlkWarpSmem &sm, const int li, const int tb,
+                                             const int cnt, const int lane, const int split, const int part) {
+  constexpr double kScale = kernel_weight_scale<FAM, FAST>();
+  const int a_end = tb + cnt;
+  double xt[NT], yt[NT], zt[NT], wt[NT], acc[NT];
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    const int i = 32 * u + lane;
+    xt[u] = yt[u] = zt[u] = wt[u] = acc[u] = 0.0;
+    if (i < cnt) {
+      xt[u] = a.sx[tb + i];
+      yt[u] = a.sy[tb + i];
+      zt[u] = a.sz[tb + i];
+      wt[u] = a.w[(size_t)a.rhs0 * a.n + tb + i] * kScale;
+    }
+  }
+  double *pl = sm.part + lane;
+
+  // ---- diagonal block (split part 0)
+  if (part == 0) {
+#pragma unroll
+    for (int g = 0; g < NT; ++g) {
+      const int mg = min(32, cnt - 32 * g);  // warp-uniform
+      if (mg <= 0) break;
+      sm.st[g & 1][0][lane] = make_double2(xt[g], yt[g]);
+      sm.st[g & 1][1][lane] = make_double2(zt[g], wt[g]);
+      __syncwarp();
+      const double2(*t)[32] = sm.st[g & 1];
+#pragma unroll 2
+      for (int j = 0; j < mg; ++j) {
+        const double2 p0 = t[0][j], p1 = t[1][j];
+        double ps = 0.0;
+#pragma unroll
+        for (int u = 0; u <= g; ++u) {
+          const double dx = xt[u] - p0.x, dy = yt[u] - p0.y, dz = zt[u] - p1.x;
+          double r2 = dx * dx;
+          r2 += dy * dy;
+          r2 += dz * dz;
+          const double v = kernel_mag<FAM, FAST, true>(r2, a.kp);
+          kernel_acc<FAM>(acc[u], v, p1.y);
+          if (u < g) ps = u == 0 ? v * wt[0] : fma(v, wt[u], ps);
+        }
+        if (g > 0) pl[j * kBlkStride] = ps;
+      }
+      if (g > 0) {
+        __syncwarp();
+        const double s = blk_row_sum(sm, lane);  // source side of target 32 g + lane: this lane's own row
+        if (lane < mg) kernel_acc<FAM>(acc[g], s, 1.0);
+        __syncwarp();
+      }
+    }
+  }
+  __syncwarp();
+
+  // ---- symmetric tiles: the part of the merged U ranges behind the tile
+  long long e = a.u_ptr[li];
+  const long long e_end = a.u_ptr[li + 1];
+  int pos = 0, end = 0;  // current clipped range [pos, end)
+  auto next_range = [&]() {
+    while (e < e_end) {
+      const int b = a.u_begin[e], n = a.u_count[e];
+      ++e;
+      pos = max(b, a_end);
+      end = b + n;
+      if (pos < end) return;
+    }
+    pos = end = 0;
+  };
+  next_range();
+  double rx = 0, ry = 0, rz = 0, rw = 0;
+  int rp = 0;       // sorted position of this lane's source in the fetched tile
+  int skip = part;  // tiles to pass over before the next one of this warp
+  auto fetch = [&](int &m) {  // the next tile of this warp: up to 32 sources gathered across ranges, this lane's one
+    for (;;) {
+      m = 0;
+      if (pos >= end) return;
+      const bool mine = skip == 0;
+      skip = mine ? split - 1 : skip - 1;
+      while (m < 32 && pos < end) {
+        const int k = min(32 - m, end - pos);
+        if (mine && lane >= m && lane < m + k) {
+          rp = pos + lane - m;
+          rx = a.sx[rp];
+          ry = a.sy[rp];
+          rz = a.sz[rp];
+          rw = a.w[(size_t)a.rhs0 * a.n + rp] * kScale;
+        }
+        m += k;
+        pos += k;
+        if (pos >= end) next_range();
+      }
+      if (mine) return;
+    }
+  };
+  int m_cur = 0, m_next = 0, buf = 0;
+  fetch(m_cur);
+  int rp_cur = rp;
+  if (lane < m_cur) {
+    sm.st[0][0][lane] = make_double2(rx, ry);
+    sm.st[0][1][lane] = make_double2(rz, rw);
+  }
+  __syncwarp();
+  while (m_cur > 0) {
+    fetch(m_next);  // global loads of the next tile overlap the arithmetic below
+    const double2(*t)[32] = sm.st[buf];
+#pragma unroll 2
+    for (int j = 0; j < m_cur; ++j) {
+      const double2 p0 = t[0][j], p1 = t[1][j];
+      double ps;
+#pragma unroll
+      for (int u = 0; u < NT; ++u) {
+        const double dx = xt[u] - p0.x, dy = yt[u] - p0.y, dz = zt[u] - p1.x;
+        double r2 = dx * dx;
+        r2 += dy * dy;
+        r2 += dz * dz;
+        const double v = kernel_mag<FAM, FAST, true>(r2, a.kp);
+        kernel_acc<FAM>(acc[u], v, p1.y);
+        ps = u == 0 ? v * wt[0] : fma(v, wt[u], ps);
+      }
+      pl[j * kBlkStride] = ps;
+    }
+    __syncwarp();
+    const double s = blk_row_sum(sm, lane);  // source side: row `lane`, one RED per source
+    if (lane < m_cur) atomicAdd(a.out + (size_t)a.sym_row[rp_cur] * a.nrhs + a.rhs0, FAM == KF_LINEAR ? -s : s);
+    buf ^= 1;
+    if (lane < m_next) {
+      sm.st[buf][0][lane] = make_double2(rx, ry);
+      sm.st[buf][1][lane] = make_double2(rz, rw);
+    }
+    __syncwarp();
+    m_cur = m_next;
+    rp_cur = rp;
+  }
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    const int i = 32 * u + lane;
+    if (i < cnt) atomicAdd(a.out + (size_t)a.sym_row[tb + i] * a.nrhs + a.rhs0, acc[u]);
+  }
+}
+
+// 20 warps per SM where the body fits 96 registers without spills (linear in both square-root modes, cubic with the
+// second-order one), else 16
+template <int FAM, bool FAST>
+constexpr int blk_min_ctas() {
+  return (FAM == KF_LINEAR || (FAM == KF_CUBIC && FAST)) ? 5 : 4;
+}
+
+template <int FAM, bool FAST>
+__global__ void __launch_bounds__(kBlkWPC * 32, blk_min_ctas<FAM, FAST>())
+    k_p2p_sym_blocked(const DirectArgs a, const int split) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long gw = (long long)blockIdx.x * kBlkWPC + warp;
+  const int slot = (int)(gw / split);
+  const int part = (int)(gw - (long long)slot * split);
+  if (slot >= *a.ts.n_tiles_dev) return;
+  // the all-sources set lists its tiles heaviest first (fmm.cu): the big leaves start at the head of the grid
+  const int tile = a.ts.sym_tile_order ? a.ts.sym_tile_order[slot] : slot;
+  const int li = a.ts.tile_leaf[tile];
+  // target i of the set is the source at the sorted position own_lo + i
+  const int tb = a.ts.own_lo + a.ts.leaf_begin[li] + a.ts.tile_off[tile];
+  const int cnt = min(kTile, a.ts.own_lo + a.ts.leaf_end[li] - tb);
+  if (cnt <= 0) return;
+  extern __shared__ __align__(16) unsigned char dsm_raw[];
+  BlkWarpSmem &sm = reinterpret_cast<BlkWarpSmem *>(dsm_raw)[warp];
+  if (cnt > 64) p2p_blk_body<FAM, FAST, 4>(a, sm, li, tb, cnt, lane, split, part);
+  else if (cnt > 32) p2p_blk_body<FAM, FAST, 2>(a, sm, li, tb, cnt, lane, split, part);
+  else p2p_blk_body<FAM, FAST, 1>(a, sm, li, tb, cnt, lane, split, part);
+}
+
+std::atomic<unsigned long long> g_p2p_blocked_launches{0};
+
+// FB_GENERIC_P2P=1 keeps one-column passes on k_p2p_sym (A/B baseline)
+static bool p2p_force_generic() {
+  static const bool on = [] {
+    const char *v = std::getenv("FB_GENERIC_P2P");
+    return v && v[0] == '1';
+  }();
+  return on;
+}
+
+template <int FAM>
+static void p2p_blocked_launch(const DirectArgs &a, cudaStream_t s) {
+  static_assert(kTile == 128, "four 32-target blocks per tile");
+  const size_t smem = sizeof(BlkWarpSmem) * kBlkWPC;
+  // about three waves of warps (148 SMs x 20 resident warps) keep the uneven tiles from leaving SMs idle at the end
+  const long long tiles = std::max<long long>(1, (long long)(a.ts.m / kTile));
+  const int split = (int)std::min<long long>(8, std::max<long long>(1, (148 * 20 * 3) / tiles));
+  const unsigned grid = (unsigned)(((long long)a.ts.max_tiles * split + kBlkWPC - 1) / kBlkWPC);
+  if (kernel_has_fast<FAM>() && a.kp.fast) {
+    constexpr bool F = kernel_has_fast<FAM>();
+    FB_CUDA(cudaFuncSetAttribute(k_p2p_sym_blocked<FAM, F>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FB_LAUNCH((k_p2p_sym_blocked<FAM, F>), grid, kBlkWPC * 32, smem, s, a, split);
+  } else {
+    FB_CUDA(cudaFuncSetAttribute(k_p2p_sym_blocked<FAM, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FB_LAUNCH((k_p2p_sym_blocked<FAM, false>), grid, kBlkWPC * 32, smem, s, a, split);
+  }
+  g_p2p_blocked_launches.fetch_add(1, std::memory_order_relaxed);
+}
+
 template <int FAM, int NR>
 static void p2p_sym_launch(const DirectArgs &a, cudaStream_t s) {
   static_assert(kTile == 128, "two 64-target warps per tile");
+  if (NR == 1 && !p2p_force_generic()) {
+    p2p_blocked_launch<FAM>(a, s);
+    return;
+  }
   const size_t smem = sizeof(SymWarpSmem<NR>) * kSymWPC;
   // about three waves of warps (148 SMs x 20 resident warps) keep the uneven chunks from leaving SMs idle at the end
   const long long chunks = std::max<long long>(1, (long long)(a.ts.m / 64));
@@ -292,3 +541,5 @@ void launch_p2p_sym(const DirectArgs &a0, cudaStream_t s) {
 }
 
 }  // namespace fb
+
+uint64_t fb_p2p_blocked_launch_count(void) { return fb::g_p2p_blocked_launches.load(); }

@@ -199,6 +199,10 @@ int fb_m2l_stream_warps(int P, int compression_type);
 /* the same for a built tree: the MMA warps of the streaming plan it holds, 0 when it runs the generic kernel (its P
  * is not served, FB_M2L_STREAM=0 at build time, depth < 2, or no V-list entries)                                  */
 int fb_tree_m2l_stream_warps(const fb_tree *t);
+/* launches of the one-column symmetric P2P kernel blocked on whole 128-target tiles (csrc/p2p_sym.cu) since the
+ * library was loaded.  FB_GENERIC_P2P=1, read once per process, keeps those passes on the two-target kernel and
+ * this count at 0.                                                                                                */
+uint64_t fb_p2p_blocked_launch_count(void);
 
 
 /* ---- multi-GPU sharding by Morton-contiguous leaf ranges (SURVEY.md §8e) ---------------------------------
