@@ -194,6 +194,8 @@ SOLVER_SIGNATURES = {
     "fr_isosurface_refine_stats": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "fr_isosurface_free": (None, [C.c_void_p]),
     "fr_dense_spd_solve": (C.c_int, [_dp, C.c_int, _dp, C.c_int, _dp, _i32p]),
+    "fr_ddm_level_solve": (C.c_int, [_dp, _sz, C.c_int, C.POINTER(FrSettings), C.POINTER(FrParams), C.c_int, C.c_int,
+                                     _dp, C.c_int, _dp, _u64p, _u64p]),
     "fr_evaluate_monomials": (C.c_int, [_dp, _sz, C.c_int, C.c_int, _dp, _dp, _dp, _i32p]),
     "fr_ddm_level": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p, _u64p, _u64p, _u64p, _u8p]),
     "fr_host_ddm_new": (C.c_int, [_dp, _sz, C.c_int, _pd, _pd, C.POINTER(FrSettings), C.POINTER(FrParams),

@@ -875,8 +875,9 @@ struct DeviceSolver {
       lv.big_inverse = true;
     } else {
       FB_LAUNCH(k_cholesky, (unsigned)nd, 256, smem, stream, lv.tab, lv.lpool.p, lv.fail.p);
-      FB_LAUNCH(k_inv_diag_inplace, dim3((unsigned)nd, (unsigned)((lv.max_mm + kNB - 1) / kNB)), 32, 0, stream, lv.tab,
-                lv.lpool.p);
+      if (lv.max_mm > 0)
+        FB_LAUNCH(k_inv_diag_inplace, dim3((unsigned)nd, (unsigned)((lv.max_mm + kNB - 1) / kNB)), 32, 0, stream, lv.tab,
+                  lv.lpool.p);
     }
   }
 
@@ -992,7 +993,8 @@ struct DeviceSolver {
     const KParams kp = M.kp;
     FB_LAUNCH(k_dom_prep, (unsigned)nd, 128, 0, stream, t, px.p, py.p, pz.p, kp, M.st.nugget, lv->qpool.p, scratch.p);
     const unsigned tiles = (unsigned)((lv->max_mm + 31) / 32);
-    for (size_t d0 = 0; d0 < nd; d0 += 32768) {  // grid.z limit
+    // tiles == 0: every domain has as many points as special points (mm = 0), Q^T A Q is empty
+    for (size_t d0 = 0; tiles > 0 && d0 < nd; d0 += 32768) {  // grid.z limit
       DomainTable tt = t;
       const unsigned cnt = (unsigned)std::min<size_t>(32768, nd - d0);
       tt.pt_ptr += d0;
@@ -1222,35 +1224,35 @@ std::unique_ptr<fb_tree, void (*)(fb_tree *)> fr_model::transient_tree(bool spar
   return t;
 }
 
-void fr_model::fit() {
+namespace {
+
+using TreePtr = std::unique_ptr<fb_tree, void (*)(fb_tree *)>;
+
+// The set-up of the solve, shared by fr_model::fit and fr_ddm_level_solve: kernel-space points and monomial scaling, the
+// DDM hierarchy (or the single dense domain below naive_solve_threshold) with every level factorised on the device and,
+// with_tree, the FMM tree and the levels' target sets.  mono_pts receives the inverse-transformed points of a trend
+// fit.  On return S.s is the stream the solve runs on.
+void setup_solve(fr_model &M, DeviceSolver &S, cudaStream_t setup_stream, bool with_tree, std::vector<double> &mono_pts,
+                 TreePtr &tree) {
   using clk = std::chrono::steady_clock;
-  const auto t_start = clk::now();
-  info = fr_model_info{};
-  info.dim = (uint64_t)dim;
-  info.n_cols = n_cols;
-  info.basis_size = (uint64_t)st.basis_size;
-  const size_t m = (size_t)st.basis_size;
-  translation.assign(dim, 0.0);
-  scale.assign(dim, 1.0);
+  const size_t n = M.n, m = (size_t)M.st.basis_size;
+  const int dim = M.dim;
+  M.translation.assign(dim, 0.0);
+  M.scale.assign(dim, 1.0);
   // global trend (rbf.rs:361-371): kernel space = transformed points; monomials are evaluated at the inverse
   // transform of those (rbf.rs:477-484, domain.rs:169-175), which also become the public points (rbf.rs:579-581)
-  std::vector<double> mono_pts;
-  if (has_trend) {
-    build_trend_transform();
-    kpts.resize(n * dim);
-    apply_affine(aff, points.data(), n, dim, 1, kpts.data());
+  if (M.has_trend) {
+    M.build_trend_transform();
+    M.kpts.resize(n * dim);
+    M.apply_affine(M.aff, M.points.data(), n, dim, 1, M.kpts.data());
     mono_pts.resize(n * dim);
-    apply_affine(aff_inv, kpts.data(), n, dim, 1, mono_pts.data());
+    M.apply_affine(M.aff_inv, M.kpts.data(), n, dim, 1, mono_pts.data());
   }
-  const double *kp_ptr = kernel_points();
-  const double *mono_ptr = has_trend ? mono_pts.data() : nullptr;
-  if (m) cheb_cube_scaling(kp_ptr, nullptr, n, dim, translation.data(), scale.data());  // rbf.rs:418-421
-  point_coeff.assign(n * n_cols, 0.0);
-  poly_coeff.assign(m * n_cols, 0.0);
-  const size_t nt = n + m;
+  const double *kp_ptr = M.kernel_points();
+  const double *mono_ptr = M.has_trend ? mono_pts.data() : nullptr;
+  if (m) cheb_cube_scaling(kp_ptr, nullptr, n, dim, M.translation.data(), M.scale.data());  // rbf.rs:418-421
 
-  std::unique_ptr<fb_tree, void (*)(fb_tree *)> tree(nullptr, fb_tree_free);
-  const bool naive = n < params.naive_solve_threshold;
+  const bool naive = n < M.params.naive_solve_threshold;
   const bool verbose = std::getenv("FB_TIMING") != nullptr;
   auto lap = [&](const char *what, clk::time_point &t0) {
     if (verbose) fprintf(stderr, "[fr_fit] %-28s %8.3f s\n", what, std::chrono::duration<double>(clk::now() - t0).count());
@@ -1260,53 +1262,72 @@ void fr_model::fit() {
   // Setup order: the device factorises a DDM level (assembly + batched Cholesky, ~0.15 s for the finest level of a
   // 1M-point fit) while the host builds the next level and then the FMM tree (~0.15 s of host work): the hierarchy comes
   // first, every finished level is queued on a setup stream at once, the tree is built under it.
-  cudaStream_t setup_stream = nullptr;
-  FB_CUDA(cudaStreamCreateWithFlags(&setup_stream, cudaStreamNonBlocking));
-  std::unique_ptr<DeviceSolver> solver(new DeviceSolver(*this, nullptr));
-  solver->s = setup_stream;
-  cudaStream_t stream = setup_stream;
-  try {
-    DeviceSolver &S = *solver;
-    S.upload_points(setup_stream);
-    if (m && !naive) {
-      std::vector<double> Pm(n * m), Qm(n * m);
-      evaluate_monomials(mono_ptr ? mono_ptr : points.data(), nullptr, n, dim, st.polynomial_degree, (int)m, translation.data(),
-                         scale.data(), Pm.data());
-      thin_q_rowmajor(Pm.data(), n, (int)m, Qm.data());
-      S.P.upload(Pm, setup_stream);
-      S.Qp.upload(Qm, setup_stream);
-      S.proj.reserve(m);
-    }
-    lap("points / monomials / thin Q", t_lap);
-    if (naive) {  // single dense domain (rbf.rs:423-454)
-      LevelHost lh;
-      lh.point_indices.resize(n);
-      for (size_t i = 0; i < n; ++i) lh.point_indices[i] = (int64_t)i;
-      DomainHost d;
-      d.idx = lh.point_indices;
-      d.mask.assign(n, 1);
-      d.prepare(kp_ptr, dim, st, true, mono_ptr);
-      lh.domains.push_back(std::move(d));
-      ddm.clear();
-      ddm.push_back(std::move(lh));
-      S.build_level_launch(ddm[0], true, setup_stream);
-    } else {
-      const LevelCallback queue_level = [&](size_t, const LevelHost &level, bool is_coarse) {
-        S.build_level_launch(level, is_coarse, setup_stream);
-      };
-      ddm = build_ddm(kp_ptr, n, dim, st, params, mono_ptr, &queue_level);
-      lap("ddm hierarchy (host) + queued factorisations", t_lap);
-      tree.reset(make_tree(true, nullptr));  // adaptive, sparse, own extents (rbf.rs:456-467)
+  S.s = setup_stream;
+  S.upload_points(setup_stream);
+  if (m && !naive) {
+    std::vector<double> Pm(n * m), Qm(n * m);
+    evaluate_monomials(mono_ptr ? mono_ptr : M.points.data(), nullptr, n, dim, M.st.polynomial_degree, (int)m,
+                       M.translation.data(), M.scale.data(), Pm.data());
+    thin_q_rowmajor(Pm.data(), n, (int)m, Qm.data());
+    S.P.upload(Pm, setup_stream);
+    S.Qp.upload(Qm, setup_stream);
+    S.proj.reserve(m);
+  }
+  lap("points / monomials / thin Q", t_lap);
+  std::vector<LevelHost> &ddm = M.ddm;
+  if (naive) {  // single dense domain (rbf.rs:423-454)
+    LevelHost lh;
+    lh.point_indices.resize(n);
+    for (size_t i = 0; i < n; ++i) lh.point_indices[i] = (int64_t)i;
+    DomainHost d;
+    d.idx = lh.point_indices;
+    d.mask.assign(n, 1);
+    d.prepare(kp_ptr, dim, M.st, true, mono_ptr);
+    lh.domains.push_back(std::move(d));
+    ddm.clear();
+    ddm.push_back(std::move(lh));
+    S.build_level_launch(ddm[0], true, setup_stream);
+  } else {
+    const LevelCallback queue_level = [&](size_t, const LevelHost &level, bool is_coarse) {
+      S.build_level_launch(level, is_coarse, setup_stream);
+    };
+    ddm = build_ddm(kp_ptr, n, dim, M.st, M.params, mono_ptr, &queue_level);
+    lap("ddm hierarchy (host) + queued factorisations", t_lap);
+    if (with_tree) {
+      tree.reset(M.make_tree(true, nullptr));  // adaptive, sparse, own extents (rbf.rs:456-467)
       lap("fmm tree + operators", t_lap);
       S.tree = tree.get();
     }
-    FB_CUDA(cudaStreamSynchronize(setup_stream));
-    if (tree) {  // from here on everything runs on the tree's stream
-      stream = tree->stream;
-      S.s = stream;
-    }
-    for (size_t l = 0; l < ddm.size(); ++l) S.finish_level(l, ddm[l], stream);
-    lap("factorisations finished + level target sets", t_lap);
+  }
+  FB_CUDA(cudaStreamSynchronize(setup_stream));
+  if (tree) S.s = tree->stream;  // from here on everything runs on the tree's stream
+  for (size_t l = 0; l < ddm.size(); ++l) S.finish_level(l, ddm[l], S.s);
+  lap("factorisations finished + level target sets", t_lap);
+}
+
+}  // namespace
+
+void fr_model::fit() {
+  using clk = std::chrono::steady_clock;
+  const auto t_start = clk::now();
+  info = fr_model_info{};
+  info.dim = (uint64_t)dim;
+  info.n_cols = n_cols;
+  info.basis_size = (uint64_t)st.basis_size;
+  const size_t m = (size_t)st.basis_size;
+  const size_t nt = n + m;
+  const bool naive = n < params.naive_solve_threshold;
+  std::vector<double> mono_pts;
+  TreePtr tree(nullptr, fb_tree_free);
+  cudaStream_t setup_stream = nullptr;
+  FB_CUDA(cudaStreamCreateWithFlags(&setup_stream, cudaStreamNonBlocking));
+  std::unique_ptr<DeviceSolver> solver(new DeviceSolver(*this, nullptr));
+  try {
+    DeviceSolver &S = *solver;
+    setup_solve(*this, S, setup_stream, true, mono_pts, tree);
+    const cudaStream_t stream = S.s;
+    point_coeff.assign(n * n_cols, 0.0);
+    poly_coeff.assign(m * n_cols, 0.0);
     info.ddm_levels = ddm.size();
     for (size_t l = 0; l < ddm.size() && l < 8; ++l) info.ddm_domains[l] = ddm[l].domains.size();
     const auto t_setup = clk::now();
@@ -1710,6 +1731,56 @@ int fr_fit(const double *points, size_t n, int dim, ptrdiff_t p_rs, ptrdiff_t p_
                       cb_or_null, user, out);
 }
 
+// fr_fit_trend up to the solve, shared with fr_ddm_level_solve: settings, params and trend checked, the points (and the
+// values, if any) copied and freed of duplicates (rbf.rs:341-359)
+static void init_model(fr_model &M, const double *points, size_t n, int dim, ptrdiff_t p_rs, ptrdiff_t p_cs,
+                       const double *values, size_t n_cols, ptrdiff_t v_rs, ptrdiff_t v_cs, const fr_settings *settings,
+                       const fr_params *params_or_null, const fr_global_trend *trend_or_null) {
+  FB_REQUIRE(dim >= 1 && dim <= 3, "Unsupported number of dimensions: " + std::to_string(dim));  // rbf.rs:329-333
+  M.dim = dim;
+  if (trend_or_null) {
+    FB_REQUIRE(trend_or_null->dim == dim, "GlobalTrend variant does not match the dimensionality of the points");
+    for (int d = 0; d < dim; ++d) FB_REQUIRE(trend_or_null->ratios[d] > 0.0, "GlobalTrend ratios must be positive");
+    M.has_trend = true;
+    M.trend = *trend_or_null;
+  }
+  std::string err;
+  FB_REQUIRE(resolve_settings(*settings, dim, M.st, err), err);
+  FB_REQUIRE(make_kparams(M.st.kparams, M.kp), "unknown kernel");
+  if (params_or_null)
+    M.params = *params_or_null;
+  else
+    fr_params_default(settings->kernel_type, &M.params);
+  std::vector<double> pts(n * dim), vals(n * n_cols);
+  for (size_t i = 0; i < n; ++i) {
+    for (int d = 0; d < dim; ++d) pts[i * dim + d] = points[(ptrdiff_t)i * p_rs + (ptrdiff_t)d * p_cs];
+    for (size_t c = 0; c < n_cols; ++c) vals[i * n_cols + c] = values[(ptrdiff_t)i * v_rs + (ptrdiff_t)c * v_cs];
+  }
+  M.n_in = n;
+  const bool verbose = std::getenv("FB_TIMING") != nullptr;
+  const auto t_dedup = std::chrono::steady_clock::now();
+  if (M.params.test_unique) {  // rbf.rs:341-359
+    std::vector<int64_t> keep = remove_duplicates(pts.data(), n, dim, M.kp);
+    if (keep.size() != n) {
+      M.emit(FR_EVENT_DUPLICATES_REMOVED, n - keep.size(), 0, 0, nullptr);
+      std::vector<double> p2(keep.size() * dim), v2(keep.size() * n_cols);
+      for (size_t k = 0; k < keep.size(); ++k) {
+        std::copy(&pts[keep[k] * dim], &pts[keep[k] * dim] + dim, &p2[k * dim]);
+        std::copy(&vals[keep[k] * n_cols], &vals[keep[k] * n_cols] + n_cols, &v2[k * n_cols]);
+      }
+      pts.swap(p2);
+      vals.swap(v2);
+    }
+  }
+  M.points.swap(pts);
+  M.values.swap(vals);
+  M.n = M.points.size() / dim;
+  M.n_cols = n_cols;
+  if (verbose)
+    fprintf(stderr, "[fr_fit] %-28s %8.3f s\n", "copy + remove_duplicates",
+            std::chrono::duration<double>(std::chrono::steady_clock::now() - t_dedup).count());
+}
+
 int fr_fit_trend(const double *points, size_t n, int dim, ptrdiff_t p_rs, ptrdiff_t p_cs, const double *values,
                  size_t n_cols, ptrdiff_t v_rs, ptrdiff_t v_cs, const fr_settings *settings,
                  const fr_params *params_or_null, const fr_global_trend *trend_or_null, fr_progress_cb cb_or_null,
@@ -1719,53 +1790,10 @@ int fr_fit_trend(const double *points, size_t n, int dim, ptrdiff_t p_rs, ptrdif
   fr_model *M = nullptr;
   const int rc = fr_guarded([&] {
     FB_REQUIRE(points && values && settings && n > 0 && n_cols > 0, "points, values and settings are required");
-    FB_REQUIRE(dim >= 1 && dim <= 3, "Unsupported number of dimensions: " + std::to_string(dim));  // rbf.rs:329-333
     M = new fr_model();
-    M->dim = dim;
-    if (trend_or_null) {
-      FB_REQUIRE(trend_or_null->dim == dim, "GlobalTrend variant does not match the dimensionality of the points");
-      for (int d = 0; d < dim; ++d)
-        FB_REQUIRE(trend_or_null->ratios[d] > 0.0, "GlobalTrend ratios must be positive");
-      M->has_trend = true;
-      M->trend = *trend_or_null;
-    }
     M->cb = cb_or_null;
     M->cb_user = user;
-    std::string err;
-    FB_REQUIRE(resolve_settings(*settings, dim, M->st, err), err);
-    FB_REQUIRE(make_kparams(M->st.kparams, M->kp), "unknown kernel");
-    if (params_or_null)
-      M->params = *params_or_null;
-    else
-      fr_params_default(settings->kernel_type, &M->params);
-    std::vector<double> pts(n * dim), vals(n * n_cols);
-    for (size_t i = 0; i < n; ++i) {
-      for (int d = 0; d < dim; ++d) pts[i * dim + d] = points[(ptrdiff_t)i * p_rs + (ptrdiff_t)d * p_cs];
-      for (size_t c = 0; c < n_cols; ++c) vals[i * n_cols + c] = values[(ptrdiff_t)i * v_rs + (ptrdiff_t)c * v_cs];
-    }
-    M->n_in = n;
-    const bool verbose = std::getenv("FB_TIMING") != nullptr;
-    const auto t_dedup = std::chrono::steady_clock::now();
-    if (M->params.test_unique) {  // rbf.rs:341-359
-      std::vector<int64_t> keep = remove_duplicates(pts.data(), n, dim, M->kp);
-      if (keep.size() != n) {
-        M->emit(FR_EVENT_DUPLICATES_REMOVED, n - keep.size(), 0, 0, nullptr);
-        std::vector<double> p2(keep.size() * dim), v2(keep.size() * n_cols);
-        for (size_t k = 0; k < keep.size(); ++k) {
-          std::copy(&pts[keep[k] * dim], &pts[keep[k] * dim] + dim, &p2[k * dim]);
-          std::copy(&vals[keep[k] * n_cols], &vals[keep[k] * n_cols] + n_cols, &v2[k * n_cols]);
-        }
-        pts.swap(p2);
-        vals.swap(v2);
-      }
-    }
-    M->points.swap(pts);
-    M->values.swap(vals);
-    M->n = M->points.size() / dim;
-    M->n_cols = n_cols;
-    if (verbose)
-      fprintf(stderr, "[fr_fit] %-28s %8.3f s\n", "copy + remove_duplicates",
-              std::chrono::duration<double>(std::chrono::steady_clock::now() - t_dedup).count());
+    init_model(*M, points, n, dim, p_rs, p_cs, values, n_cols, v_rs, v_cs, settings, params_or_null, trend_or_null);
     M->fit();
     M->info.n_duplicates = n - M->n;
     char msg[256];
@@ -2107,6 +2135,52 @@ int fr_dense_spd_solve(const double *a, int n, const double *b, int nrhs, double
       throw;
     }
     cudaStreamDestroy(stream);
+  });
+}
+
+// One DDM level's subdomain solves on nvec residual vectors (n_kept + basis_size each, row after row), set up as fr_fit
+// sets up the solve (duplicate removal, scaling, hierarchy or single dense domain, factorisations) but without an FMM
+// tree: out[v] = solve_level(level, coarse level ? mode 1 : mode 0, add_poly) of res[v], out zeroed first.
+int fr_ddm_level_solve(const double *points, size_t n, int dim, const fr_settings *settings, const fr_params *params_or_null,
+                       int level, int add_poly, const double *res, int nvec, double *out, uint64_t *n_fallback_or_null,
+                       uint64_t *domain_ranks_or_null) {
+  return fr_guarded([&] {
+    FB_REQUIRE(points && settings && res && out && n > 0 && nvec > 0, "fr_ddm_level_solve: bad arguments");
+    fr_model M;
+    init_model(M, points, n, dim, dim, 1, nullptr, 0, 0, 0, settings, params_or_null, nullptr);
+    std::vector<double> mono_pts;
+    TreePtr tree(nullptr, fb_tree_free);
+    cudaStream_t setup_stream = nullptr;
+    FB_CUDA(cudaStreamCreateWithFlags(&setup_stream, cudaStreamNonBlocking));
+    std::unique_ptr<DeviceSolver> solver(new DeviceSolver(M, nullptr));
+    try {
+      DeviceSolver &S = *solver;
+      setup_solve(M, S, setup_stream, false, mono_pts, tree);
+      FB_REQUIRE(level >= 0 && (size_t)level < M.ddm.size(),
+                 "level " + std::to_string(level) + " out of range: the hierarchy has " + std::to_string(M.ddm.size()));
+      const LevelDev &lv = *S.levels[level];
+      const bool coarse = (size_t)level + 1 == M.ddm.size();
+      if (n_fallback_or_null) *n_fallback_or_null = (uint64_t)lv.n_fallback;
+      if (domain_ranks_or_null)
+        for (size_t d = 0; d < M.ddm[level].domains.size(); ++d) domain_ranks_or_null[d] = M.ddm[level].domains[d].rank;
+      const size_t nt = S.nt;
+      DBuf<double> dr, dx;
+      dr.reserve(nt);
+      dx.reserve(nt);
+      for (int v = 0; v < nvec; ++v) {
+        FB_CUDA(cudaMemcpyAsync(dr.p, res + (size_t)v * nt, nt * sizeof(double), cudaMemcpyHostToDevice, S.s));
+        FB_CUDA(cudaMemsetAsync(dx.p, 0, nt * sizeof(double), S.s));
+        S.solve_level(lv, dr.p, dx.p, coarse ? 1 : 0, add_poly, S.s);
+        FB_CUDA(cudaMemcpyAsync(out + (size_t)v * nt, dx.p, nt * sizeof(double), cudaMemcpyDeviceToHost, S.s));
+        FB_CUDA(cudaStreamSynchronize(S.s));
+      }
+    } catch (...) {
+      solver.reset();
+      cudaStreamDestroy(setup_stream);
+      throw;
+    }
+    solver.reset();
+    cudaStreamDestroy(setup_stream);
   });
 }
 

@@ -211,8 +211,19 @@ int fr_host_ddm_level(const fr_host_ddm *h, int level, uint64_t *n_domains, uint
  * (blocked Cholesky with the DMMA trailing update, forward / backward substitution; an indefinite matrix takes the
  * fallback of domain.rs:63-68) -- linalg.rs:638-764 (make_spd) runs against it.  b, x: n x nrhs row-major.
  * fr_evaluate_monomials: polynomials.rs:15-62 / its tests :163-239 (column order [1, x, y, z, x^2, xy, xz, y^2, yz, z^2]);
- * host only, translation / scale may be NULL (0 / 1).                                                               */
+ * host only, translation / scale may be NULL (0 / 1).
+ * fr_ddm_level_solve: the subdomain solves of one DDM level, for tests against dense references.  The points (n x dim,
+ * row-major) go through fr_fit's set-up without the FMM tree: duplicate removal, monomial scaling, the hierarchy (or the
+ * single dense domain below naive_solve_threshold; fr_host_ddm_level shows its domains) and every level's
+ * factorisation.  Then each of the nvec residuals res (n_kept + basis_size rows each, one after the other) is solved on
+ * `level`: fine levels write the point rows of every domain's internal points, the coarse level those of all its points
+ * and, with add_poly, the recovered polynomial into the last `rank` rows; out (same layout) is zeroed first, so rows
+ * nothing writes stay 0.  n_fallback_or_null: domains of the level that took the indefinite fallback;
+ * domain_ranks_or_null: special points per domain (one entry per domain of the level).                            */
 int fr_dense_spd_solve(const double *a, int n, const double *b, int nrhs, double *x, int *used_fallback_or_null);
+int fr_ddm_level_solve(const double *points, size_t n, int dim, const fr_settings *settings, const fr_params *params_or_null,
+                       int level, int add_poly, const double *res, int nvec, double *out, uint64_t *n_fallback_or_null,
+                       uint64_t *domain_ranks_or_null);
 int fr_evaluate_monomials(const double *points, size_t n, int dim, int degree, const double *translation_or_null,
                           const double *scale_or_null, double *out, int *basis_out);
 
