@@ -6,7 +6,7 @@ from .bbfmm import (Communicator, FmmKernelType, FmmParams, FmmTree, KernelParam
                     M2LCompressionType, SpheroidalOrder)
 from . import config, interpolant_config, progress  # noqa: F401,E402
 from .rbf import Coefficients, GlobalTrend, RBFInterpolator  # noqa: F401,E402
-from .isosurface import lattice_isosurface  # noqa: F401,E402
+from .isosurface import Solid, lattice_isosurface, lattice_solid  # noqa: F401,E402
 
 
 def set_sqrt_mode(fast: bool) -> None:

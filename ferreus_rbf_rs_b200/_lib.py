@@ -193,6 +193,10 @@ SOLVER_SIGNATURES = {
     "fr_isosurface_timing": (C.c_int, [C.c_void_p, _dp]),
     "fr_isosurface_refine_stats": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p]),
     "fr_isosurface_free": (None, [C.c_void_p]),
+    "fr_isosurface_extract_solid": (C.c_int, [C.c_void_p, _dp, _u64p, _dp, C.c_int, C.c_int, C.c_int, C.c_int,
+                                              C.POINTER(C.c_void_p)]),
+    "fr_lattice_solid": (C.c_int, [C.c_void_p, _u64p, _dp, C.c_double, C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]),
+    "fr_isosurface_solid_info": (C.c_int, [C.c_void_p, C.c_int, _u64p, _u64p, _dp, _dp]),
     "fr_dense_spd_solve": (C.c_int, [_dp, C.c_int, _dp, C.c_int, _dp, _i32p]),
     "fr_ddm_level_solve": (C.c_int, [_dp, _sz, C.c_int, C.POINTER(FrSettings), C.POINTER(FrParams), C.c_int, C.c_int,
                                      _dp, C.c_int, _dp, _u64p, _u64p]),

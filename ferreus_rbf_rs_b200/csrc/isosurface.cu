@@ -8,6 +8,9 @@
 //  - one vertex per crossing edge, numbered by its edge id 7 p(a) + mask - 1: the node's base (a scan of the
 //    popcounts of the 7-bit crossing masks) plus the popcount of the mask's lower bits;
 //  - triangles in the order (cube, pi, triangle), oriented by kSwap from the below side to the other side.
+// Solids (fr_lattice_solid, fr_isosurface_extract_solid) close that mesh at the lattice box with caps built from the
+// boundary nodes of the solid's side and the existing rim vertices (tests/solid_oracle.py, DESIGN.md "Solids"), and
+// reduce the volume and the isosurface area from the final vertices.
 #include "isosurface.h"
 
 #include <cub/cub.cuh>
@@ -92,7 +95,7 @@ struct NodeVertices {  // vertices owned by node p; 0 past the end (the scan's n
   __host__ __device__ unsigned long long operator()(uint64_t p) const { return p < n ? popc(mask[p] & 0x7fu) : 0; }
 };
 
-struct CubeFaces {
+struct CubeFaces {  // also the cap faces per box-face square
   const uint8_t *count;
   uint64_t n;
   __host__ __device__ unsigned long long operator()(uint64_t c) const { return c < n ? count[c] : 0; }
@@ -203,9 +206,10 @@ __device__ __forceinline__ void tet_pairs(unsigned m, unsigned &t0, unsigned &t1
   t1 = 0;
 }
 
+// flip (the solid above the level set) exchanges every triangle's last two vertices, so that it faces out of the solid
 __global__ void k_iso_triangles(const uint8_t *__restrict__ mask, IsoLattice L,
                                 const unsigned long long *__restrict__ voff, const unsigned long long *__restrict__ foff,
-                                long long *__restrict__ faces) {
+                                bool flip, long long *__restrict__ faces) {
   const uint64_t c = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
   if (c >= L.cubes()) return;
   uint64_t base;
@@ -224,13 +228,273 @@ __global__ void k_iso_triangles(const uint8_t *__restrict__ mask, IsoLattice L,
         const unsigned x = (tp[t] >> (4 * e)) & 3u, y = (tp[t] >> (4 * e + 2)) & 3u;
         vid[e] = tet_vertex(mask, voff, L, base, pi, x < y ? x : y, x < y ? y : x);
       }
-      const bool swap = (kSwap[pi] >> (2 * m + t)) & 1u;
+      const bool swap = (bool)((kSwap[pi] >> (2 * m + t)) & 1u) != flip;
       faces[3 * f] = vid[0];
       faces[3 * f + 1] = swap ? vid[2] : vid[1];
       faces[3 * f + 2] = swap ? vid[1] : vid[2];
       ++f;
     }
   }
+}
+
+// ------------------------------------------------------------------------------------------- solids
+// The caps close the isosurface at the lattice box.  On box face f (0-5: x lo, x hi, y lo, y hi, z lo, z hi; in-plane
+// axes u < v) square (au, av) has index au + (nu - 1) av and the triangles T0 = (a, a + e_u, a + e_u + e_v) and
+// T1 = (a, a + e_v, a + e_u + e_v), the boundary faces of the Kuhn tetrahedra, so every triangle edge is a lattice edge
+// with its vertex already numbered.  A triangle is clipped to the solid's side: one inside corner q against r1 < r2
+// gives (q, e(q,r1), e(q,r2)); two inside corners q1 < q2 against r give (q1, q2, e(q2,r)) and (q1, e(q2,r), e(q1,r));
+// three give the triangle.  Cap vertices are the boundary nodes of the solid's side in ascending node index.
+
+// bit 2 (8 tri + inside mask) + sub-triangle of kCapSwap[box face]: exchange the sub-triangle's last two vertices so
+// that (B-A) x (C-A) points out of the box.  Decided once on the unit square with the crossing points at the edge
+// midpoints (tests/solid_oracle.py, cap_swap_table), like kSwap.
+__constant__ uint32_t kCapSwap[6] = {0x0c1071c4u, 0x71c40c10u, 0x71c40c10u, 0x0c1071c4u, 0x0c1071c4u, 0x71c40c10u};
+
+// the class bit of a node's mask against the solid's side: side 0 holds the below nodes, side 1 the others
+__host__ __device__ __forceinline__ unsigned inside(uint8_t m, unsigned side) { return (unsigned)(m >> 7) ^ side; }
+
+__host__ __device__ __forceinline__ uint64_t boundary_count(const IsoLattice &L) {
+  return L.nodes() - (L.n[0] - 2) * (L.n[1] - 2) * (L.n[2] - 2);
+}
+
+// Boundary nodes in ascending node index: the k = 0 layer, then per inner layer its j = 0 row, the i = 0 and
+// i = nx - 1 nodes of its inner rows and its j = ny - 1 row (2 nx + 2 (ny - 2) nodes), then the k = nz - 1 layer.
+__host__ __device__ __forceinline__ uint64_t boundary_node(const IsoLattice &L, uint64_t b) {
+  const uint64_t nx = L.n[0], ny = L.n[1], layer = nx * ny, ring = 2 * nx + 2 * (ny - 2), inner = (L.n[2] - 2) * ring;
+  if (b < layer) return b;
+  b -= layer;
+  if (b >= inner) return L.nodes() - layer + (b - inner);
+  const uint64_t k = 1 + b / ring, r = b % ring;
+  uint64_t i, j;
+  if (r < nx) {
+    i = r;
+    j = 0;
+  } else if (r >= ring - nx) {
+    i = r - (ring - nx);
+    j = ny - 1;
+  } else {
+    j = 1 + (r - nx) / 2;
+    i = ((r - nx) & 1) ? nx - 1 : 0;
+  }
+  return i + nx * (j + ny * k);
+}
+
+// inverse of boundary_node for a node p on the boundary
+__device__ __forceinline__ uint64_t boundary_rank(const IsoLattice &L, uint64_t p) {
+  const uint64_t nx = L.n[0], ny = L.n[1], layer = nx * ny, ring = 2 * nx + 2 * (ny - 2);
+  const uint64_t i = p % nx, j = (p / nx) % ny, k = p / layer;
+  if (k == 0) return p;
+  if (k == L.n[2] - 1) return layer + (L.n[2] - 2) * ring + (p - k * layer);
+  const uint64_t b = layer + (k - 1) * ring;
+  if (j == 0) return b + i;
+  if (j == ny - 1) return b + ring - nx + i;
+  return b + nx + 2 * (j - 1) + (i != 0);
+}
+
+struct CapNodes {  // 1 for a boundary node of the solid's side; 0 past the end
+  const uint8_t *mask;
+  IsoLattice L;
+  unsigned side;
+  uint64_t n;
+  __host__ __device__ unsigned long long operator()(uint64_t b) const {
+    return b < n ? inside(mask[boundary_node(L, b)], side) : 0;
+  }
+};
+
+// first square of every box face (start[6] = all squares)
+struct CapSquares {
+  uint64_t start[7];
+};
+
+CapSquares cap_squares(const IsoLattice &L) {
+  CapSquares S;
+  S.start[0] = 0;
+  for (int f = 0; f < 6; ++f) {
+    const int w = f / 2, u = w == 0 ? 1 : 0, v = w == 2 ? 1 : 2;
+    S.start[f + 1] = S.start[f] + (L.n[u] - 1) * (L.n[v] - 1);
+  }
+  return S;
+}
+
+__device__ __forceinline__ uint64_t axis_n(const IsoLattice &L, int d) { return d == 0 ? L.n[0] : d == 1 ? L.n[1] : L.n[2]; }
+__device__ __forceinline__ uint64_t axis_stride(const IsoLattice &L, int d) {
+  return d == 0 ? 1 : d == 1 ? L.n[0] : L.n[0] * L.n[1];
+}
+
+// square g of all box faces: its box face, the node of its minimum corner and the edge masks of e_u and e_v
+// (selects rather than indexed arrays keep the kernels free of a stack frame)
+__device__ __forceinline__ int cap_square(const IsoLattice &L, const CapSquares &S, uint64_t g, uint64_t &a,
+                                          unsigned &su, unsigned &sv) {
+  int f = 0;
+  uint64_t first = 0;
+#pragma unroll
+  for (int k = 1; k < 6; ++k)
+    if (g >= S.start[k]) {
+      f = k;
+      first = S.start[k];
+    }
+  const uint64_t q = g - first;
+  const int w = f / 2, u = w == 0 ? 1 : 0, v = w == 2 ? 1 : 2;
+  const uint64_t nu1 = axis_n(L, u) - 1;
+  a = (q % nu1) * axis_stride(L, u) + (q / nu1) * axis_stride(L, v) +
+      ((f & 1) ? (axis_n(L, w) - 1) * axis_stride(L, w) : 0);
+  su = 1u << u;
+  sv = 1u << v;
+  return f;
+}
+
+// corner q of triangle t of a square, as an edge mask from the square's minimum corner: (0, e_u or e_v, e_u + e_v)
+__device__ __forceinline__ unsigned cap_corner(unsigned su, unsigned sv, int t, unsigned q) {
+  return q == 0 ? 0u : q == 1 ? (t ? sv : su) : (su | sv);
+}
+
+// inside mask of triangle t of a square: bit q = corner q is inside
+__device__ __forceinline__ unsigned cap_triangle(const uint8_t *__restrict__ mask, const IsoLattice &L, uint64_t a,
+                                                 unsigned su, unsigned sv, int t, unsigned side) {
+  unsigned m = 0;
+#pragma unroll
+  for (unsigned q = 0; q < 3; ++q) m |= inside(mask[a + node_offset(L, cap_corner(su, sv, t, q))], side) << q;
+  return m;
+}
+
+__device__ __forceinline__ unsigned cap_subtriangles(unsigned m) {
+  const unsigned n = popc(m);
+  return n == 2 ? 2u : n ? 1u : 0u;
+}
+
+__global__ void k_iso_cap_counts(const uint8_t *__restrict__ mask, IsoLattice L, CapSquares S, unsigned side,
+                                 uint8_t *__restrict__ count) {
+  const uint64_t g = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (g >= S.start[6]) return;
+  uint64_t a;
+  unsigned su, sv;
+  cap_square(L, S, g, a, su, sv);
+  count[g] = (uint8_t)(cap_subtriangles(cap_triangle(mask, L, a, su, sv, 0, side)) +
+                       cap_subtriangles(cap_triangle(mask, L, a, su, sv, 1, side)));
+}
+
+__global__ void k_iso_cap_nodes(const uint8_t *__restrict__ mask, IsoLattice L, unsigned side,
+                                const unsigned long long *__restrict__ coff, uint64_t nv, double *__restrict__ verts,
+                                unsigned long long *__restrict__ cap_node) {
+  const uint64_t b = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (b >= boundary_count(L)) return;
+  const uint64_t p = boundary_node(L, b);
+  if (!inside(mask[p], side)) return;
+  const unsigned long long o = coff[b];
+  const uint64_t idx[3] = {p % L.n[0], (p / L.n[0]) % L.n[1], p / (L.n[0] * L.n[1])};
+#pragma unroll
+  for (int d = 0; d < 3; ++d) verts[3 * (nv + o) + d] = coord(L, d, idx[d]);
+  cap_node[o] = p;
+}
+
+__global__ void k_iso_cap_faces(const uint8_t *__restrict__ mask, IsoLattice L, CapSquares S, unsigned side,
+                                const unsigned long long *__restrict__ voff, const unsigned long long *__restrict__ coff,
+                                const unsigned long long *__restrict__ soff, uint64_t nv, uint64_t nf,
+                                long long *__restrict__ faces) {
+  const uint64_t g = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (g >= S.start[6]) return;
+  uint64_t a;
+  unsigned su, sv;
+  const int f = cap_square(L, S, g, a, su, sv);
+  unsigned long long o = nf + soff[g];
+#pragma unroll
+  for (int t = 0; t < 2; ++t) {
+    const unsigned m = cap_triangle(mask, L, a, su, sv, t, side);
+    if (!m) continue;
+    auto node = [&](unsigned q) {
+      return (long long)(nv + coff[boundary_rank(L, a + node_offset(L, cap_corner(su, sv, t, q)))]);
+    };
+    auto rim = [&](unsigned q, unsigned r) {  // vertex of the edge between corners q and r, numbered as tet_vertex
+      const unsigned cl = cap_corner(su, sv, t, q < r ? q : r), s = cap_corner(su, sv, t, q < r ? r : q) & ~cl;
+      const uint64_t x = a + node_offset(L, cl);
+      return (long long)(voff[x] + popc(mask[x] & ((1u << (s - 1)) - 1u)));
+    };
+    long long v0[3], v1[3];
+    const unsigned n = popc(m);
+    if (n == 3) {
+      v0[0] = node(0);
+      v0[1] = node(1);
+      v0[2] = node(2);
+    } else {
+      const unsigned lone = n == 1 ? m : ~m & 7u, q = __ffs(lone) - 1, r1 = __ffs(7u & ~lone) - 1,
+                     r2 = 31 - __clz(7u & ~lone);
+      if (n == 1) {
+        v0[0] = node(q);
+        v0[1] = rim(q, r1);
+        v0[2] = rim(q, r2);
+      } else {  // inside r1 < r2, outside q
+        v0[0] = node(r1);
+        v0[1] = node(r2);
+        v0[2] = rim(r2, q);
+        v1[0] = v0[0];
+        v1[1] = v0[2];
+        v1[2] = rim(r1, q);
+      }
+    }
+#pragma unroll
+    for (unsigned k = 0; k < 2; ++k) {
+      if (k == 1 && n != 2) break;
+      const long long *vid = k ? v1 : v0;
+      const bool swap = (kCapSwap[f] >> (2 * (8 * t + m) + k)) & 1u;
+      faces[3 * o] = vid[0];
+      faces[3 * o + 1] = swap ? vid[2] : vid[1];
+      faces[3 * o + 2] = swap ? vid[1] : vid[2];
+      ++o;
+    }
+  }
+}
+
+// 6 x the signed volume of the tetrahedron (o, A, B, C)
+struct FaceVolume {
+  const double *v;
+  const long long *f;
+  double o[3];
+  __host__ __device__ double operator()(uint64_t i) const {
+    double x[3][3];
+    for (int e = 0; e < 3; ++e)
+      for (int d = 0; d < 3; ++d) x[e][d] = v[3 * f[3 * i + e] + d] - o[d];
+    return x[0][0] * (x[1][1] * x[2][2] - x[1][2] * x[2][1]) + x[0][1] * (x[1][2] * x[2][0] - x[1][0] * x[2][2]) +
+           x[0][2] * (x[1][0] * x[2][1] - x[1][1] * x[2][0]);
+  }
+};
+
+// 2 x the area of face i
+struct FaceArea {
+  const double *v;
+  const long long *f;
+  __host__ __device__ double operator()(uint64_t i) const {
+    const double *a = v + 3 * f[3 * i], *b = v + 3 * f[3 * i + 1], *c = v + 3 * f[3 * i + 2];
+    const double p[3] = {b[0] - a[0], b[1] - a[1], b[2] - a[2]}, q[3] = {c[0] - a[0], c[1] - a[1], c[2] - a[2]};
+    const double x = p[1] * q[2] - p[2] * q[1], y = p[2] * q[0] - p[0] * q[2], z = p[0] * q[1] - p[1] * q[0];
+    return sqrt(x * x + y * y + z * z);
+  }
+};
+
+template <class F>
+void reduce_sum(F f, uint64_t n, double *out, IsoScratch &w, cudaStream_t s) {
+  auto in = thrust::make_transform_iterator(thrust::counting_iterator<uint64_t>(0), f);
+  size_t bytes = 0;
+  FB_CUDA(cub::DeviceReduce::Sum(nullptr, bytes, in, out, (int64_t)n, s));
+  w.cub.reserve(bytes);
+  FB_CUDA(cub::DeviceReduce::Sum(w.cub.p, bytes, in, out, (int64_t)n, s));
+  g_launches.fetch_add(1);
+}
+
+__global__ void k_iso_cap_normals(IsoLattice L, const unsigned long long *__restrict__ cap_node, uint64_t cv,
+                                  double *__restrict__ nrm) {
+  const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
+  if (i >= cv) return;
+  const uint64_t p = cap_node[i];
+  const uint64_t idx[3] = {p % L.n[0], (p / L.n[0]) % L.n[1], p / (L.n[0] * L.n[1])};
+  double n[3], len = 0.0;
+#pragma unroll
+  for (int d = 0; d < 3; ++d) {
+    n[d] = idx[d] == 0 ? -1.0 : idx[d] == L.n[d] - 1 ? 1.0 : 0.0;
+    len += n[d] * n[d];
+  }
+  const double inv = 1.0 / sqrt(len);
+#pragma unroll
+  for (int d = 0; d < 3; ++d) nrm[3 * i + d] = n[d] * inv;
 }
 
 // ------------------------------------------------------------------------------------------- refinement
@@ -297,14 +561,15 @@ __global__ void k_iso_refine_update(const double *__restrict__ vals, int n_cols,
   keep[i] = !done;
 }
 
-__global__ void k_iso_normals(const double *__restrict__ g, int n_cols, int col, uint64_t nv,
+// negate: the solid above the level set, whose outward normal is the negated gradient
+__global__ void k_iso_normals(const double *__restrict__ g, int n_cols, int col, uint64_t nv, bool negate,
                               double *__restrict__ nrm) {
   const uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
   if (i >= nv) return;
   const double *gi = g + i * (uint64_t)(3 * n_cols) + 3 * col;
   const double x = gi[0], y = gi[1], z = gi[2];
   const double len = sqrt(x * x + y * y + z * z);
-  const double inv = len > 0.0 ? 1.0 / len : 0.0;
+  const double inv = len > 0.0 ? (negate ? -1.0 : 1.0) / len : 0.0;
   nrm[3 * i] = x * inv;
   nrm[3 * i + 1] = y * inv;
   nrm[3 * i + 2] = z * inv;
@@ -351,6 +616,11 @@ uint64_t iso_first_nonfinite(const double *d_v, size_t stride, uint64_t n, IsoSc
 void iso_extract(const double *d_v, size_t stride, const IsoLattice &L, IsoScratch &w, IsoSurface &out,
                  cudaStream_t s) {
   const uint64_t n = L.nodes(), nc = L.cubes();
+  const bool solid = out.side != kIsoOpen;
+  const unsigned side = solid ? (unsigned)out.side : 0u;
+  const uint64_t nb = boundary_count(L);
+  const CapSquares S = cap_squares(L);
+  const uint64_t ns = S.start[6];
   w.mask.reserve(n);
   w.voff.reserve(n + 1);
   w.ccount.reserve(nc);
@@ -359,22 +629,42 @@ void iso_extract(const double *d_v, size_t stride, const IsoLattice &L, IsoScrat
   scan_counts(NodeVertices{w.mask.p, n}, n, w.voff.p, w, s);
   FB_LAUNCH(k_iso_cube_counts, nblocks(nc, 256), 256, 0, s, w.mask.p, L, w.ccount.p);
   scan_counts(CubeFaces{w.ccount.p, nc}, nc, w.foff.p, w, s);
-  unsigned long long tot[2] = {0, 0};
+  unsigned long long tot[4] = {0, 0, 0, 0};
   FB_CUDA(cudaMemcpyAsync(&tot[0], w.voff.p + n, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
   FB_CUDA(cudaMemcpyAsync(&tot[1], w.foff.p + nc, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  if (solid) {
+    w.coff.reserve(nb + 1);
+    w.scount.reserve(ns);
+    w.soff.reserve(ns + 1);
+    scan_counts(CapNodes{w.mask.p, L, side, nb}, nb, w.coff.p, w, s);
+    FB_LAUNCH(k_iso_cap_counts, nblocks(ns, 256), 256, 0, s, w.mask.p, L, S, side, w.scount.p);
+    scan_counts(CubeFaces{w.scount.p, ns}, ns, w.soff.p, w, s);
+    FB_CUDA(cudaMemcpyAsync(&tot[2], w.coff.p + nb, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    FB_CUDA(cudaMemcpyAsync(&tot[3], w.soff.p + ns, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+  }
   FB_CUDA(cudaStreamSynchronize(s));
   out.nv = tot[0];
   out.nf = tot[1];
+  out.cv = tot[2];
+  out.cf = tot[3];
+  if (out.nv + out.cv) out.verts.reserve(3 * (out.nv + out.cv));
   if (out.nv) {
-    out.verts.reserve(3 * out.nv);
     out.edge.reserve(out.nv);
     FB_LAUNCH(k_iso_vertices, nblocks(n, 256), 256, 0, s, d_v, stride, L, out.iso, w.mask.p, w.voff.p, out.verts.p,
               out.edge.p);
   }
-  if (out.nf) {
-    out.faces.reserve(3 * out.nf);
-    FB_LAUNCH(k_iso_triangles, nblocks(nc, 256), 256, 0, s, w.mask.p, L, w.voff.p, w.foff.p, out.faces.p);
+  if (out.cv) {
+    out.cap_node.reserve(out.cv);
+    FB_LAUNCH(k_iso_cap_nodes, nblocks(nb, 256), 256, 0, s, w.mask.p, L, side, w.coff.p, out.nv, out.verts.p,
+              out.cap_node.p);
   }
+  if (out.nf + out.cf) out.faces.reserve(3 * (out.nf + out.cf));
+  if (out.nf)
+    FB_LAUNCH(k_iso_triangles, nblocks(nc, 256), 256, 0, s, w.mask.p, L, w.voff.p, w.foff.p, solid && side == 1,
+              out.faces.p);
+  if (out.cf)
+    FB_LAUNCH(k_iso_cap_faces, nblocks(ns, 256), 256, 0, s, w.mask.p, L, S, side, w.voff.p, w.coff.p, w.soff.p, out.nv,
+              out.nf, out.faces.p);
 }
 
 void iso_refine(const double *d_v, size_t stride, const IsoLattice &L, int n_cols, int col, const IsoEval &eval,
@@ -413,11 +703,29 @@ void iso_refine(const double *d_v, size_t stride, const IsoLattice &L, int n_col
   }
 }
 
-void iso_normals(const double *d_grads, int n_cols, int col, IsoSurface &surf, cudaStream_t s) {
+void iso_normals(const double *d_grads, int n_cols, int col, const IsoLattice &L, IsoSurface &surf, cudaStream_t s) {
   surf.has_normals = true;
-  if (!surf.nv) return;
-  surf.normals.reserve(3 * surf.nv);
-  FB_LAUNCH(k_iso_normals, nblocks(surf.nv, 256), 256, 0, s, d_grads, n_cols, col, surf.nv, surf.normals.p);
+  if (!surf.nv && !surf.cv) return;
+  surf.normals.reserve(3 * (surf.nv + surf.cv));
+  if (surf.nv)
+    FB_LAUNCH(k_iso_normals, nblocks(surf.nv, 256), 256, 0, s, d_grads, n_cols, col, surf.nv, surf.side == 1,
+              surf.normals.p);
+  if (surf.cv)
+    FB_LAUNCH(k_iso_cap_normals, nblocks(surf.cv, 256), 256, 0, s, L, surf.cap_node.p, surf.cv,
+              surf.normals.p + 3 * surf.nv);
+}
+
+void iso_measure(const IsoLattice &L, IsoScratch &w, IsoSurface &surf, cudaStream_t s) {
+  w.sums.reserve(2);
+  FB_CUDA(cudaMemsetAsync(w.sums.p, 0, 2 * sizeof(double), s));
+  if (surf.nf + surf.cf)  // relative to the lattice's lo corner: at UTM coordinates the products would cancel
+    reduce_sum(FaceVolume{surf.verts.p, surf.faces.p, {L.lo[0], L.lo[1], L.lo[2]}}, surf.nf + surf.cf, w.sums.p, w, s);
+  if (surf.nf) reduce_sum(FaceArea{surf.verts.p, surf.faces.p}, surf.nf, w.sums.p + 1, w, s);
+  double h[2] = {0, 0};
+  FB_CUDA(cudaMemcpyAsync(h, w.sums.p, sizeof(h), cudaMemcpyDeviceToHost, s));
+  FB_CUDA(cudaStreamSynchronize(s));
+  surf.volume = h[0] / 6.0;
+  surf.area = 0.5 * h[1];
 }
 
 }  // namespace fb
@@ -434,53 +742,83 @@ const IsoSurface &surface_of(const fr_isosurface *h, int which) {
 }
 }  // namespace
 
+namespace {
+// the mesh of fr_lattice_isosurface (side kIsoOpen) or the solid of fr_lattice_solid
+void lattice_mesh(const double *d_values, const uint64_t *resolution, const double *extents, double isovalue, int side,
+                  void *stream, fr_isosurface **out) {
+  FB_REQUIRE(out, "output handle required");
+  *out = nullptr;
+  FB_REQUIRE(d_values, "values must be an nz x ny x nx device array");
+  const IsoLattice L = iso_lattice(extents, resolution);
+  FB_REQUIRE(std::isfinite(isovalue), "isovalue must be finite");
+  int device = 0;
+  FB_CUDA(cudaGetDevice(&device));
+  require_device_matrix(d_values, L.nodes(), 1, 1, 1, device, "values");
+  const auto t0 = std::chrono::steady_clock::now();
+  auto h = std::make_unique<fr_isosurface>();
+  h->device = device;
+  const cudaStream_t s = (cudaStream_t)stream;
+  IsoScratch w;
+  const uint64_t bad = iso_first_nonfinite(d_values, 1, L.nodes(), w, s);
+  FB_REQUIRE(bad == L.nodes(), "lattice value " + std::to_string(bad) + " is not finite");
+  h->surf.push_back(std::make_unique<IsoSurface>());
+  h->surf[0]->iso = isovalue;
+  h->surf[0]->side = side;
+  iso_extract(d_values, 1, L, w, *h->surf[0], s);
+  if (side != kIsoOpen) iso_measure(L, w, *h->surf[0], s);
+  FB_CUDA(cudaStreamSynchronize(s));
+  h->ms[1] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  *out = h.release();
+}
+}  // namespace
+
 extern "C" {
 
 int fr_lattice_isosurface(const double *d_values, const uint64_t *resolution, const double *extents, double isovalue,
                           void *stream, fr_isosurface **out) {
+  return guarded([&] { lattice_mesh(d_values, resolution, extents, isovalue, kIsoOpen, stream, out); });
+}
+
+int fr_lattice_solid(const double *d_values, const uint64_t *resolution, const double *extents, double isovalue,
+                     int side, void *stream, fr_isosurface **out) {
   return guarded([&] {
-    FB_REQUIRE(out, "output handle required");
-    *out = nullptr;
-    FB_REQUIRE(d_values, "values must be an nz x ny x nx device array");
-    const IsoLattice L = iso_lattice(extents, resolution);
-    FB_REQUIRE(std::isfinite(isovalue), "isovalue must be finite");
-    int device = 0;
-    FB_CUDA(cudaGetDevice(&device));
-    require_device_matrix(d_values, L.nodes(), 1, 1, 1, device, "values");
-    const auto t0 = std::chrono::steady_clock::now();
-    auto h = std::make_unique<fr_isosurface>();
-    h->device = device;
-    const cudaStream_t s = (cudaStream_t)stream;
-    IsoScratch w;
-    const uint64_t bad = iso_first_nonfinite(d_values, 1, L.nodes(), w, s);
-    FB_REQUIRE(bad == L.nodes(), "lattice value " + std::to_string(bad) + " is not finite");
-    h->surf.push_back(std::make_unique<IsoSurface>());
-    h->surf[0]->iso = isovalue;
-    iso_extract(d_values, 1, L, w, *h->surf[0], s);
-    FB_CUDA(cudaStreamSynchronize(s));
-    h->ms[1] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    *out = h.release();
+    if (out) *out = nullptr;
+    FB_REQUIRE(side == 0 || side == 1, "side must be 0 (below) or 1 (above)");
+    lattice_mesh(d_values, resolution, extents, isovalue, side, stream, out);
   });
 }
 
 int fr_isosurface_counts(const fr_isosurface *s, int which, uint64_t *n_vertices, uint64_t *n_faces) {
   return guarded([&] {
     const IsoSurface &f = surface_of(s, which);
-    if (n_vertices) *n_vertices = f.nv;
-    if (n_faces) *n_faces = f.nf;
+    if (n_vertices) *n_vertices = f.nv + f.cv;
+    if (n_faces) *n_faces = f.nf + f.cf;
   });
 }
 
 int fr_isosurface_copy(const fr_isosurface *s, int which, double *vertices, int64_t *faces, double *normals_or_null) {
   return guarded([&] {
     const IsoSurface &f = surface_of(s, which);
-    FB_REQUIRE((vertices || !f.nv) && (faces || !f.nf), "vertices and faces outputs are required");
+    const uint64_t nv = f.nv + f.cv, nf = f.nf + f.cf;
+    FB_REQUIRE((vertices || !nv) && (faces || !nf), "vertices and faces outputs are required");
     FB_REQUIRE(!normals_or_null || f.has_normals, "this isosurface has no normals: lattice values carry no gradient");
     FB_CUDA(cudaSetDevice(s->device));
-    if (f.nv) FB_CUDA(cudaMemcpy(vertices, f.verts.p, 3 * f.nv * sizeof(double), cudaMemcpyDefault));
-    if (f.nf) FB_CUDA(cudaMemcpy(faces, f.faces.p, 3 * f.nf * sizeof(int64_t), cudaMemcpyDefault));
-    if (normals_or_null && f.nv)
-      FB_CUDA(cudaMemcpy(normals_or_null, f.normals.p, 3 * f.nv * sizeof(double), cudaMemcpyDefault));
+    if (nv) FB_CUDA(cudaMemcpy(vertices, f.verts.p, 3 * nv * sizeof(double), cudaMemcpyDefault));
+    if (nf) FB_CUDA(cudaMemcpy(faces, f.faces.p, 3 * nf * sizeof(int64_t), cudaMemcpyDefault));
+    if (normals_or_null && nv)
+      FB_CUDA(cudaMemcpy(normals_or_null, f.normals.p, 3 * nv * sizeof(double), cudaMemcpyDefault));
+  });
+}
+
+int fr_isosurface_solid_info(const fr_isosurface *s, int which, uint64_t *surface_vertices, uint64_t *surface_faces,
+                             double *volume, double *surface_area) {
+  return guarded([&] {
+    const IsoSurface &f = surface_of(s, which);
+    FB_REQUIRE(f.side != kIsoOpen, "this handle holds open isosurfaces, not solids");
+    if (surface_vertices) *surface_vertices = f.nv;
+    if (surface_faces) *surface_faces = f.nf;
+    if (volume) *volume = f.volume;
+    if (surface_area) *surface_area = f.area;
   });
 }
 

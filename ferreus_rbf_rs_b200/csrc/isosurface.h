@@ -21,14 +21,20 @@ struct IsoLattice {
 // FB_ERR_INVALID_ARGUMENT unless lo < hi (finite) and n >= 2 on every axis and the node count is at most kIsoMaxNodes
 IsoLattice iso_lattice(const double *extents, const uint64_t *resolution);
 
+constexpr int kIsoOpen = -1;  // IsoSurface::side of an open isosurface; 0 = the solid {f < iso}, 1 = {f >= iso}
+
 struct IsoSurface {
   double iso = 0;
-  uint64_t nv = 0, nf = 0;
-  DBuf<double> verts, normals;       // nv x 3 row-major
-  DBuf<long long> faces;             // nf x 3 row-major
-  DBuf<unsigned long long> edge;     // edge id of every vertex, 7 p(a) + mask - 1
+  int side = kIsoOpen;
+  uint64_t nv = 0, nf = 0;           // isosurface vertices and faces
+  uint64_t cv = 0, cf = 0;           // solids: cap nodes and cap faces, after the isosurface's in verts and faces
+  DBuf<double> verts, normals;       // (nv + cv) x 3 row-major
+  DBuf<long long> faces;             // (nf + cf) x 3 row-major
+  DBuf<unsigned long long> edge;     // edge id of every isosurface vertex, 7 p(a) + mask - 1
+  DBuf<unsigned long long> cap_node; // lattice node of every cap vertex
   bool has_normals = false;
   uint64_t evaluations = 0, max_iterations = 0;  // refinement: trial points evaluated, iterations of the slowest vertex
+  double volume = 0, area = 0;       // solids: enclosed volume, area of the isosurface faces
 };
 
 // regula falsi state of one vertex: bracket [ta, tb] on its edge a -> b with f - iso at both ends, next trial t
@@ -48,21 +54,28 @@ struct IsoScratch {
   DBuf<int> n_sel;
   DBuf<IsoRefine> state;
   DBuf<double> pts, vals;
+  DBuf<unsigned long long> coff, soff;      // solids: cap node offsets per boundary node, cap face offsets per square
+  DBuf<uint8_t> scount;                     // solids: cap faces per box-face square
+  DBuf<double> sums;                        // solids: volume and area sums
 };
 
 // node coordinates, n x 3 row-major, node p = i + nx * (j + ny * k)
 void iso_lattice_points(const IsoLattice &L, double *d_xyz, cudaStream_t s);
 // index of the first non-finite value of d_v[p * stride], or the node count when all are finite; blocks
 uint64_t iso_first_nonfinite(const double *d_v, size_t stride, uint64_t n, IsoScratch &w, cudaStream_t s);
-// vertices and faces of the level set `out.iso` of the lattice values d_v[p * stride]; blocks for the counts
+// vertices and faces of the level set `out.iso` of the lattice values d_v[p * stride], and for out.side >= 0 the cap
+// nodes and faces that close it into a solid; blocks once for the counts
 void iso_extract(const double *d_v, size_t stride, const IsoLattice &L, IsoScratch &w, IsoSurface &out, cudaStream_t s);
 // evaluates the interpolant at m points (m x 3 row-major, device) into vals (m x n_cols row-major, device), on s
 using IsoEval = std::function<void(const double *pts, size_t m, double *vals)>;
 // Illinois regula falsi on every vertex's edge, the lattice values as the first bracket
 void iso_refine(const double *d_v, size_t stride, const IsoLattice &L, int n_cols, int col, const IsoEval &eval,
                 IsoScratch &w, IsoSurface &surf, cudaStream_t s);
-// normals[v] = gradient of column col at vertex v (d_grads: nv x (n_cols * 3) row-major), normalised
-void iso_normals(const double *d_grads, int n_cols, int col, IsoSurface &surf, cudaStream_t s);
+// normals[v] = gradient of column col at vertex v (d_grads: nv x (n_cols * 3) row-major), normalised; for solids negated
+// on side 1, and on the cap nodes the normalised sum of the outward normals of the box faces they lie on
+void iso_normals(const double *d_grads, int n_cols, int col, const IsoLattice &L, IsoSurface &surf, cudaStream_t s);
+// solids: volume and isosurface area from the final vertex positions, by fixed-order reductions; blocks
+void iso_measure(const IsoLattice &L, IsoScratch &w, IsoSurface &surf, cudaStream_t s);
 
 }  // namespace fb
 

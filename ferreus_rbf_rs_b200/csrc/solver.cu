@@ -1999,75 +1999,92 @@ int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_ta
   });
 }
 
+// the meshes of fr_isosurface_extract (side kIsoOpen) or the solids of fr_isosurface_extract_solid
+static void extract_meshes(fr_model *m, const double *extents, const uint64_t *resolution, const double *isovalues,
+                           int n_iso, int column, int refine, int side, fr_isosurface **out) {
+  FB_REQUIRE(out, "output handle required");
+  *out = nullptr;
+  FB_REQUIRE(m, "model required");
+  FB_REQUIRE(m->dim == 3, "isosurfaces need a 3-D model, this one is " + std::to_string(m->dim) + "-D");
+  const IsoLattice L = iso_lattice(extents, resolution);
+  FB_REQUIRE(isovalues && n_iso >= 1, "at least one isovalue is required");
+  for (int i = 0; i < n_iso; ++i) FB_REQUIRE(std::isfinite(isovalues[i]), "isovalues must be finite");
+  FB_REQUIRE(column >= 0 && (size_t)column < m->n_cols,
+             "column " + std::to_string(column) + " is out of range for " + std::to_string(m->n_cols) +
+                 " value column(s)");
+  using clk = std::chrono::steady_clock;
+  auto ms = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
+  const auto t0 = clk::now();
+  // one transient tree over the union of the lattice and the source points, as fr_evaluate_device; the lattice, every
+  // refinement batch and the normals are served from its leaf pass
+  double ext[6] = {L.lo[0], L.lo[1], L.lo[2], L.hi[0], L.hi[1], L.hi[2]};
+  m->evaluation_extents(ext, ext);
+  auto tree = m->transient_tree(false, ext);
+  fb_tree *t = tree.get();
+  t->downward(t->d_flag_all.p);
+  const cudaStream_t s = t->stream;
+  const uint64_t nodes = L.nodes();
+  const size_t nc = m->n_cols;
+  DBuf<double> xyz, vals;
+  xyz.reserve(3 * nodes);
+  vals.reserve(nodes * nc);
+  iso_lattice_points(L, xyz.p, s);
+  m->eval_tree(t, xyz.p, nodes, 3, 1, true, false, vals.p, nullptr);
+  IsoScratch w;
+  const double *v = vals.p + column;  // column `column` of the lattice values, stride n_cols
+  const uint64_t bad = iso_first_nonfinite(v, nc, nodes, w, s);
+  FB_REQUIRE(bad == nodes, "the interpolant is not finite at lattice node " + std::to_string(bad));
+  const auto t1 = clk::now();
+  auto h = std::make_unique<fr_isosurface>();
+  h->device = t->device;
+  for (int i = 0; i < n_iso; ++i) {
+    h->surf.push_back(std::make_unique<IsoSurface>());
+    h->surf.back()->iso = isovalues[i];
+    h->surf.back()->side = side;
+    iso_extract(v, nc, L, w, *h->surf.back(), s);
+  }
+  FB_CUDA(cudaStreamSynchronize(s));
+  const auto t2 = clk::now();
+  if (refine) {
+    const IsoEval eval = [&](const double *pts, size_t cnt, double *out_vals) {
+      m->eval_tree(t, pts, cnt, 3, 1, true, false, out_vals, nullptr);
+    };
+    for (auto &f : h->surf) iso_refine(v, nc, L, (int)nc, column, eval, w, *f, s);
+  }
+  if (side != kIsoOpen)  // from the final vertex positions
+    for (auto &f : h->surf) iso_measure(L, w, *f, s);
+  FB_CUDA(cudaStreamSynchronize(s));
+  const auto t3 = clk::now();
+  DBuf<double> gv, gg;
+  for (auto &f : h->surf) {
+    if (f->nv) {
+      gv.reserve(f->nv * nc);
+      gg.reserve(f->nv * nc * 3);
+      m->eval_tree(t, f->verts.p, f->nv, 3, 1, true, false, gv.p, gg.p);
+    }
+    iso_normals(gg.p, (int)nc, column, L, *f, s);
+  }
+  FB_CUDA(cudaStreamSynchronize(s));
+  const auto t4 = clk::now();
+  h->ms[0] = ms(t0, t1);
+  h->ms[1] = ms(t1, t2);
+  h->ms[2] = ms(t2, t3);
+  h->ms[3] = ms(t3, t4);
+  *out = h.release();
+}
+
 int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *resolution, const double *isovalues,
                           int n_iso, int column, int refine, fr_isosurface **out) {
+  return fr_guarded([&] { extract_meshes(m, extents, resolution, isovalues, n_iso, column, refine, kIsoOpen, out); });
+}
+
+int fr_isosurface_extract_solid(fr_model *m, const double *extents, const uint64_t *resolution,
+                                const double *isovalues, int n_iso, int column, int refine, int side,
+                                fr_isosurface **out) {
   return fr_guarded([&] {
-    FB_REQUIRE(out, "output handle required");
-    *out = nullptr;
-    FB_REQUIRE(m, "model required");
-    FB_REQUIRE(m->dim == 3, "isosurfaces need a 3-D model, this one is " + std::to_string(m->dim) + "-D");
-    const IsoLattice L = iso_lattice(extents, resolution);
-    FB_REQUIRE(isovalues && n_iso >= 1, "at least one isovalue is required");
-    for (int i = 0; i < n_iso; ++i) FB_REQUIRE(std::isfinite(isovalues[i]), "isovalues must be finite");
-    FB_REQUIRE(column >= 0 && (size_t)column < m->n_cols,
-               "column " + std::to_string(column) + " is out of range for " + std::to_string(m->n_cols) +
-                   " value column(s)");
-    using clk = std::chrono::steady_clock;
-    auto ms = [](clk::time_point a, clk::time_point b) { return std::chrono::duration<double, std::milli>(b - a).count(); };
-    const auto t0 = clk::now();
-    // one transient tree over the union of the lattice and the source points, as fr_evaluate_device; the lattice, every
-    // refinement batch and the normals are served from its leaf pass
-    double ext[6] = {L.lo[0], L.lo[1], L.lo[2], L.hi[0], L.hi[1], L.hi[2]};
-    m->evaluation_extents(ext, ext);
-    auto tree = m->transient_tree(false, ext);
-    fb_tree *t = tree.get();
-    t->downward(t->d_flag_all.p);
-    const cudaStream_t s = t->stream;
-    const uint64_t nodes = L.nodes();
-    const size_t nc = m->n_cols;
-    DBuf<double> xyz, vals;
-    xyz.reserve(3 * nodes);
-    vals.reserve(nodes * nc);
-    iso_lattice_points(L, xyz.p, s);
-    m->eval_tree(t, xyz.p, nodes, 3, 1, true, false, vals.p, nullptr);
-    IsoScratch w;
-    const double *v = vals.p + column;  // column `column` of the lattice values, stride n_cols
-    const uint64_t bad = iso_first_nonfinite(v, nc, nodes, w, s);
-    FB_REQUIRE(bad == nodes, "the interpolant is not finite at lattice node " + std::to_string(bad));
-    const auto t1 = clk::now();
-    auto h = std::make_unique<fr_isosurface>();
-    h->device = t->device;
-    for (int i = 0; i < n_iso; ++i) {
-      h->surf.push_back(std::make_unique<IsoSurface>());
-      h->surf.back()->iso = isovalues[i];
-      iso_extract(v, nc, L, w, *h->surf.back(), s);
-    }
-    FB_CUDA(cudaStreamSynchronize(s));
-    const auto t2 = clk::now();
-    if (refine) {
-      const IsoEval eval = [&](const double *pts, size_t cnt, double *out_vals) {
-        m->eval_tree(t, pts, cnt, 3, 1, true, false, out_vals, nullptr);
-      };
-      for (auto &f : h->surf) iso_refine(v, nc, L, (int)nc, column, eval, w, *f, s);
-    }
-    FB_CUDA(cudaStreamSynchronize(s));
-    const auto t3 = clk::now();
-    DBuf<double> gv, gg;
-    for (auto &f : h->surf) {
-      if (f->nv) {
-        gv.reserve(f->nv * nc);
-        gg.reserve(f->nv * nc * 3);
-        m->eval_tree(t, f->verts.p, f->nv, 3, 1, true, false, gv.p, gg.p);
-      }
-      iso_normals(gg.p, (int)nc, column, *f, s);
-    }
-    FB_CUDA(cudaStreamSynchronize(s));
-    const auto t4 = clk::now();
-    h->ms[0] = ms(t0, t1);
-    h->ms[1] = ms(t1, t2);
-    h->ms[2] = ms(t2, t3);
-    h->ms[3] = ms(t3, t4);
-    *out = h.release();
+    if (out) *out = nullptr;
+    FB_REQUIRE(side == 0 || side == 1, "side must be 0 (below) or 1 (above)");
+    extract_meshes(m, extents, resolution, isovalues, n_iso, column, refine, side, out);
   });
 }
 

@@ -1,6 +1,7 @@
 """Isosurface meshes of lattices and of fitted 3-D interpolants (fr_isosurface_* / fr_lattice_isosurface,
 include/ferreus_rbf_b200.h).  The meshes are built and held on the GPU; this module reads them out of the handle."""
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 
@@ -20,6 +21,19 @@ def lattice_args(extents, resolution):
         raise ValueError("resolution must be an int or a 3-tuple")
     # a negative count cannot be a uint64: pass 0, which the library rejects with the other counts below 2
     return ext, np.array([max(int(r), 0) for r in res], dtype=np.uint64)
+
+
+Solid = namedtuple("Solid", "vertices faces normals volume surface_area n_surface_vertices n_surface_faces")
+Solid.__doc__ = """A level set closed at the lattice box into a solid: vertices (V, 3) float64, faces (F, 3) int64 pointing out of
+the solid, normals (V, 3) float64 or None; the first n_surface_vertices / n_surface_faces rows are the isosurface, the
+rest the caps on the box faces.  volume is the enclosed volume, surface_area the area of the isosurface faces."""
+
+
+def side_code(side):
+    """0 for "below" (the region {f < iso}, the inside of a signed distance), 1 for "above" ({f >= iso})"""
+    if isinstance(side, str) and side in ("below", "above"):
+        return 0 if side == "below" else 1
+    raise ValueError(f'side must be "below" or "above", not {side!r}')
 
 
 def check(rc):
@@ -67,6 +81,13 @@ class Handle:
         check(_lib.lib().fr_isosurface_timing(self.h, _lib.dptr(ms)))
         return [float(x) for x in ms]
 
+    def solid(self, which, normals, device=None):
+        """the Solid `which` of a handle of solids"""
+        v, f, nr = self.mesh(which, normals, device)
+        nv, nf, vol, area = C.c_uint64(), C.c_uint64(), C.c_double(), C.c_double()
+        check(_lib.lib().fr_isosurface_solid_info(self.h, which, C.byref(nv), C.byref(nf), C.byref(vol), C.byref(area)))
+        return Solid(v, f, nr, vol.value, area.value, nv.value, nf.value)
+
     def refine_stats(self, which):
         """(trial points evaluated, iterations of the slowest vertex) of the refinement of surface `which`"""
         ev, it = C.c_uint64(), C.c_uint64()
@@ -90,3 +111,20 @@ def lattice_isosurface(values, extents, isovalue):
                                                float(isovalue), _lib.cuda_stream(v.device), C.byref(h.h)))
         verts, faces, _ = h.mesh(0, False, v.device)
     return verts, faces
+
+
+def lattice_solid(values, extents, isovalue, *, side="below"):
+    """The level set `isovalue` of lattice values (as lattice_isosurface) closed at the lattice box into the solid
+    {f < isovalue} (side "below") or {f >= isovalue} ("above").  Returns a Solid of CUDA tensors on the values' device,
+    with normals None; a side with no node gives no faces and volume 0, a side with every node the box."""
+    sd = side_code(side)
+    import torch
+    if not isinstance(values, torch.Tensor) or not values.is_cuda or values.dtype != torch.float64 or values.dim() != 3:
+        raise TypeError("Expected a 3D float64 CUDA tensor (nz, ny, nx) for values")
+    v = values.contiguous()
+    nz, ny, nx = v.shape
+    ext, res = lattice_args(extents, (nx, ny, nz))
+    with torch.cuda.device(v.device), Handle() as h:
+        check(_lib.lib().fr_lattice_solid(v.data_ptr(), res.ctypes.data_as(_u64p), _lib.dptr(ext), float(isovalue), sd,
+                                          _lib.cuda_stream(v.device), C.byref(h.h)))
+        return h.solid(0, False, v.device)

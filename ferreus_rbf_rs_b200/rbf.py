@@ -352,16 +352,21 @@ class RBFInterpolator:
         return self._eval_cuda(self._L.fr_evaluate_targets_device, targets, gradients)
 
     # ---- isosurfaces (fr_isosurface_extract): one lattice evaluation and one transient tree for all isovalues ------
-    def _isosurfaces(self, isovalues, extents, resolution, column, refine, device):
-        """(meshes, {"ms": stage times, "refine": [(evaluations, iterations)] per isovalue})"""
+    def _isosurfaces(self, isovalues, extents, resolution, column, refine, device, sd=None):
+        """(meshes, or Solids for side code sd 0 / 1 (isosurface.side_code), {"ms": stage times, "refine":
+        [(evaluations, iterations)] per isovalue})"""
         from .isosurface import Handle, lattice_args
         ext, res = lattice_args(extents, resolution)
         iso = np.ascontiguousarray(np.atleast_1d(np.asarray(isovalues, dtype=np.float64)).ravel())
+        args = (self._h, _lib.dptr(ext), res.ctypes.data_as(C.POINTER(C.c_uint64)), _lib.dptr(iso), iso.size,
+                int(column), int(bool(refine)))
         with Handle() as h:
-            self._check(self._L.fr_isosurface_extract(self._h, _lib.dptr(ext), res.ctypes.data_as(C.POINTER(C.c_uint64)),
-                                                      _lib.dptr(iso), iso.size, int(column), int(bool(refine)),
-                                                      C.byref(h.h)))
-            meshes = [h.mesh(i, True, device) for i in range(iso.size)]
+            if sd is None:
+                self._check(self._L.fr_isosurface_extract(*args, C.byref(h.h)))
+                meshes = [h.mesh(i, True, device) for i in range(iso.size)]
+            else:
+                self._check(self._L.fr_isosurface_extract_solid(*args, sd, C.byref(h.h)))
+                meshes = [h.solid(i, True, device) for i in range(iso.size)]
             stats = {"ms": h.timing(), "refine": [h.refine_stats(i) for i in range(iso.size)]}
         return meshes, stats
 
@@ -380,6 +385,26 @@ class RBFInterpolator:
         import torch
         dev = torch.device("cuda", torch.cuda.current_device())
         return self._isosurfaces(isovalues, extents, resolution, column, refine, dev)[0]
+
+    def extract_solids(self, isovalues, extents, resolution, *, side="below", column=0, refine=True):
+        """The level sets of extract_isosurfaces closed at the lattice box into solids: one Solid (vertices, faces,
+        normals, volume, surface_area, n_surface_vertices, n_surface_faces) per isovalue, for the region {f < iso}
+        (side "below", the inside of a signed distance) or {f >= iso} ("above", a grade shell).  The first
+        n_surface_vertices / n_surface_faces rows are extract_isosurfaces' mesh for the same arguments (faces with their
+        last two columns exchanged for "above"); the cap follows: the lattice's boundary nodes on the solid's side and
+        the faces that close the mesh on the six box faces.  Every mesh edge is shared by exactly two faces, all faces
+        and normals point out of the solid, and volume / surface_area (the area of the isosurface faces inside the box)
+        are computed on the GPU from the final vertices."""
+        from .isosurface import side_code
+        return self._isosurfaces(isovalues, extents, resolution, column, refine, None, side_code(side))[0]
+
+    def extract_solids_cuda(self, isovalues, extents, resolution, *, side="below", column=0, refine=True):
+        """extract_solids with the arrays as torch CUDA tensors on the current CUDA device."""
+        import torch
+        from .isosurface import side_code
+        sd = side_code(side)
+        dev = torch.device("cuda", torch.cuda.current_device())
+        return self._isosurfaces(isovalues, extents, resolution, column, refine, dev, sd)[0]
 
     # ---- introspection -----------------------------------------------------------------------
     def ddm_level(self, level):

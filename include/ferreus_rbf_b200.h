@@ -174,8 +174,17 @@ int fr_evaluate_targets_device(fr_model *m, const double *d_targets, size_t n_ta
  *  - fr_isosurface_timing: milliseconds of {lattice evaluation with the tree, extraction, refinement, normals}.
  *  - fr_isosurface_refine_stats: trial points evaluated by the refinement and its iteration count (the slowest
  *    vertex's evaluations).
+ * Solids: fr_isosurface_extract_solid and fr_lattice_solid take the arguments above plus side (0: the region
+ * {f < iso}, 1: {f >= iso}) and close each isosurface at the lattice box into the boundary of that region.  The
+ * isosurface's vertices and faces come first, unchanged except that side 1 exchanges every face's last two vertices;
+ * then the boundary nodes on the solid's side (ascending node index) and the cap faces on the six box faces.  Every
+ * face points out of the solid; normals (model path) are outward too.  fr_isosurface_counts / _copy include the cap.
+ *  - fr_isosurface_solid_info: the number of isosurface vertices and faces at the front, the enclosed volume and the
+ *    area of the isosurface faces, computed on the device from the final vertices by fixed-order reductions (the same
+ *    bits from call to call).  FB_ERR_INVALID_ARGUMENT on a handle of open isosurfaces.
+ *  - for solids the refinement time of fr_isosurface_timing includes the volume and area reductions.
  * Invalid arguments (a model that is not 3-D, a bad lattice, n_iso < 1, a non-finite isovalue or lattice value, a
- * column out of range) return FB_ERR_INVALID_ARGUMENT and leave the model usable.                                 */
+ * column out of range, a side other than 0 or 1) return FB_ERR_INVALID_ARGUMENT and leave the model usable.       */
 typedef struct fr_isosurface fr_isosurface;
 int fr_isosurface_extract(fr_model *m, const double *extents, const uint64_t *resolution, const double *isovalues,
                           int n_iso, int column, int refine, fr_isosurface **out);
@@ -186,6 +195,13 @@ int fr_isosurface_copy(const fr_isosurface *s, int which, double *vertices, int6
 int fr_isosurface_timing(const fr_isosurface *s, double *ms_out4);
 int fr_isosurface_refine_stats(const fr_isosurface *s, int which, uint64_t *evaluations, uint64_t *iterations);
 void fr_isosurface_free(fr_isosurface *s);
+int fr_isosurface_extract_solid(fr_model *m, const double *extents, const uint64_t *resolution,
+                                const double *isovalues, int n_iso, int column, int refine, int side,
+                                fr_isosurface **out);
+int fr_lattice_solid(const double *d_values, const uint64_t *resolution, const double *extents, double isovalue,
+                     int side, void *stream, fr_isosurface **out);
+int fr_isosurface_solid_info(const fr_isosurface *s, int which, uint64_t *surface_vertices, uint64_t *surface_faces,
+                             double *volume, double *surface_area);
 
 /* ---- introspection for the parity gates ------------------------------------------------------------- */
 /* DDM hierarchy: level l (0 = finest ... levels-1 = coarse): number of domains, and per domain the point
